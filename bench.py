@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CudaIntegrator path (one rank per GPU)
     python bench.py --impl reference --steps K --warmup W    # the reference's own CPU implementation, same workload
+    python bench.py --steps K --warmup W --dump-outputs DIR  # + the last timed frame's per-pixel sums as DIR/*.npy
 
 A *step* is ONE FRAME of the workload.  The default workload is BASELINE.json configs[2] — bunny.sp, 1920x1080, 256 spp,
 iterative_rrnee — the config BASELINE.json quotes "at 1/2/4/8 GPUs".  With N ranks the frame's 256 samples per pixel are
@@ -173,7 +174,7 @@ def load_scene(ctx, scene_name: str, spp_total: int):
 # one workload, measured
 # =====================================================================================================================
 def measure(ctx, args, workload: str, spp_total: int, steps: int, warmup: int, world: int, rank: int, clocks_index=None,
-            e2e_steps: int = 3) -> dict:
+            e2e_steps: int = 3, keep_outputs: bool = False) -> dict:
     import torch
     import torch.distributed as dist
     from simplepath_b200 import capi, distributed
@@ -224,6 +225,8 @@ def measure(ctx, args, workload: str, spp_total: int, steps: int, warmup: int, w
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     total_ms = float(ms.item())
+    # what the last timed step handed its caller: rank 0's per-pixel sums after the reduction (the later steps overwrite them)
+    outputs = {"rgb_sum": rgb.cpu().numpy(), "lum_sumsq": sq.cpu().numpy()} if keep_outputs and rank == 0 else None
 
     # ---- per-kernel CUDA-event durations, same workload, directly after the timed steps (one event pair per launch would
     # perturb the headline number in the wavefront pipeline, so they are taken on their own steps) --------------------------
@@ -367,7 +370,24 @@ def measure(ctx, args, workload: str, spp_total: int, steps: int, warmup: int, w
         "roofline": roof,
         "stages_ms_per_step": {k: v / stage_steps for k, v in stage_ms.items() if stage_launches.get(k)},
         "_flat": flat,
+        **({"_outputs": outputs} if outputs is not None else {}),
     }
+
+
+def dump_outputs(directory: Path, outputs: dict, limit: int = 64 << 20) -> None:
+    """Writes each output as <directory>/<name>.npy.  Outputs larger than `limit` in all (the 4K frames) are written as the
+    same seeded sample of pixels for every array, with that sample's flat pixel indices as pixel_index.npy."""
+    directory.mkdir(parents=True, exist_ok=True)
+    total = sum(a.nbytes for a in outputs.values())
+    if total > limit:
+        h, w = outputs["lum_sumsq"].shape
+        keep = (limit - 4096) // (total // (h * w) + 8)   # bytes per pixel of the outputs and of its float64 index; .npy headers
+        pick = np.sort(np.random.default_rng(0).choice(h * w, keep, replace=False))
+        n_pix = h * w
+        outputs = {k: a.reshape(n_pix, *a.shape[2:])[pick] for k, a in outputs.items()}
+        outputs["pixel_index"] = pick.astype(np.float64)
+    for name, a in outputs.items():
+        np.save(directory / f"{name}.npy", np.ascontiguousarray(a))
 
 
 def ordered_walk_report(ctx, flat) -> dict:
@@ -419,14 +439,22 @@ def run_cuda(args) -> None:
 
     spp_total = args.spp or WORKLOADS[args.workload][1]
     main = measure(ctx, args, args.workload, spp_total, args.steps, args.warmup, world, rank, clocks_index=local_rank,
-                   e2e_steps=max(1, min(args.steps, 3)))
+                   e2e_steps=max(1, min(args.steps, 3)), keep_outputs=args.dump_outputs is not None)
+    if rank == 0 and args.dump_outputs is not None:
+        dump_outputs(Path(args.dump_outputs), main.pop("_outputs"))
     side: dict[str, dict] = {}
     if world > 1 and args.workload == DEFAULT_WORKLOAD and world == 8 and not args.no_side_configs:
-        # BASELINE configs[4]: lucy 3840x2160 256 spp "on 8xB200" — the whole config, two timed frames
-        r = measure(ctx, args, "lucy_4k_256spp", 256, 2, 3, world, rank, e2e_steps=1)
-        if rank == 0:
-            r.pop("_flat")
-            side["c5_lucy_4k_256spp_8gpu"] = r
+        # BASELINE configs[4]: lucy 3840x2160 256 spp "on 8xB200" — the whole config, two timed frames.  Every rank takes
+        # the same branch: a scene that cannot be loaded here must not leave the other ranks waiting in a collective.
+        from simplepath_b200 import host
+        if host.loadable("c5_lucy_standin"):
+            r = measure(ctx, args, "lucy_4k_256spp", 256, 2, 3, world, rank, e2e_steps=1)
+            if rank == 0:
+                r.pop("_flat")
+                side["c5_lucy_4k_256spp_8gpu"] = r
+        elif rank == 0:
+            side["c5_lucy_4k_256spp_8gpu"] = {"error": "c5_lucy_standin needs the reference's parser (libsphost.so), "
+                                                       "which is not built"}
     if rank != 0:
         ctx.close()
         if world > 1:
@@ -676,7 +704,13 @@ def main() -> None:
     ap.add_argument("--batch-lanes", type=int, default=0,
                     help="wavefront batches in flight at once (SPCU_OPT_BATCH_LANES; 0 = the library's default, 4)")
     ap.add_argument("--wavefront-size", type=int, default=0, help="slots per wavefront batch (spcu_set_wavefront_size; 0 = default 2^24)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the headline workload's per-pixel sums of the last timed step as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "cuda":
+        ap.error("--dump-outputs writes what the CUDA path computed: it needs --impl cuda")
     if args.warmup < 3 and args.impl == "cuda":
         args.warmup = 3
     if args.impl == "reference":

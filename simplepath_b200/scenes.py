@@ -365,6 +365,19 @@ def _specs():
     }
 
 
+# Mesh scenes that host.assemble() puts together without the reference's parser: name -> (tiny scene of the same .sp text
+# whose flattened form is committed, meshes in .sp order as (triangles, lo, hi, translate, uniform scale, material)).
+# material = the flattener's index of the mesh's material: sp_bunny's four meshes use material_glossy_clearcoat,
+# material_lambertian_clearcoat, material_lambertian and material_glossy; sp_elf's mesh material_glossy_clearcoat.
+_BUNNY_MESHES = ((2.25, 6), (0.75, 4), (-0.75, 2), (-2.25, 1))
+ASSEMBLED = {
+    "c3_bunny": ("g_bunny", [(BUNNY_TRIS, BUNNY_LO, BUNNY_HI, (tx, 0.0, 0.0), 10.0, m) for tx, m in _BUNNY_MESHES]),
+    "c4_elf": ("g_elf", [(ELF_TRIS, ELF_LO, ELF_HI, (0.0, 0.0, 0.0), 1.0, 2)]),
+    "g_bunny": ("g_bunny", [(420, BUNNY_LO, BUNNY_HI, (tx, 0.0, 0.0), 10.0, m) for tx, m in _BUNNY_MESHES]),
+    "g_elf": ("g_elf", [(1_500, ELF_LO, ELF_HI, (0.0, 0.0, 0.0), 1.0, 2)]),
+}
+
+
 def _ply(out: Path, stem: str, n_tris: int, lo, hi) -> str:
     path = out / f"{stem}_{n_tris}.ply"
     if not path.exists():

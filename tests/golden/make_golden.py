@@ -36,7 +36,7 @@ N_EACH = 4096
 
 def main() -> None:
     if not ref.available():
-        raise SystemExit("oracle/_ref/libsp_ref.so missing: run `make -C oracle` where /root/reference exists")
+        raise SystemExit("oracle/_ref/libsp_ref.so missing: run `make -C oracle REF=<the reference sources>`")
     for name in (sys.argv[1:] or NAMES):   # python tests/golden/make_golden.py [scene ...]
         path = scenes.ensure(name)
         w, h, spp = scenes.info(name)

@@ -27,7 +27,7 @@ HEAD_KEYS = ("n_prims", "n_unbounded", "n_nodes", "root", "root_count", "max_dep
 
 def main() -> None:
     if not ref.available():
-        raise SystemExit("oracle/_ref/libsp_ref.so missing: run `make -C oracle` where /root/reference exists")
+        raise SystemExit("oracle/_ref/libsp_ref.so missing: run `make -C oracle REF=<the reference sources>`")
     out = {}
     for name, (bounds, non_tri, first_id) in bvhcases.cases().items():
         r = ref.build_bvh(bounds, non_tri, first_id)

@@ -7,7 +7,6 @@ For every config it renders `iterative_rrnee` with the REAL reference (libsp_ref
 mt19937_64 sampler) at the stated sample count and stores, per block of BxB pixels (B = 1 for the 256x256 config, B = 8 =
 the reference's tile size for the 1080p configs, so that the file stays a few hundred KB):
 
-    rgb       block mean of the per-pixel mean radiance               [H/B, W/B, 3]
     lum       block mean of the per-pixel mean luminance              [H/B, W/B]
     lum_var   block mean of the per-pixel luminance VARIANCE (RunningStats, base/RunningStats.h:12-69)  [H/B, W/B]
     spp, block, width, height
@@ -47,7 +46,7 @@ def block_mean(a: np.ndarray, b: int) -> np.ndarray:
 
 def main() -> None:
     if not ref.available():
-        raise SystemExit("oracle/_ref/libsp_ref.so missing: run `make -C oracle` where /root/reference exists")
+        raise SystemExit("oracle/_ref/libsp_ref.so missing: run `make -C oracle REF=<the reference sources>`")
     import os
     threads = os.cpu_count() or 1
     for cfg in (sys.argv[1:] or list(CONFIGS)):
@@ -56,7 +55,9 @@ def main() -> None:
         rs = ref.RefScene(scenes.ensure(scene))
         rgb, mean, var, secs = rs.render("iterative_rrnee", spp, threads)
         rs.close()
-        np.savez_compressed(HERE / f"converged_{cfg}.npz", rgb=block_mean(rgb, b), lum=block_mean(mean, b),
+        # no colour image: the relMSE is taken over luminance, and the image kept converged_c1.npz above 1 MB (files
+        # written before this change still hold it as rgb, which nothing reads)
+        np.savez_compressed(HERE / f"converged_{cfg}.npz", lum=block_mean(mean, b),
                             lum_var=block_mean(var, b), spp=np.array(spp), block=np.array(b),
                             width=np.array(rgb.shape[1]), height=np.array(rgb.shape[0]))
         print(cfg, scene, f"{spp} spp, render {secs:.1f} s, total {time.time() - t0:.1f} s", flush=True)

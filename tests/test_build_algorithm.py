@@ -25,7 +25,7 @@ def test_tie_heavy_inputs_against_the_live_reference(oracle_port):
     """Coordinates drawn from a handful of values (signed zeros among them): ties in every fold and every partition."""
     from oracle import ref
     if not ref.available():
-        pytest.skip("reference library not built (needs /root/reference)")
+        pytest.skip("reference library not built (needs the reference sources: SP_REFERENCE, or a checkout named reference beside the repository)")
     rng = np.random.default_rng(99)
     values = np.array([-0.0, 0.0, -1.0, 1.0, 0.5, 2.0, -2.0], dtype=np.float32)
     for trial in range(200):

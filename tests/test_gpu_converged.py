@@ -46,8 +46,8 @@ def test_relmse_against_the_reference_render(ctx, cfg):
     path = GOLDEN / f"converged_{cfg.split('_')[0]}.npz"
     if not path.exists():
         pytest.skip(f"{path.name} not generated")
-    if not host.available():
-        pytest.skip("libsphost.so (the reference's parser + the flattener) is not built")
+    if not host.loadable(scene):
+        pytest.skip(f"{scene} needs the reference's parser + the flattener (libsphost.so), which is not built")
     gold = np.load(path)
     b, n_ref = int(gold["block"]), int(gold["spp"])
     flat = host.workload(scene)

@@ -20,8 +20,8 @@ SCENES = ["c3_bunny", "t_lucy_1m"]
 
 @pytest.fixture(scope="module", params=SCENES)
 def big_scene(request, ctx):
-    if not host.available():
-        pytest.skip("libsphost.so (the reference's parser + the flattener) is not built")
+    if not host.loadable(request.param):
+        pytest.skip(f"{request.param} needs the reference's parser + the flattener (libsphost.so), which is not built")
     flat = host.workload(request.param)
     jitter = rsequence.jitter_table(4)
     ctx.upload_scene(flat.pointer(), jitter, keepalive=flat)

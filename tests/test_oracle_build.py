@@ -64,7 +64,7 @@ def test_oracle_rebuilds_the_scene_bvh(oracle_port, name):
 def test_oracle_build_on_live_reference(oracle_port):
     from oracle import ref
     if not ref.available():
-        pytest.skip("reference library not built (needs /root/reference)")
+        pytest.skip("reference library not built (needs the reference sources: SP_REFERENCE, or a checkout named reference beside the repository)")
     rng = np.random.default_rng(77)
     for n in (7, 100, 4097, 60000):
         b = bvhcases.boxes(rng, n, spread=float(rng.uniform(0.1, 100)), size=float(rng.uniform(1e-4, 1.0)))

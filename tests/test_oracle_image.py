@@ -29,7 +29,7 @@ def test_oracle_image_on_live_reference(oracle_port, tmp_path):
     from oracle import ref
     import imagecases
     if not ref.available():
-        pytest.skip("reference library not built (needs /root/reference)")
+        pytest.skip("reference library not built (needs the reference sources: SP_REFERENCE, or a checkout named reference beside the repository)")
     sums, spp = imagecases.sums(seed=5, w=33, h=17, spp=64)
     ref.write_image(sums, spp, tmp_path / "a.pfm")
     ref.write_image(sums, spp, tmp_path / "a.ppm")

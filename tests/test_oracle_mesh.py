@@ -36,7 +36,7 @@ def test_oracle_ingest_on_live_reference(oracle_port, tmp_path):
     from oracle import ref
     from simplepath_b200 import scenes
     if not ref.available():
-        pytest.skip("reference library not built (needs /root/reference)")
+        pytest.skip("reference library not built (needs the reference sources: SP_REFERENCE, or a checkout named reference beside the repository)")
     v, f = meshcases.mesh(n_tris=20000, seed=8)
     xf = meshcases.transform(seed=12)
     scenes.write_ply(tmp_path / "m.ply", v, f)
@@ -116,7 +116,7 @@ def test_small_degenerate_meshes_on_live_reference(oracle_port, tmp_path):
     from oracle import ref
     from simplepath_b200 import scenes
     if not ref.available():
-        pytest.skip("reference library not built (needs /root/reference)")
+        pytest.skip("reference library not built (needs the reference sources: SP_REFERENCE, or a checkout named reference beside the repository)")
     rng = np.random.default_rng(123)
     values = np.array([0.0, 1.0, -1.0, 0.5, 2.0], dtype=np.float32)
     xf = meshcases.transform(seed=21)

@@ -11,7 +11,7 @@ from simplepath_b200.flat import FlatSceneData
 import raybatches
 
 pytestmark = pytest.mark.skipif(not (ref.available(ref.STRICT) and ref.available(ref.FAST)),
-                                reason="reference libraries not built (needs /root/reference)")
+                                reason="reference libraries not built (needs the reference sources: SP_REFERENCE, or a checkout named reference beside the repository)")
 
 
 @pytest.fixture(scope="module")
