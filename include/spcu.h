@@ -298,6 +298,40 @@ int spcu_render_frame(spcu_ctx* ctx, const spcu_partition* part, float* rgb_sum,
 int spcu_render_device(spcu_ctx* ctx, const spcu_partition* part, float* d_rgb_sum, float* d_lum_sumsq,
                        spcu_stats* stats, void* stream);
 
+/* ---- adaptive sampling --------------------------------------------------------------------------------------------------
+ * Renders each pixel until the standard error of its mean luminance meets a target, instead of the same sample count
+ * everywhere.  Replaces nothing in the reference (it renders num_pixel_samples for every pixel, main.cpp:90-102).
+ * The partition's sample_end is the budget (the most samples any pixel gets); sample_begin must be 0.  Passes end at fixed
+ * sample counts that depend only on these parameters, never on the image:
+ *   s_0 = min(min_spp, sample_end),  s_{k+1} = min(s_k + pass_spp, sample_end).
+ * Pass 0 renders samples [0, s_0) of every pixel of the partition; at each boundary s_k < sample_end every pixel still active
+ * is tested with n = s_k, and the pass after it renders [s_k, s_{k+1}) of the pixels that failed the test only.  The test,
+ * float32 with one rounding per operation (R, G, B = the pixel's rgb_sum, Q = its lum_sumsq):
+ *   L = (0.2126 R + 0.7152 G) + 0.0722 B;  m = L / n;  d = Q / n - m m;  v = d > 0 ? d (n / (n - 1)) : 0;
+ *   stop  <=>  R, G, B, Q finite  and  v / n <= (rel_error (m + abs_floor))^2
+ * So pixel p gets samples [0, n_p) with min(min_spp, sample_end) <= n_p <= sample_end, and its sums equal bit for bit those
+ * of a fixed render of [0, n_p): the result does not depend on the tile partition, the batch shape or the kernel
+ * organisation.  Stopping on an estimated variance biases the mean slightly in principle (DESIGN.md). */
+typedef struct spcu_adaptive {
+    uint32_t min_spp;   /* samples before the first test, >= 2                                              */
+    uint32_t pass_spp;  /* samples added per pass, >= 1                                                     */
+    float    rel_error; /* target standard error relative to the mean luminance, finite, >= 0             */
+    float    abs_floor; /* added to the mean in the target, so that near-black pixels can stop; finite, >= 0 */
+} spcu_adaptive;
+
+/* Adaptive render of a tile partition into host buffers, OVERWRITTEN like spcu_render_frame's: rgb_sum / lum_sumsq (may be
+ * NULL) as there, spp_map[y*w+x] = n_p (0 outside the partition).  n_passes (may be NULL) = passes rendered.  stats are
+ * summed over the passes, device_ms covers the whole call.  SPCU_ERR_INVALID for parameters outside the rules above or
+ * sample_begin != 0; the context stays usable. */
+int spcu_render_adaptive(spcu_ctx* ctx, const spcu_partition* part, const spcu_adaptive* ad, float* rgb_sum, float* lum_sumsq,
+                         uint32_t* spp_map, uint32_t* n_passes, spcu_stats* stats);
+/* Same into DEVICE buffers of the image's size on `stream` (cudaStream_t as void*, NULL = default stream), also
+ * overwritten; d_lum_sumsq may be NULL.  With tile partitions the ranks' sums can then be added by spcu_reduce_to_root (and
+ * their spp maps, which are 0 outside each rank's tiles, likewise by the caller).  The call synchronises once per pass: the
+ * host needs the number of active pixels to shape the next pass. */
+int spcu_render_adaptive_device(spcu_ctx* ctx, const spcu_partition* part, const spcu_adaptive* ad, float* d_rgb_sum,
+                                float* d_lum_sumsq, uint32_t* d_spp_map, uint32_t* n_passes, spcu_stats* stats, void* stream);
+
 /* ---- multi-GPU: accumulators summed into rank 0 with NCCL over NVLink (SURVEY.md §8e) ------------------------------------
  * The scene is replicated (every rank uploads it), the work is partitioned by spcu_partition (tiles or sample ranges), there
  * is no exchange during tracing; ONE ncclReduce(sum, root 0) per accumulator ends a frame.  Replaces nothing in the reference
@@ -442,6 +476,10 @@ int spcu_triangle_bounds(spcu_ctx* ctx, const spcu_prim_geom* tris, uint32_t n, 
 #define SPCU_IMAGE_PPM 1u
 /* Packs host-resident per-pixel sums (rgb_sum[(y*w+x)*3+c], as spcu_render returns them). */
 int spcu_pack_image(spcu_ctx* ctx, const float* rgb_sum, uint32_t width, uint32_t height, uint32_t spp, uint32_t format, void* out);
+/* spcu_pack_image with a per-pixel divisor: spp_map[y*w+x] (host, as spcu_render_adaptive returns it) in place of spp.  A
+ * pixel with 0 samples packs as 0. */
+int spcu_pack_image_counts(spcu_ctx* ctx, const float* rgb_sum, const uint32_t* spp_map, uint32_t width, uint32_t height,
+                           uint32_t format, void* out);
 /* spcu_render_frame + packing of the device-resident sums: only the packed image crosses to the host.  The divisor is the
  * partition's sample count (sample_end - sample_begin). */
 int spcu_render_image(spcu_ctx* ctx, const spcu_partition* part, uint32_t format, void* out, spcu_stats* stats);

@@ -101,6 +101,11 @@ class Stats(C.Structure):
         return {n: getattr(self, n) for n, _ in self._fields_ if not n.startswith("_")}
 
 
+class Adaptive(C.Structure):
+    """spcu_adaptive: parameters of spcu_render_adaptive (include/spcu.h)."""
+    _fields_ = [("min_spp", C.c_uint32), ("pass_spp", C.c_uint32), ("rel_error", C.c_float), ("abs_floor", C.c_float)]
+
+
 class StageTime(C.Structure):
     _fields_ = [("name", C.c_char * 24), ("launches", C.c_uint64), ("items", C.c_uint64), ("ms", C.c_float),
                 ("traverses", C.c_uint32)]
@@ -115,6 +120,7 @@ EXPORTS = [
     "spcu_extend_batch", "spcu_shadow_batch",
     "spcu_comm_unique_id", "spcu_comm_init_rank", "spcu_comm_init_all", "spcu_comm_destroy", "spcu_comm_rank", "spcu_comm_size",
     "spcu_reduce_to_root", "spcu_render_frame_reduced",
+    "spcu_render_adaptive", "spcu_render_adaptive_device", "spcu_pack_image_counts",
 ]
 NCCL_ID_BYTES = 128
 OPT_COUNT_NODES, OPT_STAGE_TIMING, OPT_PIPELINE, OPT_TRAVERSAL, OPT_GENERIC_KERNELS, OPT_BATCH_LANES = 0, 1, 2, 3, 4, 5
@@ -206,6 +212,14 @@ def load(path: Path | str | None = None) -> C.CDLL:
     lib.spcu_ingest_mesh_stl.restype = C.c_int
     lib.spcu_pack_image.argtypes = [vp, vp, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, vp]
     lib.spcu_pack_image.restype = C.c_int
+    lib.spcu_pack_image_counts.argtypes = [vp, vp, vp, C.c_uint32, C.c_uint32, C.c_uint32, vp]
+    lib.spcu_pack_image_counts.restype = C.c_int
+    lib.spcu_render_adaptive.argtypes = [vp, C.POINTER(Partition), C.POINTER(Adaptive), vp, vp, vp, C.POINTER(C.c_uint32),
+                                         C.POINTER(Stats)]
+    lib.spcu_render_adaptive.restype = C.c_int
+    lib.spcu_render_adaptive_device.argtypes = [vp, C.POINTER(Partition), C.POINTER(Adaptive), vp, vp, vp, C.POINTER(C.c_uint32),
+                                                C.POINTER(Stats), vp]
+    lib.spcu_render_adaptive_device.restype = C.c_int
     lib.spcu_render_image.argtypes = [vp, C.POINTER(Partition), C.c_uint32, vp, C.POINTER(Stats)]
     lib.spcu_render_image.restype = C.c_int
     lib.spcu_triangle_bounds.argtypes = [vp, vp, C.c_uint32, vp]
@@ -472,13 +486,38 @@ class Context:
         return run_ingest(lambda *a: self._check(self.lib.spcu_ingest_mesh_stl(self.h, *a), "spcu_ingest_mesh_stl"),
                           vertices, faces, object_to_world, normal_xf, material, with_ms=True, face_normals=face_normals)
 
-    def pack_image(self, rgb_sum, spp: int, fmt: int) -> np.ndarray:
-        """Host sums [H, W, 3] -> write_pfm payload (float32) / write_ppm numbers (uint16), rows bottom-up."""
+    def pack_image(self, rgb_sum, spp, fmt: int) -> np.ndarray:
+        """Host sums [H, W, 3] -> write_pfm payload (float32) / write_ppm numbers (uint16), rows bottom-up.  spp: the samples
+        of every pixel (int), or the per-pixel counts [H, W] of render_adaptive (spcu_pack_image_counts)."""
         rgb_sum = np.ascontiguousarray(rgb_sum, dtype=np.float32)
         h, w = rgb_sum.shape[:2]
         out = np.empty((h, w, 3), dtype=IMAGE_DTYPES[fmt])
+        if isinstance(spp, np.ndarray):
+            counts = np.ascontiguousarray(spp, dtype=np.uint32)
+            if counts.shape != (h, w):
+                raise ValueError(f"spp map of shape {counts.shape} for a {h}x{w} image")
+            self._check(self.lib.spcu_pack_image_counts(self.h, _ptr(rgb_sum), _ptr(counts), w, h, fmt, _ptr(out)),
+                        "spcu_pack_image_counts")
+            return out
         self._check(self.lib.spcu_pack_image(self.h, _ptr(rgb_sum), w, h, spp, fmt, _ptr(out)), "spcu_pack_image")
         return out
+
+    def render_adaptive(self, part: Partition, rel_error: float, min_spp: int = 16, pass_spp: int = 16, abs_floor: float = 0.0,
+                        want_sumsq: bool = True):
+        """Adaptive sampling (spcu_render_adaptive): each pixel of the partition gets samples [0, n_p) until the standard error of
+        its mean luminance is at most rel_error * (mean + abs_floor), n_p <= part.sample_end (the budget).  Outputs are
+        overwritten: (rgb_sum [H,W,3], lum_sumsq [H,W] | None, spp_map [H,W] uint32 = n_p, stats dict with "passes")."""
+        rgb = np.empty((self.height, self.width, 3), dtype=np.float32)
+        sq = np.empty((self.height, self.width), dtype=np.float32) if want_sumsq else None
+        spp_map = np.empty((self.height, self.width), dtype=np.uint32)
+        ad = Adaptive(min_spp, pass_spp, rel_error, abs_floor)
+        passes = C.c_uint32()
+        st = Stats()
+        self._check(self.lib.spcu_render_adaptive(self.h, C.byref(part), C.byref(ad), _ptr(rgb), _ptr(sq) if want_sumsq else None,
+                                                  _ptr(spp_map), C.byref(passes), C.byref(st)), "spcu_render_adaptive")
+        stats = st.as_dict()
+        stats["passes"] = passes.value
+        return rgb, sq, spp_map, stats
 
     def render_image(self, part: Partition, fmt: int):
         """Render + pack on the device: (packed image [H, W, 3], stats)."""

@@ -120,6 +120,10 @@ struct spcu_ctx
     uint32_t                  pix_list_offset = ~0u, pix_list_stride = 0, pix_list_n = 0;
     spcu::DevBuf              host_rgb, host_sq; // device accumulators of the host-buffer entry point
     spcu::DevBuf              packed;            // packed output image (spcu_render_image / spcu_pack_image)
+    // adaptive sampling (spcu_render_adaptive): ping-pong active pixel lists, the per-pixel sample counts, a lum_sumsq
+    // accumulator for callers that pass none, the compaction's scratch + active count, and the call's event pair
+    spcu::DevBuf              ad_list[2], ad_spp_map, ad_sq, ad_scratch;
+    cudaEvent_t               ad_ev[2] = { nullptr, nullptr };
     void*                     stage[2]    = { nullptr, nullptr }; // page-locked staging of large host->device copies
     cudaEvent_t               stage_ev[2] = { nullptr, nullptr };
     bool                      stage_busy[2] = { false, false };
@@ -145,7 +149,9 @@ int need_scene(spcu_ctx* c);
 // staging buffers (CPU memcpy of chunk k+1 overlaps the DMA of chunk k); the source is fully consumed when the call returns.
 int copy_to_device(spcu_ctx* c, void* dst, const void* src, size_t bytes);
 // image_kernels.cu: mean, row order and sRGB quantisation of device-resident sums, result copied to the host buffer `out`
-int pack_device_image(spcu_ctx* c, const float* d_rgb_sum, uint32_t w, uint32_t h, uint32_t spp, uint32_t format, void* out);
+// d_counts (may be NULL): per-pixel sample counts dividing the sums in place of spp
+int pack_device_image(spcu_ctx* c, const float* d_rgb_sum, const uint32_t* d_counts, uint32_t w, uint32_t h, uint32_t spp,
+                      uint32_t format, void* out);
 // build_kernels.cu: geometry of an UNBUILT scene -> bounds, BVH and leaf-order gather on the device (spcu_upload_scene_build)
 int build_scene_geometry(spcu_ctx* c, const spcu_flat_scene* s, const spcu_bounds* extra_bounds, uint32_t* order_out,
                          spcu_accel* built, bool* proper_boxes);

@@ -123,6 +123,17 @@ cudaError_t launch_smwave(const Launch& l, const DScene& s, const uint32_t* d_pi
                           uint32_t n_samples, uint64_t seed, uint32_t integrator, float4* d_radiance,
                           unsigned long long* d_counters, TraceCounters* d_cnt);
 
+// ---- adaptive_kernels.cu (exact float32 arithmetic: --fmad=false, no fast-math) ----------------------------------------------
+// The stopping test of spcu_render_adaptive at a pass boundary, for list entries [0, n) after n_samples samples: pixels that
+// pass get d_spp_map[pix] = n_samples, the others are copied, in list order, to d_next_list; *d_n_next = how many.
+// d_scratch: adaptive_scratch_bytes(n) bytes.  Enqueue only.
+size_t      adaptive_scratch_bytes(uint32_t n);
+cudaError_t launch_adaptive_compact(const uint32_t* d_list, uint32_t n, const float* d_rgb_sum, const float* d_lum_sumsq,
+                                    uint32_t n_samples, float rel_error, float abs_floor, uint32_t* d_spp_map, uint32_t* d_next_list,
+                                    void* d_scratch, uint32_t* d_n_next, cudaStream_t st);
+// d_spp_map[d_list[i]] = value for i < n
+cudaError_t launch_adaptive_fill(const uint32_t* d_list, uint32_t n, uint32_t value, uint32_t* d_spp_map, cudaStream_t st);
+
 // pixel list of one rank: tiles t with t % stride == offset, 8x8 tiles row major (TileScheduler.h:66-82)
 uint32_t    count_partition_pixels(uint32_t width, uint32_t height, uint32_t tile_offset, uint32_t tile_stride);
 // d_tile_prefix_scratch: one uint32 per owned tile.  Synchronises the stream.

@@ -264,7 +264,8 @@ void spcu_destroy(spcu_ctx* c)
     spcu_comm_destroy(c);
     for (DevBuf* b : { &c->geom_wide, &c->geom_big, &c->geom_nodes, &c->geom_prims, &c->geom_shade, &c->geom_meta, &c->light_nodes, &c->lights,
                        &c->light_order, &c->materials, &c->bxdfs, &c->pool, &c->jitter, &c->q_rays, &c->q_out, &c->q_aux,
-                       &c->q_cnt, &c->queue_counts, &c->counters, &c->pix_list, &c->host_rgb, &c->host_sq, &c->path_radiance, &c->sorted_queue, &c->packed }) {
+                       &c->q_cnt, &c->queue_counts, &c->counters, &c->pix_list, &c->host_rgb, &c->host_sq, &c->path_radiance, &c->sorted_queue, &c->packed,
+                       &c->ad_list[0], &c->ad_list[1], &c->ad_spp_map, &c->ad_sq, &c->ad_scratch }) {
         b->release();
     }
     for (auto& b : c->wave_bufs) {
@@ -280,6 +281,9 @@ void spcu_destroy(spcu_ctx* c)
         if (lane.stream) cudaStreamDestroy(lane.stream);
     }
     if (c->resolved) cudaEventDestroy(c->resolved);
+    for (auto e : c->ad_ev) {
+        if (e) cudaEventDestroy(e);
+    }
     for (auto e : c->stage_events) {
         cudaEventDestroy(e);
     }

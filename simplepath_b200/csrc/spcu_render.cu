@@ -10,6 +10,7 @@
 #include "ctx.h"
 
 #include <chrono>
+#include <cmath>
 
 using namespace spcu;
 
@@ -198,8 +199,8 @@ int read_back_stats(spcu_ctx* c, cudaStream_t st, spcu_stats* stats, uint64_t la
 }
 
 // SPCU_PIPELINE_PATHS: one persistent kernel per batch (path_kernels.cu) + resolve.
-int render_paths(spcu_ctx* c, const spcu_partition* part, float* d_rgb_sum, float* d_lum_sumsq, spcu_stats* stats,
-                 cudaStream_t st, uint32_t n_pix, uint32_t n_samples, bool sm_local)
+int render_paths(spcu_ctx* c, const spcu_partition* part, const uint32_t* d_pix_list, uint32_t n_pix, uint32_t sample_begin,
+                 uint32_t n_samples, float* d_rgb_sum, float* d_lum_sumsq, spcu_stats* stats, cudaStream_t st, bool sm_local)
 {
     const DScene& s = c->ds;
     // batch = whole pixel list x as many samples as fit in the radiance buffer (16 B per path)
@@ -217,7 +218,6 @@ int render_paths(spcu_ctx* c, const spcu_partition* part, float* d_rgb_sum, floa
     CK(c, c->counters.reserve(kCounterBlock * sizeof(unsigned long long) + sizeof(TraceCounters)));
     auto*          d_counters = c->counters.as<unsigned long long>();
     TraceCounters* d_cnt = c->options[SPCU_OPT_COUNT_NODES] ? reinterpret_cast<TraceCounters*>(d_counters + kCounterBlock) : nullptr;
-    const uint32_t* d_pix_list = c->pix_list.as<uint32_t>();
     const Launch    L{ c->sm_count, st, c->features };
     StageTimer      timer{ c, c->options[SPCU_OPT_STAGE_TIMING] != 0, st };
     uint64_t        launches = 0;
@@ -231,10 +231,10 @@ int render_paths(spcu_ctx* c, const spcu_partition* part, float* d_rgb_sum, floa
             const uint32_t ns = std::min(smp_per_batch, n_samples - sb);
             timer.begin(kStPaths);
             if (sm_local) {
-                CK(c, launch_smwave(L, s, d_pix_list + pb, np, part->sample_begin + sb, ns, part->seed, part->integrator,
+                CK(c, launch_smwave(L, s, d_pix_list + pb, np, sample_begin + sb, ns, part->seed, part->integrator,
                                     d_radiance, d_counters, d_cnt));
             } else {
-                launch_paths(L, s, d_pix_list + pb, np, part->sample_begin + sb, ns, part->seed, part->integrator, d_radiance,
+                launch_paths(L, s, d_pix_list + pb, np, sample_begin + sb, ns, part->seed, part->integrator, d_radiance,
                              d_counters, d_cnt);
             }
             timer.end();
@@ -263,8 +263,10 @@ uint32_t resolve_pipeline(const spcu_ctx* c)
     return (c->features == FeatAnalytic::id && smwave_supports(c->ds)) ? SPCU_PIPELINE_SMWAVE : SPCU_PIPELINE_WAVEFRONT;
 }
 
-int render_impl(spcu_ctx* c, const spcu_partition* part, float* d_rgb_sum, float* d_lum_sumsq, spcu_stats* stats,
-                cudaStream_t caller_stream, bool have_caller_stream)
+// Argument checks of a render call, ordering of the context's scratch after earlier renders on other streams, and the
+// partition's pixel list (c->pix_list, c->pix_list_n).  st = the stream the call runs on.
+int prepare_render(spcu_ctx* c, const spcu_partition* part, const float* d_rgb_sum, cudaStream_t caller_stream, bool have_caller_stream,
+                   cudaStream_t& st)
 {
     if (int rc = need_scene(c); rc != SPCU_OK) return rc;
     if (!part || !d_rgb_sum) {
@@ -282,7 +284,7 @@ int render_impl(spcu_ctx* c, const spcu_partition* part, float* d_rgb_sum, float
         return fail(c, SPCU_ERR_INVALID, "unknown integrator %u", part->integrator);
     }
     // The caller's stream (spcu_render_device) orders this call after the caller's earlier work on that stream.
-    const cudaStream_t st = have_caller_stream ? caller_stream : c->stream;
+    st = have_caller_stream ? caller_stream : c->stream;
     // The wavefront state, queues and counters are context-owned scratch: a render on ANOTHER stream than the previous one
     // must not start before that one has finished with them (ev1 is recorded at the end of every render).
     if (c->scratch_in_use && c->scratch_stream != st) {
@@ -290,24 +292,24 @@ int render_impl(spcu_ctx* c, const spcu_partition* part, float* d_rgb_sum, float
     }
     c->scratch_in_use = true;
     c->scratch_stream = st;
+    return ensure_pixel_list(c, *part);
+}
 
-    if (int rc = ensure_pixel_list(c, *part); rc != SPCU_OK) return rc;
-    const uint32_t n_pix     = c->pix_list_n;
-    const uint32_t n_samples = part->sample_end - part->sample_begin;
-    if (stats) {
-        std::memset(stats, 0, sizeof *stats);
-    }
-    if (n_pix == 0 || n_samples == 0) {
-        return SPCU_OK;
-    }
-
+// The batch loop: samples [sample_begin, sample_begin + n_samples) of the n_pix pixels of d_pix_list (n_pix, n_samples > 0),
+// added to the accumulators in sample order.  keep_capacity: reuse wavefront buffers that are already large enough instead of
+// re-sizing them to this call's batch (the adaptive passes shrink from one pass to the next).
+int render_batches(spcu_ctx* c, const spcu_partition* part, const uint32_t* d_pix_list, uint32_t n_pix, uint32_t sample_begin,
+                   uint32_t n_samples, float* d_rgb_sum, float* d_lum_sumsq, spcu_stats* stats, cudaStream_t st, bool keep_capacity)
+{
+    const DScene&  s        = c->ds;
     const uint32_t pipeline = resolve_pipeline(c);
     if (pipeline == SPCU_PIPELINE_SMWAVE && !smwave_supports(s)) {
         return fail(c, SPCU_ERR_INVALID, "SPCU_PIPELINE_SMWAVE: max_depth %u / %u lights exceed its packed path flags",
                     s.max_depth, s.n_lights);
     }
     if (pipeline == SPCU_PIPELINE_PATHS || pipeline == SPCU_PIPELINE_SMWAVE) {
-        return render_paths(c, part, d_rgb_sum, d_lum_sumsq, stats, st, n_pix, n_samples, pipeline == SPCU_PIPELINE_SMWAVE);
+        return render_paths(c, part, d_pix_list, n_pix, sample_begin, n_samples, d_rgb_sum, d_lum_sumsq, stats, st,
+                            pipeline == SPCU_PIPELINE_SMWAVE);
     }
 
     // batch shape: whole pixel list x as many samples as fit, or a slice of the pixel list x one sample
@@ -320,7 +322,10 @@ int render_impl(spcu_ctx* c, const spcu_partition* part, float* d_rgb_sum, float
         pix_per_batch = static_cast<uint32_t>(target);
         smp_per_batch = 1;
     }
-    const uint32_t capacity = pix_per_batch * smp_per_batch;
+    uint32_t capacity = pix_per_batch * smp_per_batch;
+    if (keep_capacity && c->wave.capacity >= capacity && c->wave_lights == s.n_lights) {
+        capacity = c->wave.capacity; // (also the stride of the per-light planes and material segments: used as such below)
+    }
     if (int rc = ensure_wave(c, capacity); rc != SPCU_OK) return rc;
 
     const uint32_t n_lights    = s.n_lights;
@@ -337,7 +342,6 @@ int render_impl(spcu_ctx* c, const spcu_partition* part, float* d_rgb_sum, float
 
     auto*          d_counters = c->counters.as<unsigned long long>();
     TraceCounters* d_cnt      = c->options[SPCU_OPT_COUNT_NODES] ? reinterpret_cast<TraceCounters*>(d_counters + kCounterBlock) : nullptr;
-    const uint32_t* d_pix_list = c->pix_list.as<uint32_t>();
     StageTimer      timer{ c, c->options[SPCU_OPT_STAGE_TIMING] != 0, st };
     uint64_t        launches = 0;
 
@@ -398,7 +402,7 @@ int render_impl(spcu_ctx* c, const spcu_partition* part, float* d_rgb_sum, float
 
             uint32_t* n_cur = new_count();
             timer.begin(kStRaygen);
-            launch_raygen(L, s, lane.wave, d_pix_list + pb, np, part->sample_begin + sb, ns, q[kQCur], n_cur, d_counters);
+            launch_raygen(L, s, lane.wave, d_pix_list + pb, np, sample_begin + sb, ns, q[kQCur], n_cur, d_counters);
             timer.end();
             ++launches;
 
@@ -511,6 +515,113 @@ int render_impl(spcu_ctx* c, const spcu_partition* part, float* d_rgb_sum, float
     return SPCU_OK;
 }
 
+int render_impl(spcu_ctx* c, const spcu_partition* part, float* d_rgb_sum, float* d_lum_sumsq, spcu_stats* stats,
+                cudaStream_t caller_stream, bool have_caller_stream)
+{
+    cudaStream_t st = nullptr;
+    if (int rc = prepare_render(c, part, d_rgb_sum, caller_stream, have_caller_stream, st); rc != SPCU_OK) return rc;
+    const uint32_t n_pix     = c->pix_list_n;
+    const uint32_t n_samples = part->sample_end - part->sample_begin;
+    if (stats) {
+        std::memset(stats, 0, sizeof *stats);
+    }
+    if (n_pix == 0 || n_samples == 0) {
+        return SPCU_OK;
+    }
+    return render_batches(c, part, c->pix_list.as<uint32_t>(), n_pix, part->sample_begin, n_samples, d_rgb_sum, d_lum_sumsq, stats,
+                          st, false);
+}
+
+// spcu_render_adaptive(_device): the pass loop over shrinking pixel lists (schedule and stopping test: include/spcu.h).  Pass 0
+// renders the partition's own list (c->pix_list, read only); after it the active pixels ping-pong between c->ad_list[0/1].
+int adaptive_impl(spcu_ctx* c, const spcu_partition* part, const spcu_adaptive* ad, float* d_rgb_sum, float* d_lum_sumsq,
+                  uint32_t* d_spp_map, uint32_t* n_passes, spcu_stats* stats, cudaStream_t caller_stream, bool have_caller_stream)
+{
+    if (int rc = need_scene(c); rc != SPCU_OK) return rc;
+    if (!ad || !d_spp_map) {
+        return fail(c, SPCU_ERR_INVALID, "adaptive parameters or spp map is NULL");
+    }
+    if (ad->min_spp < 2 || ad->pass_spp < 1 || !std::isfinite(ad->rel_error) || !(ad->rel_error >= 0.0f) ||
+        !std::isfinite(ad->abs_floor) || !(ad->abs_floor >= 0.0f)) {
+        return fail(c, SPCU_ERR_INVALID, "bad adaptive parameters: min_spp %u (>= 2), pass_spp %u (>= 1), rel_error %g, abs_floor %g "
+                    "(finite, >= 0)", ad->min_spp, ad->pass_spp, ad->rel_error, ad->abs_floor);
+    }
+    if (part && part->sample_begin != 0) {
+        return fail(c, SPCU_ERR_INVALID, "adaptive rendering starts at sample 0 (sample_begin %u)", part->sample_begin);
+    }
+    cudaStream_t st = nullptr;
+    if (int rc = prepare_render(c, part, d_rgb_sum, caller_stream, have_caller_stream, st); rc != SPCU_OK) return rc;
+
+    const size_t n_pixels = static_cast<size_t>(c->ds.width) * c->ds.height;
+    float*       d_sq     = d_lum_sumsq;
+    if (!d_sq) { // the stopping test needs the sums of squares
+        CK(c, c->ad_sq.reserve(n_pixels * sizeof(float)));
+        d_sq = c->ad_sq.as<float>();
+    }
+    for (auto& e : c->ad_ev) {
+        if (!e) CK(c, cudaEventCreate(&e));
+    }
+    CK(c, cudaEventRecord(c->ad_ev[0], st));
+    CK(c, cudaMemsetAsync(d_rgb_sum, 0, n_pixels * 3 * sizeof(float), st));
+    CK(c, cudaMemsetAsync(d_sq, 0, n_pixels * sizeof(float), st));
+    CK(c, cudaMemsetAsync(d_spp_map, 0, n_pixels * sizeof(uint32_t), st));
+    spcu_stats total{};
+    uint32_t   passes = 0;
+    const uint32_t  budget = part->sample_end;
+    const uint32_t* list   = c->pix_list.as<uint32_t>();
+    uint32_t        n      = c->pix_list_n;
+    if (n > 0 && budget > 0) {
+        for (auto& l : c->ad_list) {
+            CK(c, l.reserve(static_cast<size_t>(n) * sizeof(uint32_t)));
+        }
+        CK(c, c->ad_scratch.reserve(sizeof(uint32_t) + adaptive_scratch_bytes(n))); // active count, then the compaction's scratch
+        uint32_t* d_n_next = c->ad_scratch.as<uint32_t>();
+        uint32_t  begin = 0, end = std::min(ad->min_spp, budget);
+        for (;;) {
+            spcu_stats ps{}; // (read back after every pass: the fault counter is checked there)
+            if (int rc = render_batches(c, part, list, n, begin, end - begin, d_rgb_sum, d_sq, &ps, st, true); rc != SPCU_OK) return rc;
+            ++passes;
+            total.paths += ps.paths;
+            total.rays_closest += ps.rays_closest;
+            total.rays_any += ps.rays_any;
+            total.rays_lights += ps.rays_lights;
+            total.nodes_visited += ps.nodes_visited;
+            total.prims_tested += ps.prims_tested;
+            total.xf_prims_tested += ps.xf_prims_tested;
+            total.shade_calls += ps.shade_calls;
+            total.kernel_launches += ps.kernel_launches;
+            total.trace_ms += ps.trace_ms;
+            total.shade_ms += ps.shade_ms;
+            if (end >= budget) {
+                break;
+            }
+            uint32_t* next = c->ad_list[passes & 1u].as<uint32_t>(); // never the list being read (pass 0 reads c->pix_list)
+            CK(c, launch_adaptive_compact(list, n, d_rgb_sum, d_sq, end, ad->rel_error, ad->abs_floor, d_spp_map, next, d_n_next + 1,
+                                          d_n_next, st));
+            total.kernel_launches += 3;
+            CK(c, cudaMemcpyAsync(&n, d_n_next, sizeof n, cudaMemcpyDeviceToHost, st));
+            CK(c, cudaStreamSynchronize(st)); // the next pass's batches are shaped by the number of active pixels
+            list = next;
+            if (n == 0) {
+                break;
+            }
+            begin = end;
+            end   = std::min(end + ad->pass_spp, budget);
+        }
+        CK(c, launch_adaptive_fill(list, n, budget, d_spp_map, st)); // still active when the budget ran out
+    }
+    CK(c, cudaEventRecord(c->ad_ev[1], st));
+    if (stats) {
+        CK(c, cudaEventSynchronize(c->ad_ev[1]));
+        CK(c, cudaEventElapsedTime(&total.device_ms, c->ad_ev[0], c->ad_ev[1]));
+        *stats = total;
+    }
+    if (n_passes) {
+        *n_passes = passes;
+    }
+    return SPCU_OK;
+}
+
 // The host-buffer entry points synchronise anyway: they also read the fault counter (kCntErrors) when no stats were asked
 // for, so a kernel that gave up on a bounded wait fails the call instead of returning a void image.
 int sync_and_check_faults(spcu_ctx* c, bool already_checked)
@@ -536,6 +647,36 @@ int spcu_render_device(spcu_ctx* c, const spcu_partition* part, float* d_rgb_sum
 {
     // stream == NULL means the legacy default stream, as in the CUDA runtime
     return render_impl(c, part, d_rgb_sum, d_lum_sumsq, stats, static_cast<cudaStream_t>(stream), true);
+}
+
+int spcu_render_adaptive_device(spcu_ctx* c, const spcu_partition* part, const spcu_adaptive* ad, float* d_rgb_sum, float* d_lum_sumsq,
+                                uint32_t* d_spp_map, uint32_t* n_passes, spcu_stats* stats, void* stream)
+{
+    return adaptive_impl(c, part, ad, d_rgb_sum, d_lum_sumsq, d_spp_map, n_passes, stats, static_cast<cudaStream_t>(stream), true);
+}
+
+int spcu_render_adaptive(spcu_ctx* c, const spcu_partition* part, const spcu_adaptive* ad, float* rgb_sum, float* lum_sumsq,
+                         uint32_t* spp_map, uint32_t* n_passes, spcu_stats* stats)
+{
+    if (int rc = need_scene(c); rc != SPCU_OK) return rc;
+    if (!rgb_sum || !spp_map) {
+        return fail(c, SPCU_ERR_INVALID, "rgb_sum or spp_map is NULL");
+    }
+    const size_t n_pixels = static_cast<size_t>(c->ds.width) * c->ds.height;
+    CK(c, c->host_rgb.reserve(n_pixels * 3 * sizeof(float)));
+    CK(c, c->host_sq.reserve(n_pixels * sizeof(float)));
+    CK(c, c->ad_spp_map.reserve(n_pixels * sizeof(uint32_t)));
+    if (int rc = adaptive_impl(c, part, ad, c->host_rgb.as<float>(), c->host_sq.as<float>(), c->ad_spp_map.as<uint32_t>(), n_passes,
+                               stats, nullptr, false);
+        rc != SPCU_OK) {
+        return rc;
+    }
+    CK(c, cudaMemcpyAsync(rgb_sum, c->host_rgb.p, n_pixels * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    if (lum_sumsq) {
+        CK(c, cudaMemcpyAsync(lum_sumsq, c->host_sq.p, n_pixels * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    }
+    CK(c, cudaMemcpyAsync(spp_map, c->ad_spp_map.p, n_pixels * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+    return sync_and_check_faults(c, true); // (every pass's fault counter has been read)
 }
 
 int spcu_render(spcu_ctx* c, const spcu_partition* part, float* rgb_sum, float* lum_sumsq, spcu_stats* stats)
@@ -628,7 +769,8 @@ int spcu_render_image(spcu_ctx* c, const spcu_partition* part, uint32_t format, 
     CK(c, cudaMemsetAsync(c->host_rgb.p, 0, n_pixels * 3 * sizeof(float), c->stream));
     if (int rc = render_impl(c, part, c->host_rgb.as<float>(), nullptr, stats, nullptr, false); rc != SPCU_OK) return rc;
     if (int rc = sync_and_check_faults(c, stats != nullptr); rc != SPCU_OK) return rc;
-    return pack_device_image(c, c->host_rgb.as<float>(), c->ds.width, c->ds.height, part->sample_end - part->sample_begin, format, out);
+    return pack_device_image(c, c->host_rgb.as<float>(), nullptr, c->ds.width, c->ds.height, part->sample_end - part->sample_begin, format,
+                             out);
 }
 
 // Ray batches through the renderer's own traversal stages: the kernels a frame runs (begin + persistent walk, lane refill,

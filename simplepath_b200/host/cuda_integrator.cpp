@@ -4,6 +4,7 @@
 
 #include "base/Scene.h"
 
+#include <algorithm>
 #include <chrono>
 #include <cmath>
 #include <cstdlib>
@@ -126,7 +127,8 @@ CudaIntegrator::CudaIntegrator(Options options)
 CudaIntegrator::~CudaIntegrator() = default;
 
 // Sum of radiance samples per pixel, row major W*H*3.
-void CudaIntegrator::render_sum(const Scene& scene, unsigned spp, std::vector<float>& rgb_sum) const
+void CudaIntegrator::render_sum(const Scene& scene, unsigned spp, std::vector<float>& rgb_sum, std::vector<std::uint32_t>* spp_map,
+                                float rel_error) const
 {
     if (m_devices.empty()) {
         for (int i = 0; i < m_options.n_devices; ++i) {
@@ -220,6 +222,24 @@ void CudaIntegrator::render_sum(const Scene& scene, unsigned spp, std::vector<fl
 
     const auto           n_dev = static_cast<std::uint32_t>(m_devices.size());
     const std::uint32_t  code  = integrator_code(m_options.inner);
+    if (spp_map) { // (one device: render_frame checks)
+        // passes of 16 samples (fewer when the budget is smaller); the first test needs at least 2 samples
+        const std::uint32_t  k = std::min(16u, spp);
+        const spcu_adaptive  ad{ std::max(2u, k), k, rel_error, 0.0f };
+        const spcu_partition part{ 0u, 1u, 0u, spp, spp, code, m_options.seed };
+        spp_map->resize(n / 3u);
+        std::uint32_t passes = 0;
+        m_devices[0]->check(spcu_render_adaptive(m_devices[0]->ctx, &part, &ad, rgb_sum.data(), nullptr, spp_map->data(), &passes, &m_stats),
+                            "spcu_render_adaptive");
+        std::uint64_t early = 0;
+        for (const std::uint32_t c : *spp_map) {
+            early += c < spp ? 1u : 0u;
+        }
+        const double pixels = static_cast<double>(spp_map->size());
+        std::fprintf(stderr, "CudaIntegrator: adaptive sampling to %g: %u passes, mean %.2f spp of %u, %.1f %% of pixels stopped early\n",
+                     rel_error, passes, static_cast<double>(m_stats.paths) / pixels, spp, 100.0 * static_cast<double>(early) / pixels);
+        return;
+    }
     std::vector<spcu_stats> stats(n_dev);
     // Tile-interleaved partition (base/TileScheduler.h:66-82 order): device k renders tiles t with t % n == k.  Disjoint
     // pixels, so the sum over devices is exact (every other device contributes +0): the per-device accumulators are summed on
@@ -246,16 +266,29 @@ bool CudaIntegrator::render_frame(const Scene& scene, unsigned spp, Image& image
     if (spp == 0) {
         throw std::runtime_error("CudaIntegrator: samples per pixel must be >= 1");
     }
-    std::vector<float> sum;
-    render_sum(scene, spp, sum);
+    std::vector<float>         sum;
+    std::vector<std::uint32_t> counts; // SPCU_ADAPTIVE=<rel_error>: --samples is the budget, each pixel has its own count
+    if (const char* adaptive = std::getenv("SPCU_ADAPTIVE"); adaptive && *adaptive) {
+        char*       end = nullptr;
+        const float rel = std::strtof(adaptive, &end);
+        if (end == adaptive || *end != '\0') {
+            throw std::runtime_error(std::string("CudaIntegrator: SPCU_ADAPTIVE must be a relative standard error, not '") + adaptive + "'");
+        }
+        if (m_options.n_devices > 1) {
+            throw std::runtime_error("CudaIntegrator: SPCU_ADAPTIVE renders on one device; unset SPCU_DEVICES or set it to 1");
+        }
+        render_sum(scene, spp, sum, &counts, rel);
+    } else {
+        render_sum(scene, spp, sum);
+    }
     const auto  w   = static_cast<std::size_t>(scene.image_width);
     const auto  h   = static_cast<std::size_t>(scene.image_height);
-    const float div = static_cast<float>(spp);
     for (std::size_t y = 0; y < h; ++y) {
         for (std::size_t x = 0; x < w; ++x) {
             const float* p = &sum[(y * w + x) * 3u];
             // image(p) += L ... ; image(p) /= num_pixel_samples (main.cpp:100-102)
-            RGB c{ p[0], p[1], p[2] };
+            RGB         c{ p[0], p[1], p[2] };
+            const float div = counts.empty() ? static_cast<float>(spp) : static_cast<float>(counts[y * w + x]);
             c /= div;
             image(x, y) = c;
         }

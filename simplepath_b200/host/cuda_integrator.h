@@ -53,7 +53,10 @@ public:
 private:
     RGB integrate_impl(const Ray&, const Scene& scene, MemoryArena&, Sampler&, const Point2& pixel_coords) const override;
 
-    void render_sum(const Scene& scene, unsigned spp, std::vector<float>& rgb_sum) const;
+    // spp_map != NULL: adaptive sampling (spcu_render_adaptive, one device) to the standard error `rel_error`, spp the budget;
+    // *spp_map = the samples each pixel received
+    void render_sum(const Scene& scene, unsigned spp, std::vector<float>& rgb_sum, std::vector<std::uint32_t>* spp_map = nullptr,
+                    float rel_error = 0.0f) const;
 
     struct Device;
     Options                              m_options;
