@@ -12,10 +12,21 @@
 
 namespace spcu {
 
+// Grow-only device allocation that frees itself.
 struct DevBuf
 {
     void*  p     = nullptr;
     size_t bytes = 0;
+
+    DevBuf() = default;
+    DevBuf(const DevBuf&) = delete;
+    DevBuf& operator=(const DevBuf&) = delete;
+    DevBuf(DevBuf&& o) noexcept : p(o.p), bytes(o.bytes)
+    {
+        o.p     = nullptr;
+        o.bytes = 0;
+    }
+    ~DevBuf() { release(); }
 
     cudaError_t reserve(size_t n)
     {
@@ -58,27 +69,20 @@ constexpr uint32_t kMaxMaterialSegments = 15;  // materials beyond share the las
 constexpr int      kMaxBatchLanes  = 8;        // SPCU_OPT_BATCH_LANES
 constexpr int      kDefaultBatchLanes = 4;
 
-// Wavefront state of one batch in flight beyond the first (whose state lives in the context itself): SPCU_OPT_BATCH_LANES
+// Wavefront state of one batch in flight (SPCU_OPT_BATCH_LANES): records, queues, queue counts and the material-sorted queue,
+// carved from one allocation and laid out again for every call's batch capacity (spcu_render.cu lay_out_lane).
+// Lane 0 runs on the call's stream (`stream` stays NULL); lanes 1..k on their own.
 struct WaveLane
 {
-    DWave               wave{};
-    std::vector<DevBuf> wave_bufs;
-    DevBuf              queues[kNumQueues];
-    DevBuf              queue_counts;
-    DevBuf              sorted_queue;
-    uint32_t            wave_lights = 0;
-    cudaStream_t        stream   = nullptr;
-    cudaEvent_t         resolved = nullptr; // recorded after each of the lane's resolve kernels
+    DevBuf       mem;
+    DWave        wave{};
+    uint32_t*    queues[kNumQueues] = {};
+    uint32_t*    queue_counts       = nullptr; // uint32[kMaxQueueCounts]
+    uint32_t*    sorted             = nullptr; // [n_segments][wave.capacity]: the hand-over between extend and shade
+    cudaStream_t stream   = nullptr;
+    cudaEvent_t  resolved = nullptr; // recorded after each of the lane's resolve kernels
 
-    void release()
-    {
-        for (auto& b : wave_bufs) b.release();
-        wave_bufs.clear();
-        for (auto& q : queues) q.release();
-        queue_counts.release();
-        sorted_queue.release();
-        wave.capacity = 0;
-    }
+    void release() { mem.release(); }
 };
 
 } // namespace spcu
@@ -111,10 +115,7 @@ struct spcu_ctx
 
     // wavefront
     uint64_t                  wavefront_size = 0; // 0 = default
-    spcu::DWave               wave{};
-    std::vector<spcu::DevBuf> wave_bufs;
-    spcu::DevBuf              queues[spcu::kNumQueues];
-    spcu::DevBuf              queue_counts; // uint32[kMaxQueueCounts]
+    std::vector<spcu::WaveLane> lanes = std::vector<spcu::WaveLane>(1); // lanes[0]: the context's own
     spcu::DevBuf              counters;     // unsigned long long[kNumCounters] followed by TraceCounters
     spcu::DevBuf              pix_list;
     uint32_t                  pix_list_offset = ~0u, pix_list_stride = 0, pix_list_n = 0;
@@ -128,12 +129,8 @@ struct spcu_ctx
     cudaEvent_t               stage_ev[2] = { nullptr, nullptr };
     bool                      stage_busy[2] = { false, false };
     spcu::DevBuf              path_radiance;     // float4 per slot of a batch (SPCU_PIPELINE_PATHS)
-    spcu::DevBuf              sorted_queue;      // material-sorted hand-over between extend and shade
     uint32_t                  n_materials = 0;
     int                       features    = 0; // feature set of the uploaded scene (features.h)
-    uint32_t                  wave_lights = 0; // light planes the wavefront buffers were sized for
-    cudaEvent_t               resolved = nullptr;       // lane 0's "resolve done" event
-    std::vector<spcu::WaveLane> extra_lanes;            // batches in flight beyond the first (SPCU_OPT_BATCH_LANES)
 
     uint32_t                 options[SPCU_OPT_COUNT_] = {};
     std::vector<cudaEvent_t> stage_events; // pairs, when SPCU_OPT_STAGE_TIMING is on

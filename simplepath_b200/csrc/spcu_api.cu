@@ -262,25 +262,11 @@ void spcu_destroy(spcu_ctx* c)
     cudaSetDevice(c->device);
     cudaStreamSynchronize(c->stream);
     spcu_comm_destroy(c);
-    for (DevBuf* b : { &c->geom_wide, &c->geom_big, &c->geom_nodes, &c->geom_prims, &c->geom_shade, &c->geom_meta, &c->light_nodes, &c->lights,
-                       &c->light_order, &c->materials, &c->bxdfs, &c->pool, &c->jitter, &c->q_rays, &c->q_out, &c->q_aux,
-                       &c->q_cnt, &c->queue_counts, &c->counters, &c->pix_list, &c->host_rgb, &c->host_sq, &c->path_radiance, &c->sorted_queue, &c->packed,
-                       &c->ad_list[0], &c->ad_list[1], &c->ad_spp_map, &c->ad_sq, &c->ad_scratch }) {
-        b->release();
-    }
-    for (auto& b : c->wave_bufs) {
-        b.release();
-    }
-    for (auto& q : c->queues) {
-        q.release();
-    }
-    for (auto& lane : c->extra_lanes) {
+    for (auto& lane : c->lanes) {
         if (lane.stream) cudaStreamSynchronize(lane.stream);
-        lane.release();
         if (lane.resolved) cudaEventDestroy(lane.resolved);
         if (lane.stream) cudaStreamDestroy(lane.stream);
     }
-    if (c->resolved) cudaEventDestroy(c->resolved);
     for (auto e : c->ad_ev) {
         if (e) cudaEventDestroy(e);
     }
@@ -296,7 +282,7 @@ void spcu_destroy(spcu_ctx* c)
     cudaEventDestroy(c->ev0);
     cudaEventDestroy(c->ev1);
     cudaStreamDestroy(c->stream);
-    delete c;
+    delete c; // (its device buffers free themselves)
 }
 
 int spcu_set_option(spcu_ctx* c, uint32_t option, uint32_t value)

@@ -17,86 +17,96 @@ using namespace spcu;
 namespace {
 
 enum Queue { kQCur = 0, kQNext, kQLive, kQShadow, kQLit, kQMis, kQWalk };
-constexpr int kCounterBlock = kNumCounters + kNumStages; // + per-stage item counters
+constexpr int    kCounterBlock = kNumCounters + kNumStages; // + per-stage item counters
+constexpr size_t kCounterBytes = kCounterBlock * sizeof(unsigned long long) + sizeof(TraceCounters);
 
 const char* const kStageNames[kNumStages] = { "raygen",   "extend",    "shade",     "nee_light",         "shadow",           "nee_bsdf",
                                               "mis_trace", "nee_mis_accumulate", "direct_accumulate", "advance", "resolve", "paths" };
 inline bool stage_traverses(int st) { return st == kStExtend || st == kStShadow || st == kStMisTrace; }
 
-template <typename T>
-int wave_array(spcu_ctx* c, std::vector<DevBuf>& bufs, T*& ptr, size_t n)
+int queue_fault(spcu_ctx* c, unsigned long long n_faults)
 {
-    bufs.emplace_back();
-    CK(c, bufs.back().reserve(std::max<size_t>(n, 1) * sizeof(T)));
-    ptr = bufs.back().as<T>();
+    return fail(c, SPCU_ERR_INTERNAL, "%llu kernel(s) gave up on a bounded wait (queue protocol fault); the image is void", n_faults);
+}
+
+// segments of the material-sorted queue: one per material (materials beyond the last share it) + the miss segment
+uint32_t material_segments(const spcu_ctx* c) { return std::min<uint32_t>(c->n_materials, kMaxMaterialSegments) + 1u; }
+
+// The lane's wavefront state for batches of `capacity` slots (also the stride of the per-light planes and material segments),
+// every array at a 256-byte-aligned offset of the lane's one allocation, as cudaMalloc would place it.  The allocation only
+// grows: a smaller batch reuses it with its own stride.
+int lay_out_lane(spcu_ctx* c, WaveLane& lane, uint32_t capacity, uint32_t n_segments)
+{
+    const size_t planes = std::max(1u, c->ds.n_lights); // light records and the shadow queue: one plane per light
+    auto         carve  = [&](uintptr_t base) {
+        size_t off  = 0;
+        auto   take = [&](auto*& ptr, size_t n) {
+            ptr = reinterpret_cast<std::remove_reference_t<decltype(ptr)>>(base + off);
+            off += (n * sizeof *ptr + 255) & ~size_t(255);
+        };
+        DWave& w = lane.wave;
+        take(w.path, capacity);
+        take(w.ray, capacity);
+        take(w.vertex, capacity);
+        take(w.extend, capacity);
+        take(w.s0, capacity);
+        take(w.light, capacity * planes);
+        take(w.mis, capacity);
+        take(w.occluded, capacity);
+        for (int i = 0; i < kNumQueues; ++i) {
+            take(lane.queues[i], capacity * (i == kQShadow ? planes : 1u));
+        }
+        take(lane.queue_counts, kMaxQueueCounts);
+        take(lane.sorted, static_cast<size_t>(n_segments) * capacity);
+        return off;
+    };
+    CK(c, lane.mem.reserve(carve(0)));
+    carve(reinterpret_cast<uintptr_t>(lane.mem.p));
+    lane.wave.capacity = capacity;
     return SPCU_OK;
 }
 
-// the wavefront state of one batch in flight: records, queues, queue counters
-int ensure_wave_buffers(spcu_ctx* c, DWave& w, std::vector<DevBuf>& bufs, DevBuf* queues, DevBuf& queue_counts, uint32_t& wave_lights,
-                        uint32_t capacity)
+// Lane k of SPCU_OPT_BATCH_LANES laid out for this call's batches.  Lane 0 must get its memory.  A lane k >= 1 that cannot
+// is not an error: it is released and the render goes on with the lanes before it.
+int ensure_lane(spcu_ctx* c, size_t k, uint32_t capacity, uint32_t n_segments)
 {
-    if (w.capacity == capacity && wave_lights == c->ds.n_lights) {
-        return SPCU_OK; // (capacity is also the stride of the per-light planes, so it must match exactly)
-    }
-    wave_lights = c->ds.n_lights;
-    for (auto& b : bufs) {
-        b.release();
-    }
-    bufs.clear();
-    bufs.reserve(32);
-    w.capacity = 0;
-    int rc;
-#define WAVE(field) \
-    if ((rc = wave_array(c, bufs, w.field, capacity)) != SPCU_OK) return rc
-    WAVE(path);
-    WAVE(ray);
-    WAVE(vertex);
-    WAVE(extend);
-    WAVE(s0);
-    if ((rc = wave_array(c, bufs, w.light, static_cast<size_t>(capacity) * std::max(1u, c->ds.n_lights))) != SPCU_OK) return rc;
-    WAVE(mis);
-    WAVE(occluded);
-#undef WAVE
-    for (int i = 0; i < kNumQueues; ++i) { // the shadow queue has one plane per light
-        const size_t planes = (i == kQShadow) ? std::max(1u, c->ds.n_lights) : 1u;
-        CK(c, queues[i].reserve(static_cast<size_t>(capacity) * planes * sizeof(uint32_t)));
-    }
-    CK(c, queue_counts.reserve(kMaxQueueCounts * sizeof(uint32_t)));
-    w.capacity = capacity;
-    return SPCU_OK;
-}
-
-int ensure_wave(spcu_ctx* c, uint32_t capacity)
-{
-    if (int rc = ensure_wave_buffers(c, c->wave, c->wave_bufs, c->queues, c->queue_counts, c->wave_lights, capacity); rc != SPCU_OK) {
-        return rc;
-    }
-    CK(c, c->counters.reserve(kCounterBlock * sizeof(unsigned long long) + sizeof(TraceCounters)));
-    return SPCU_OK;
-}
-
-// Lane k >= 1 of SPCU_OPT_BATCH_LANES: its own stream, event and wavefront state.  A lane that cannot be allocated is not
-// an error: the render goes on with the lanes it has (the caller shrinks its lane count to what this returns OK for).
-int ensure_extra_lane(spcu_ctx* c, size_t k, uint32_t capacity, size_t sorted_bytes)
-{
-    if (c->extra_lanes.size() <= k) {
-        c->extra_lanes.resize(k + 1);
-    }
-    WaveLane& lane = c->extra_lanes[k];
-    if (!lane.stream) {
+    WaveLane& lane = c->lanes[k];
+    if (k > 0 && !lane.stream) {
         CK(c, cudaStreamCreateWithFlags(&lane.stream, cudaStreamNonBlocking));
+    }
+    if (!lane.resolved) {
         CK(c, cudaEventCreateWithFlags(&lane.resolved, cudaEventDisableTiming));
     }
-    int rc = ensure_wave_buffers(c, lane.wave, lane.wave_bufs, lane.queues, lane.queue_counts, lane.wave_lights, capacity);
-    if (rc == SPCU_OK && lane.sorted_queue.reserve(sorted_bytes) != cudaSuccess) {
-        rc = SPCU_ERR_CUDA;
-    }
-    if (rc != SPCU_OK) {
+    const int rc = lay_out_lane(c, lane, capacity, n_segments);
+    if (rc != SPCU_OK && k > 0) {
         cudaGetLastError(); // (out of memory is sticky-free; clear it)
         lane.release();
     }
     return rc;
+}
+
+// Batch shape for `target` slots: the whole pixel list x as many samples as fit, or a slice of the pixel list x one sample.
+struct BatchShape
+{
+    uint32_t pix, smp;
+};
+
+BatchShape batch_shape(uint32_t n_pix, uint32_t n_samples, uint64_t target)
+{
+    if (n_pix > target) {
+        return { static_cast<uint32_t>(target), 1 };
+    }
+    return { n_pix, static_cast<uint32_t>(std::min<uint64_t>(n_samples, std::max<uint64_t>(1, target / n_pix))) };
+}
+
+// The wavefront state, queues and counters are context-owned scratch: work on ANOTHER stream than the previous render's must
+// not start before that render has finished with them (ev1 is recorded at the end of every render).
+int wait_for_scratch(spcu_ctx* c, cudaStream_t st)
+{
+    if (c->scratch_in_use && c->scratch_stream != st) {
+        CK(c, cudaStreamWaitEvent(st, c->ev1, 0));
+    }
+    return SPCU_OK;
 }
 
 int ensure_pixel_list(spcu_ctx* c, const spcu_partition& part)
@@ -182,8 +192,7 @@ int read_back_stats(spcu_ctx* c, cudaStream_t st, spcu_stats* stats, uint64_t la
     stats->xf_prims_tested = tc.xf;
     stats->kernel_launches = launches;
     if (h[kCntErrors]) {
-        return fail(c, SPCU_ERR_INTERNAL, "%llu kernel(s) gave up on a bounded wait (queue protocol fault); the image is void",
-                    h[kCntErrors]);
+        return queue_fault(c, h[kCntErrors]);
     }
     CK(c, cudaEventElapsedTime(&stats->device_ms, c->ev0, c->ev1));
     for (int i = 0; i < kNumStages; ++i) {
@@ -195,61 +204,6 @@ int read_back_stats(spcu_ctx* c, cudaStream_t st, spcu_stats* stats, uint64_t la
         r.traverses = stage_traverses(i) ? 1u : 0u;
     }
     timer.collect(stats->trace_ms, stats->shade_ms);
-    return SPCU_OK;
-}
-
-// SPCU_PIPELINE_PATHS: one persistent kernel per batch (path_kernels.cu) + resolve.
-int render_paths(spcu_ctx* c, const spcu_partition* part, const uint32_t* d_pix_list, uint32_t n_pix, uint32_t sample_begin,
-                 uint32_t n_samples, float* d_rgb_sum, float* d_lum_sumsq, spcu_stats* stats, cudaStream_t st, bool sm_local)
-{
-    const DScene& s = c->ds;
-    // batch = whole pixel list x as many samples as fit in the radiance buffer (16 B per path)
-    const uint64_t target = c->wavefront_size ? c->wavefront_size : (1ull << 27);
-    uint32_t       pix_per_batch, smp_per_batch;
-    if (n_pix <= target) {
-        pix_per_batch = n_pix;
-        smp_per_batch = static_cast<uint32_t>(std::min<uint64_t>(n_samples, std::max<uint64_t>(1, target / n_pix)));
-    } else {
-        pix_per_batch = static_cast<uint32_t>(target);
-        smp_per_batch = 1;
-    }
-    const size_t capacity = static_cast<size_t>(pix_per_batch) * smp_per_batch;
-    CK(c, c->path_radiance.reserve(capacity * sizeof(float4)));
-    CK(c, c->counters.reserve(kCounterBlock * sizeof(unsigned long long) + sizeof(TraceCounters)));
-    auto*          d_counters = c->counters.as<unsigned long long>();
-    TraceCounters* d_cnt = c->options[SPCU_OPT_COUNT_NODES] ? reinterpret_cast<TraceCounters*>(d_counters + kCounterBlock) : nullptr;
-    const Launch    L{ c->sm_count, st, c->features };
-    StageTimer      timer{ c, c->options[SPCU_OPT_STAGE_TIMING] != 0, st };
-    uint64_t        launches = 0;
-    float4*         d_radiance = c->path_radiance.as<float4>();
-
-    CK(c, cudaMemsetAsync(d_counters, 0, kCounterBlock * sizeof(unsigned long long) + sizeof(TraceCounters), st));
-    CK(c, cudaEventRecord(c->ev0, st));
-    for (uint32_t pb = 0; pb < n_pix; pb += pix_per_batch) {
-        const uint32_t np = std::min(pix_per_batch, n_pix - pb);
-        for (uint32_t sb = 0; sb < n_samples; sb += smp_per_batch) {
-            const uint32_t ns = std::min(smp_per_batch, n_samples - sb);
-            timer.begin(kStPaths);
-            if (sm_local) {
-                CK(c, launch_smwave(L, s, d_pix_list + pb, np, sample_begin + sb, ns, part->seed, part->integrator,
-                                    d_radiance, d_counters, d_cnt));
-            } else {
-                launch_paths(L, s, d_pix_list + pb, np, sample_begin + sb, ns, part->seed, part->integrator, d_radiance,
-                             d_counters, d_cnt);
-            }
-            timer.end();
-            timer.begin(kStResolve);
-            launch_resolve(L, d_radiance, 1, d_pix_list + pb, np, ns, d_rgb_sum, d_lum_sumsq, d_counters);
-            timer.end();
-            launches += 2;
-            CK(c, cudaGetLastError());
-        }
-    }
-    CK(c, cudaEventRecord(c->ev1, st));
-    if (stats) {
-        if (int rc = read_back_stats(c, st, stats, launches, timer); rc != SPCU_OK) return rc;
-        c->stage_report[kStPaths].items = stats->paths;
-    }
     return SPCU_OK;
 }
 
@@ -285,21 +239,17 @@ int prepare_render(spcu_ctx* c, const spcu_partition* part, const float* d_rgb_s
     }
     // The caller's stream (spcu_render_device) orders this call after the caller's earlier work on that stream.
     st = have_caller_stream ? caller_stream : c->stream;
-    // The wavefront state, queues and counters are context-owned scratch: a render on ANOTHER stream than the previous one
-    // must not start before that one has finished with them (ev1 is recorded at the end of every render).
-    if (c->scratch_in_use && c->scratch_stream != st) {
-        CK(c, cudaStreamWaitEvent(st, c->ev1, 0));
-    }
+    if (int rc = wait_for_scratch(c, st); rc != SPCU_OK) return rc;
     c->scratch_in_use = true;
     c->scratch_stream = st;
     return ensure_pixel_list(c, *part);
 }
 
-// The batch loop: samples [sample_begin, sample_begin + n_samples) of the n_pix pixels of d_pix_list (n_pix, n_samples > 0),
-// added to the accumulators in sample order.  keep_capacity: reuse wavefront buffers that are already large enough instead of
-// re-sizing them to this call's batch (the adaptive passes shrink from one pass to the next).
+// The batch loop of every pipeline: samples [sample_begin, sample_begin + n_samples) of the n_pix pixels of d_pix_list (n_pix,
+// n_samples > 0), added to the accumulators in sample order.  One batch is the persistent path / SM-local kernel on the call's
+// stream, or the queue wavefront's stage chain on lane `batch % n_lanes`; then its resolve.
 int render_batches(spcu_ctx* c, const spcu_partition* part, const uint32_t* d_pix_list, uint32_t n_pix, uint32_t sample_begin,
-                   uint32_t n_samples, float* d_rgb_sum, float* d_lum_sumsq, spcu_stats* stats, cudaStream_t st, bool keep_capacity)
+                   uint32_t n_samples, float* d_rgb_sum, float* d_lum_sumsq, spcu_stats* stats, cudaStream_t st)
 {
     const DScene&  s        = c->ds;
     const uint32_t pipeline = resolve_pipeline(c);
@@ -307,210 +257,199 @@ int render_batches(spcu_ctx* c, const spcu_partition* part, const uint32_t* d_pi
         return fail(c, SPCU_ERR_INVALID, "SPCU_PIPELINE_SMWAVE: max_depth %u / %u lights exceed its packed path flags",
                     s.max_depth, s.n_lights);
     }
-    if (pipeline == SPCU_PIPELINE_PATHS || pipeline == SPCU_PIPELINE_SMWAVE) {
-        return render_paths(c, part, d_pix_list, n_pix, sample_begin, n_samples, d_rgb_sum, d_lum_sumsq, stats, st,
-                            pipeline == SPCU_PIPELINE_SMWAVE);
-    }
-
-    // batch shape: whole pixel list x as many samples as fit, or a slice of the pixel list x one sample
-    const uint64_t target = c->wavefront_size ? c->wavefront_size : (1ull << 24);
-    uint32_t       pix_per_batch, smp_per_batch;
-    if (n_pix <= target) {
-        pix_per_batch = n_pix;
-        smp_per_batch = static_cast<uint32_t>(std::min<uint64_t>(n_samples, std::max<uint64_t>(1, target / n_pix)));
-    } else {
-        pix_per_batch = static_cast<uint32_t>(target);
-        smp_per_batch = 1;
-    }
-    uint32_t capacity = pix_per_batch * smp_per_batch;
-    if (keep_capacity && c->wave.capacity >= capacity && c->wave_lights == s.n_lights) {
-        capacity = c->wave.capacity; // (also the stride of the per-light planes and material segments: used as such below)
-    }
-    if (int rc = ensure_wave(c, capacity); rc != SPCU_OK) return rc;
+    const bool wavefront = pipeline == SPCU_PIPELINE_WAVEFRONT;
+    // the persistent kernels keep 16 B of radiance per slot, the queue wavefront its whole state
+    const BatchShape shape    = batch_shape(n_pix, n_samples, c->wavefront_size ? c->wavefront_size : wavefront ? 1ull << 24 : 1ull << 27);
+    const uint32_t   capacity = shape.pix * shape.smp;
+    CK(c, c->counters.reserve(kCounterBytes));
+    auto*          d_counters = c->counters.as<unsigned long long>();
+    TraceCounters* d_cnt      = c->options[SPCU_OPT_COUNT_NODES] ? reinterpret_cast<TraceCounters*>(d_counters + kCounterBlock) : nullptr;
+    StageTimer     timer{ c, c->options[SPCU_OPT_STAGE_TIMING] != 0, st };
+    uint64_t       launches = 0;
 
     const uint32_t n_lights    = s.n_lights;
     const uint32_t max_depth   = part->integrator == SPCU_INTEGRATOR_DIRECT_LIGHTING ? std::min(1u, s.max_depth) : s.max_depth;
     const bool     nee         = part->integrator == SPCU_INTEGRATOR_ITERATIVE_RRNEE;
     const bool     whitted     = part->integrator == SPCU_INTEGRATOR_WHITTED;
     const bool     direct      = part->integrator == SPCU_INTEGRATOR_DIRECT_LIGHTING || whitted; // per-light direct term
-    const uint32_t n_segments  = std::min<uint32_t>(c->n_materials, kMaxMaterialSegments) + 1u; // + the miss segment
+    const uint32_t n_segments  = material_segments(c);
     const uint32_t counts_need = 1 + max_depth * (4 + 7 * n_lights + n_segments);
-    CK(c, c->sorted_queue.reserve(static_cast<size_t>(n_segments) * capacity * sizeof(uint32_t)));
-    if (counts_need > static_cast<uint32_t>(kMaxQueueCounts)) {
-        return fail(c, SPCU_ERR_LIMIT, "max_depth x lights needs %u queue counters (limit %d)", counts_need, kMaxQueueCounts);
-    }
-
-    auto*          d_counters = c->counters.as<unsigned long long>();
-    TraceCounters* d_cnt      = c->options[SPCU_OPT_COUNT_NODES] ? reinterpret_cast<TraceCounters*>(d_counters + kCounterBlock) : nullptr;
-    StageTimer      timer{ c, c->options[SPCU_OPT_STAGE_TIMING] != 0, st };
-    uint64_t        launches = 0;
-
-    // ---- batches in flight (SPCU_OPT_BATCH_LANES): lane 0 = the context's own wavefront state on the call's stream ----------
-    const uint64_t n_batches = static_cast<uint64_t>((n_pix + pix_per_batch - 1) / pix_per_batch) * ((n_samples + smp_per_batch - 1) / smp_per_batch);
-    uint32_t       want_lanes = c->options[SPCU_OPT_BATCH_LANES] ? c->options[SPCU_OPT_BATCH_LANES] : kDefaultBatchLanes;
-    if (timer.on || d_cnt) {
-        want_lanes = 1; // per-launch events and the node counters describe one batch at a time
-    }
-    want_lanes = static_cast<uint32_t>(std::min<uint64_t>({ want_lanes, kMaxBatchLanes, n_batches }));
-    struct LaneView
-    {
-        DWave        wave;
-        uint32_t*    q[kNumQueues];
-        uint32_t*    d_counts;
-        uint32_t*    sorted;
-        cudaStream_t st;
-        cudaEvent_t  resolved;
-    };
-    std::vector<LaneView> lanes;
-    if (!c->resolved) {
-        CK(c, cudaEventCreateWithFlags(&c->resolved, cudaEventDisableTiming));
-    }
-    {
-        LaneView v{ c->wave, {}, c->queue_counts.as<uint32_t>(), c->sorted_queue.as<uint32_t>(), st, c->resolved };
-        for (int i = 0; i < kNumQueues; ++i) v.q[i] = c->queues[i].as<uint32_t>();
-        lanes.push_back(v);
-    }
-    for (uint32_t k = 1; k < want_lanes; ++k) {
-        if (ensure_extra_lane(c, k - 1, capacity, static_cast<size_t>(n_segments) * capacity * sizeof(uint32_t)) != SPCU_OK) {
-            break; // not enough memory for another lane: render with the ones we have
+    // ---- batches in flight (SPCU_OPT_BATCH_LANES) of the queue wavefront: lane 0 on the call's stream -----------------------
+    uint32_t n_lanes = 1;
+    if (wavefront) {
+        if (counts_need > static_cast<uint32_t>(kMaxQueueCounts)) {
+            return fail(c, SPCU_ERR_LIMIT, "max_depth x lights needs %u queue counters (limit %d)", counts_need, kMaxQueueCounts);
         }
-        WaveLane& l = c->extra_lanes[k - 1];
-        LaneView  v{ l.wave, {}, l.queue_counts.as<uint32_t>(), l.sorted_queue.as<uint32_t>(), l.stream, l.resolved };
-        for (int i = 0; i < kNumQueues; ++i) v.q[i] = l.queues[i].as<uint32_t>();
-        lanes.push_back(v);
+        const uint64_t n_batches  = static_cast<uint64_t>((n_pix + shape.pix - 1) / shape.pix) * ((n_samples + shape.smp - 1) / shape.smp);
+        uint32_t       want_lanes = c->options[SPCU_OPT_BATCH_LANES] ? c->options[SPCU_OPT_BATCH_LANES] : kDefaultBatchLanes;
+        if (timer.on || d_cnt) {
+            want_lanes = 1; // per-launch events and the node counters describe one batch at a time
+        }
+        want_lanes = static_cast<uint32_t>(std::min<uint64_t>({ want_lanes, kMaxBatchLanes, n_batches }));
+        if (c->lanes.size() < want_lanes) {
+            c->lanes.resize(want_lanes);
+        }
+        if (int rc = ensure_lane(c, 0, capacity, n_segments); rc != SPCU_OK) return rc;
+        while (n_lanes < want_lanes && ensure_lane(c, n_lanes, capacity, n_segments) == SPCU_OK) {
+            ++n_lanes; // (not enough memory for another lane: render with the ones we have)
+        }
+    } else {
+        CK(c, c->path_radiance.reserve(static_cast<size_t>(capacity) * sizeof(float4)));
     }
 
-    CK(c, cudaMemsetAsync(d_counters, 0, kCounterBlock * sizeof(unsigned long long) + sizeof(TraceCounters), st));
-    CK(c, cudaEventRecord(c->ev0, st));
-    for (size_t k = 1; k < lanes.size(); ++k) { // the other lanes start after whatever the call's stream held before
-        CK(c, cudaStreamWaitEvent(lanes[k].st, c->ev0, 0));
-    }
+    // raygen and the stage chain of one batch of the queue wavefront: slots [0, np x ns) on `lane`
+    auto stage_chain = [&](WaveLane& lane, const Launch& L, const uint32_t* d_pix, uint32_t np, uint32_t sample0, uint32_t ns) {
+        const uint32_t max_n    = np * ns;
+        uint32_t**     q        = lane.queues;
+        uint32_t*      d_counts = lane.queue_counts;
+        CK(c, cudaMemsetAsync(d_counts, 0, counts_need * sizeof(uint32_t), L.stream));
+        uint32_t next_count = 0;
+        auto     new_count  = [&]() { return d_counts + next_count++; };
 
-    uint64_t batch = 0;
-    for (uint32_t pb = 0; pb < n_pix; pb += pix_per_batch) {
-        const uint32_t np = std::min(pix_per_batch, n_pix - pb);
-        for (uint32_t sb = 0; sb < n_samples; sb += smp_per_batch) {
-            const uint32_t ns    = std::min(smp_per_batch, n_samples - sb);
-            const uint32_t max_n = np * ns;
-            LaneView&      lane     = lanes[batch % lanes.size()];
-            uint32_t**     q        = lane.q;
-            uint32_t*      d_counts = lane.d_counts;
-            const Launch   L{ c->sm_count, lane.st, c->features };
-            CK(c, cudaMemsetAsync(d_counts, 0, counts_need * sizeof(uint32_t), lane.st));
-            uint32_t next_count = 0;
-            auto     new_count  = [&]() { return d_counts + next_count++; };
+        uint32_t* n_cur = new_count();
+        timer.begin(kStRaygen);
+        launch_raygen(L, s, lane.wave, d_pix, np, sample0, ns, q[kQCur], n_cur, d_counters);
+        timer.end();
+        ++launches;
 
-            uint32_t* n_cur = new_count();
-            timer.begin(kStRaygen);
-            launch_raygen(L, s, lane.wave, d_pix_list + pb, np, sample_begin + sb, ns, q[kQCur], n_cur, d_counters);
+        uint32_t* q_cur  = q[kQCur];
+        uint32_t* q_next = q[kQNext];
+        // advance (of depth d) + the set-up of extend (of depth d + 1) as ONE kernel where the extend stage has a `begin`
+        // kernel to put it in; the live queue of depth d then goes to extend directly
+        const bool fuse_advance    = !whitted && extend_fuses_advance(L, q[kQWalk], d_cnt);
+        bool       pending_advance = false;
+        for (uint32_t depth = 0; depth < max_depth; ++depth) {
+            RenderParams p{ part->seed, part->integrator, depth, 0 };
+            SortedQueue  sorted{ lane.sorted, d_counts + next_count, n_segments, capacity };
+            next_count += n_segments;
+            timer.begin(kStExtend);
+            uint32_t*         cursor = new_count();
+            const AdvanceArgs adv{ part->seed, depth - 1u };
+            launches += launch_extend(L, s, lane.wave, q_cur, n_cur, max_n, cursor, sorted,
+                                      // (node counting is DEFINED on the reference-order walk: DESIGN.md byte model)
+                                      c->options[SPCU_OPT_TRAVERSAL] == SPCU_TRAVERSAL_ORDERED && !d_cnt, q[kQWalk], new_count(),
+                                      d_counters, d_cnt, pending_advance ? &adv : nullptr);
+            pending_advance = false;
+            timer.end();
+            uint32_t* n_live   = new_count();
+            uint32_t* n_shadow = d_counts + next_count; // one shadow queue (and counter) per light
+            next_count += n_lights;
+            uint32_t* q_shadow = (nee || direct) ? q[kQShadow] : nullptr;
+            timer.begin(kStShade);
+            launch_shade(L, s, lane.wave, p, sorted, max_n, q[kQLive], n_live, q_shadow, n_shadow, d_counters);
+            timer.end();
+            launches += 1;
+            if (nee || direct) {
+                for (uint32_t li = 0; li < n_lights; ++li) {
+                    p.light_index        = li;
+                    uint32_t* q_shadow_l = q_shadow + static_cast<size_t>(li) * capacity;
+                    uint32_t* n_lit      = direct ? nullptr : new_count();
+                    timer.begin(kStShadow);
+                    uint32_t* cursor_l = new_count();
+                    launches += launch_shadow(L, s, lane.wave, q_shadow_l, n_shadow + li, max_n, li, cursor_l,
+                                              direct ? nullptr : q[kQLit], n_lit, q[kQWalk], new_count(), d_counters, d_cnt);
+                    timer.end();
+                    if (direct) {
+                        timer.begin(kStDirectAccumulate);
+                        launch_direct_accumulate(L, s, lane.wave, p, q_shadow_l, n_shadow + li, max_n, d_counters);
+                        timer.end();
+                        ++launches;
+                        continue;
+                    }
+                    uint32_t* n_mis = new_count();
+                    timer.begin(kStNeeBsdf);
+                    launch_nee_bsdf(L, s, lane.wave, p, q[kQLit], n_lit, max_n, q[kQMis], n_mis, d_counters);
+                    timer.end();
+                    timer.begin(kStMisTrace);
+                    uint32_t* cursor_m = new_count();
+                    launches += launch_mis_trace(L, s, lane.wave, q[kQMis], n_mis, max_n, cursor_m, q[kQWalk], new_count(), d_counters, d_cnt);
+                    timer.end();
+                    timer.begin(kStNeeMisAccumulate);
+                    launch_nee_mis_accumulate(L, s, lane.wave, q[kQMis], n_mis, max_n, d_counters);
+                    timer.end();
+                    launches += 2;
+                }
+            }
+            if (direct && !whitted) {
+                break;
+            }
+            if (fuse_advance) {
+                // the live queue is read by the next depth's extend (and rewritten only by the shade stage after it):
+                // two buffers in turn, so that this depth's q_live is intact while the next one's is being filled
+                q_cur           = q[kQLive];
+                n_cur           = n_live;
+                pending_advance = true;
+                std::swap(q[kQLive], q[kQNext]);
+                continue;
+            }
+            uint32_t* n_next = new_count();
+            timer.begin(kStAdvance);
+            if (whitted) {
+                launch_whitted_advance(L, s, lane.wave, p, q[kQLive], n_live, max_n, q_next, n_next, d_counters);
+            } else {
+                launch_advance(L, s, lane.wave, p, q[kQLive], n_live, max_n, q_next, n_next, d_counters);
+            }
             timer.end();
             ++launches;
+            std::swap(q_cur, q_next);
+            n_cur = n_next;
+        }
+        return SPCU_OK;
+    };
 
-            uint32_t* q_cur  = q[kQCur];
-            uint32_t* q_next = q[kQNext];
-            // advance (of depth d) + the set-up of extend (of depth d + 1) as ONE kernel where the extend stage has a `begin`
-            // kernel to put it in; the live queue of depth d then goes to extend directly
-            const bool fuse_advance = !whitted && extend_fuses_advance(L, q[kQWalk], d_cnt);
-            bool       pending_advance = false;
-            for (uint32_t depth = 0; depth < max_depth; ++depth) {
-                RenderParams p{ part->seed, part->integrator, depth, 0 };
-                SortedQueue sorted{ lane.sorted, d_counts + next_count, n_segments, capacity };
-                next_count += n_segments;
-                timer.begin(kStExtend);
-                uint32_t*         cursor = new_count();
-                const AdvanceArgs adv{ part->seed, depth - 1u };
-                launches += launch_extend(L, s, lane.wave, q_cur, n_cur, max_n, cursor, sorted,
-                                          // (node counting is DEFINED on the reference-order walk: DESIGN.md byte model)
-                                          c->options[SPCU_OPT_TRAVERSAL] == SPCU_TRAVERSAL_ORDERED && !d_cnt, q[kQWalk], new_count(),
-                                          d_counters, d_cnt, pending_advance ? &adv : nullptr);
-                pending_advance = false;
-                timer.end();
-                uint32_t* n_live   = new_count();
-                uint32_t* n_shadow = d_counts + next_count; // one shadow queue (and counter) per light
-                next_count += n_lights;
-                uint32_t* q_shadow = (nee || direct) ? q[kQShadow] : nullptr;
-                timer.begin(kStShade);
-                launch_shade(L, s, lane.wave, p, sorted, max_n, q[kQLive], n_live, q_shadow, n_shadow, d_counters);
-                timer.end();
-                launches += 1;
-                if (nee || direct) {
-                    for (uint32_t li = 0; li < n_lights; ++li) {
-                        p.light_index           = li;
-                        uint32_t* q_shadow_l    = q_shadow + static_cast<size_t>(li) * capacity;
-                        uint32_t* n_lit         = direct ? nullptr : new_count();
-                        timer.begin(kStShadow);
-                        uint32_t* cursor_l = new_count();
-                        launches += launch_shadow(L, s, lane.wave, q_shadow_l, n_shadow + li, max_n, li, cursor_l,
-                                                  direct ? nullptr : q[kQLit], n_lit, q[kQWalk], new_count(), d_counters, d_cnt);
-                        timer.end();
-                        if (direct) {
-                            timer.begin(kStDirectAccumulate);
-                            launch_direct_accumulate(L, s, lane.wave, p, q_shadow_l, n_shadow + li, max_n, d_counters);
-                            timer.end();
-                            ++launches;
-                            continue;
-                        }
-                        uint32_t* n_mis = new_count();
-                        timer.begin(kStNeeBsdf);
-                        launch_nee_bsdf(L, s, lane.wave, p, q[kQLit], n_lit, max_n, q[kQMis], n_mis, d_counters);
-                        timer.end();
-                        timer.begin(kStMisTrace);
-                        uint32_t* cursor_m = new_count();
-                        launches += launch_mis_trace(L, s, lane.wave, q[kQMis], n_mis, max_n, cursor_m, q[kQWalk], new_count(), d_counters, d_cnt);
-                        timer.end();
-                        timer.begin(kStNeeMisAccumulate);
-                        launch_nee_mis_accumulate(L, s, lane.wave, q[kQMis], n_mis, max_n, d_counters);
-                        timer.end();
-                        launches += 2;
-                    }
-                }
-                if (direct && !whitted) {
-                    break;
-                }
-                if (fuse_advance) {
-                    // the live queue is read by the next depth's extend (and rewritten only by the shade stage after it):
-                    // two buffers in turn, so that this depth's q_live is intact while the next one's is being filled
-                    q_cur           = q[kQLive];
-                    n_cur           = n_live;
-                    pending_advance = true;
-                    std::swap(q[kQLive], q[kQNext]);
-                    continue;
-                }
-                uint32_t* n_next = new_count();
-                timer.begin(kStAdvance);
-                if (whitted) {
-                    launch_whitted_advance(L, s, lane.wave, p, q[kQLive], n_live, max_n, q_next, n_next, d_counters);
+    CK(c, cudaMemsetAsync(d_counters, 0, kCounterBytes, st));
+    CK(c, cudaEventRecord(c->ev0, st));
+    for (uint32_t k = 1; k < n_lanes; ++k) { // the other lanes start after whatever the call's stream held before
+        CK(c, cudaStreamWaitEvent(c->lanes[k].stream, c->ev0, 0));
+    }
+    uint64_t batch = 0;
+    for (uint32_t pb = 0; pb < n_pix; pb += shape.pix) {
+        const uint32_t np = std::min(shape.pix, n_pix - pb);
+        for (uint32_t sb = 0; sb < n_samples; sb += shape.smp, ++batch) {
+            const uint32_t ns   = std::min(shape.smp, n_samples - sb);
+            const uint64_t k    = batch % n_lanes;
+            WaveLane&      lane = c->lanes[k];
+            const Launch   L{ c->sm_count, k ? lane.stream : st, c->features };
+            if (wavefront) {
+                if (int rc = stage_chain(lane, L, d_pix_list + pb, np, sample_begin + sb, ns); rc != SPCU_OK) return rc;
+            } else {
+                timer.begin(kStPaths);
+                if (pipeline == SPCU_PIPELINE_SMWAVE) {
+                    CK(c, launch_smwave(L, s, d_pix_list + pb, np, sample_begin + sb, ns, part->seed, part->integrator,
+                                        c->path_radiance.as<float4>(), d_counters, d_cnt));
                 } else {
-                    launch_advance(L, s, lane.wave, p, q[kQLive], n_live, max_n, q_next, n_next, d_counters);
+                    launch_paths(L, s, d_pix_list + pb, np, sample_begin + sb, ns, part->seed, part->integrator,
+                                 c->path_radiance.as<float4>(), d_counters, d_cnt);
                 }
                 timer.end();
                 ++launches;
-                std::swap(q_cur, q_next);
-                n_cur = n_next;
             }
             // batches add their samples to the accumulators in batch order, whichever lane ran them: this resolve waits for the
             // previous batch's (the float sums, and so the image, do not depend on the number of lanes)
-            if (lanes.size() > 1 && batch > 0) {
-                CK(c, cudaStreamWaitEvent(lane.st, lanes[(batch - 1) % lanes.size()].resolved, 0));
+            if (n_lanes > 1 && batch > 0) {
+                CK(c, cudaStreamWaitEvent(L.stream, c->lanes[(batch - 1) % n_lanes].resolved, 0));
             }
             timer.begin(kStResolve);
-            launch_resolve(L, &lane.wave.path->L, 2, d_pix_list + pb, np, ns, d_rgb_sum, d_lum_sumsq, d_counters);
+            launch_resolve(L, wavefront ? &lane.wave.path->L : c->path_radiance.as<float4>(), wavefront ? 2 : 1, d_pix_list + pb, np,
+                           ns, d_rgb_sum, d_lum_sumsq, d_counters);
             timer.end();
             ++launches;
-            if (lanes.size() > 1) {
-                CK(c, cudaEventRecord(lane.resolved, lane.st));
+            if (n_lanes > 1) {
+                CK(c, cudaEventRecord(lane.resolved, L.stream));
             }
-            ++batch;
             CK(c, cudaGetLastError());
         }
     }
-    for (size_t k = 1; k < lanes.size(); ++k) { // join: the call's stream ends after every lane's last resolve
-        CK(c, cudaStreamWaitEvent(st, lanes[k].resolved, 0));
+    for (uint32_t k = 1; k < n_lanes; ++k) { // join: the call's stream ends after every lane's last resolve
+        CK(c, cudaStreamWaitEvent(st, c->lanes[k].resolved, 0));
     }
     CK(c, cudaEventRecord(c->ev1, st));
 
     if (stats) {
         if (int rc = read_back_stats(c, st, stats, launches, timer); rc != SPCU_OK) return rc;
+        if (!wavefront) {
+            c->stage_report[kStPaths].items = stats->paths;
+        }
     }
     return SPCU_OK;
 }
@@ -529,7 +468,23 @@ int render_impl(spcu_ctx* c, const spcu_partition* part, float* d_rgb_sum, float
         return SPCU_OK;
     }
     return render_batches(c, part, c->pix_list.as<uint32_t>(), n_pix, part->sample_begin, n_samples, d_rgb_sum, d_lum_sumsq, stats,
-                          st, false);
+                          st);
+}
+
+// the counters and kernel times of one adaptive pass, added to the call's (its device_ms is timed over the whole call)
+void add_stats(spcu_stats& total, const spcu_stats& pass)
+{
+    total.paths += pass.paths;
+    total.rays_closest += pass.rays_closest;
+    total.rays_any += pass.rays_any;
+    total.rays_lights += pass.rays_lights;
+    total.nodes_visited += pass.nodes_visited;
+    total.prims_tested += pass.prims_tested;
+    total.xf_prims_tested += pass.xf_prims_tested;
+    total.shade_calls += pass.shade_calls;
+    total.kernel_launches += pass.kernel_launches;
+    total.trace_ms += pass.trace_ms;
+    total.shade_ms += pass.shade_ms;
 }
 
 // spcu_render_adaptive(_device): the pass loop over shrinking pixel lists (schedule and stopping test: include/spcu.h).  Pass 0
@@ -579,19 +534,9 @@ int adaptive_impl(spcu_ctx* c, const spcu_partition* part, const spcu_adaptive* 
         uint32_t  begin = 0, end = std::min(ad->min_spp, budget);
         for (;;) {
             spcu_stats ps{}; // (read back after every pass: the fault counter is checked there)
-            if (int rc = render_batches(c, part, list, n, begin, end - begin, d_rgb_sum, d_sq, &ps, st, true); rc != SPCU_OK) return rc;
+            if (int rc = render_batches(c, part, list, n, begin, end - begin, d_rgb_sum, d_sq, &ps, st); rc != SPCU_OK) return rc;
             ++passes;
-            total.paths += ps.paths;
-            total.rays_closest += ps.rays_closest;
-            total.rays_any += ps.rays_any;
-            total.rays_lights += ps.rays_lights;
-            total.nodes_visited += ps.nodes_visited;
-            total.prims_tested += ps.prims_tested;
-            total.xf_prims_tested += ps.xf_prims_tested;
-            total.shade_calls += ps.shade_calls;
-            total.kernel_launches += ps.kernel_launches;
-            total.trace_ms += ps.trace_ms;
-            total.shade_ms += ps.shade_ms;
+            add_stats(total, ps);
             if (end >= budget) {
                 break;
             }
@@ -632,10 +577,34 @@ int sync_and_check_faults(spcu_ctx* c, bool already_checked)
                               c->stream));
     }
     CK(c, cudaStreamSynchronize(c->stream));
-    if (faults) {
-        return fail(c, SPCU_ERR_INTERNAL, "%llu kernel(s) gave up on a bounded wait (queue protocol fault); the image is void", faults);
+    return faults ? queue_fault(c, faults) : SPCU_OK;
+}
+
+// The host-buffer entry points: device accumulators for the image (c->host_rgb, and c->host_sq `with_sumsq`), zeroed or, to
+// `accumulate`, holding the caller's sums; `render(d_rgb_sum, d_lum_sumsq)` enqueues the call's work on the context's stream;
+// the sums go back to rgb_sum / lum_sumsq where those are not NULL, and the call ends in the fault check.
+template <typename Render>
+int host_buffer_render(spcu_ctx* c, bool with_sumsq, bool accumulate, float* rgb_sum, float* lum_sumsq, bool already_checked,
+                       Render&& render)
+{
+    const size_t sq_bytes = static_cast<size_t>(c->ds.width) * c->ds.height * sizeof(float), rgb_bytes = 3 * sq_bytes;
+    CK(c, c->host_rgb.reserve(rgb_bytes));
+    float* d_sq = nullptr;
+    if (with_sumsq) {
+        CK(c, c->host_sq.reserve(sq_bytes));
+        d_sq = c->host_sq.as<float>();
     }
-    return SPCU_OK;
+    if (accumulate) {
+        CK(c, cudaMemcpyAsync(c->host_rgb.p, rgb_sum, rgb_bytes, cudaMemcpyHostToDevice, c->stream));
+        if (d_sq) CK(c, cudaMemcpyAsync(d_sq, lum_sumsq, sq_bytes, cudaMemcpyHostToDevice, c->stream));
+    } else {
+        CK(c, cudaMemsetAsync(c->host_rgb.p, 0, rgb_bytes, c->stream));
+        if (d_sq) CK(c, cudaMemsetAsync(d_sq, 0, sq_bytes, c->stream));
+    }
+    if (int rc = render(c->host_rgb.as<float>(), d_sq); rc != SPCU_OK) return rc;
+    if (rgb_sum) CK(c, cudaMemcpyAsync(rgb_sum, c->host_rgb.p, rgb_bytes, cudaMemcpyDeviceToHost, c->stream));
+    if (lum_sumsq && d_sq) CK(c, cudaMemcpyAsync(lum_sumsq, d_sq, sq_bytes, cudaMemcpyDeviceToHost, c->stream));
+    return sync_and_check_faults(c, already_checked);
 }
 
 } // namespace
@@ -662,21 +631,17 @@ int spcu_render_adaptive(spcu_ctx* c, const spcu_partition* part, const spcu_ada
     if (!rgb_sum || !spp_map) {
         return fail(c, SPCU_ERR_INVALID, "rgb_sum or spp_map is NULL");
     }
-    const size_t n_pixels = static_cast<size_t>(c->ds.width) * c->ds.height;
-    CK(c, c->host_rgb.reserve(n_pixels * 3 * sizeof(float)));
-    CK(c, c->host_sq.reserve(n_pixels * sizeof(float)));
-    CK(c, c->ad_spp_map.reserve(n_pixels * sizeof(uint32_t)));
-    if (int rc = adaptive_impl(c, part, ad, c->host_rgb.as<float>(), c->host_sq.as<float>(), c->ad_spp_map.as<uint32_t>(), n_passes,
-                               stats, nullptr, false);
-        rc != SPCU_OK) {
-        return rc;
-    }
-    CK(c, cudaMemcpyAsync(rgb_sum, c->host_rgb.p, n_pixels * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-    if (lum_sumsq) {
-        CK(c, cudaMemcpyAsync(lum_sumsq, c->host_sq.p, n_pixels * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-    }
-    CK(c, cudaMemcpyAsync(spp_map, c->ad_spp_map.p, n_pixels * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
-    return sync_and_check_faults(c, true); // (every pass's fault counter has been read)
+    const size_t map_bytes = static_cast<size_t>(c->ds.width) * c->ds.height * sizeof(uint32_t);
+    CK(c, c->ad_spp_map.reserve(map_bytes));
+    // (every pass's fault counter has been read)
+    return host_buffer_render(c, true, false, rgb_sum, lum_sumsq, true, [&](float* d_rgb_sum, float* d_sq) {
+        if (int rc = adaptive_impl(c, part, ad, d_rgb_sum, d_sq, c->ad_spp_map.as<uint32_t>(), n_passes, stats, nullptr, false);
+            rc != SPCU_OK) {
+            return rc;
+        }
+        CK(c, cudaMemcpyAsync(spp_map, c->ad_spp_map.p, map_bytes, cudaMemcpyDeviceToHost, c->stream));
+        return SPCU_OK;
+    });
 }
 
 int spcu_render(spcu_ctx* c, const spcu_partition* part, float* rgb_sum, float* lum_sumsq, spcu_stats* stats)
@@ -685,21 +650,9 @@ int spcu_render(spcu_ctx* c, const spcu_partition* part, float* rgb_sum, float* 
     if (!rgb_sum) {
         return fail(c, SPCU_ERR_INVALID, "rgb_sum is NULL");
     }
-    const size_t n_pixels = static_cast<size_t>(c->ds.width) * c->ds.height;
-    CK(c, c->host_rgb.reserve(n_pixels * 3 * sizeof(float)));
-    CK(c, cudaMemcpyAsync(c->host_rgb.p, rgb_sum, n_pixels * 3 * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-    float* d_sq = nullptr;
-    if (lum_sumsq) {
-        CK(c, c->host_sq.reserve(n_pixels * sizeof(float)));
-        CK(c, cudaMemcpyAsync(c->host_sq.p, lum_sumsq, n_pixels * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-        d_sq = c->host_sq.as<float>();
-    }
-    if (int rc = render_impl(c, part, c->host_rgb.as<float>(), d_sq, stats, nullptr, false); rc != SPCU_OK) return rc;
-    CK(c, cudaMemcpyAsync(rgb_sum, c->host_rgb.p, n_pixels * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-    if (lum_sumsq) {
-        CK(c, cudaMemcpyAsync(lum_sumsq, c->host_sq.p, n_pixels * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-    }
-    return sync_and_check_faults(c, stats != nullptr);
+    return host_buffer_render(c, lum_sumsq != nullptr, true, rgb_sum, lum_sumsq, stats != nullptr, [&](float* d_rgb_sum, float* d_sq) {
+        return render_impl(c, part, d_rgb_sum, d_sq, stats, nullptr, false);
+    });
 }
 
 int spcu_resolved_pipeline(const spcu_ctx* c)
@@ -713,21 +666,9 @@ int spcu_render_frame(spcu_ctx* c, const spcu_partition* part, float* rgb_sum, f
     if (!rgb_sum) {
         return fail(c, SPCU_ERR_INVALID, "rgb_sum is NULL");
     }
-    const size_t n_pixels = static_cast<size_t>(c->ds.width) * c->ds.height;
-    CK(c, c->host_rgb.reserve(n_pixels * 3 * sizeof(float)));
-    CK(c, cudaMemsetAsync(c->host_rgb.p, 0, n_pixels * 3 * sizeof(float), c->stream));
-    float* d_sq = nullptr;
-    if (lum_sumsq) {
-        CK(c, c->host_sq.reserve(n_pixels * sizeof(float)));
-        CK(c, cudaMemsetAsync(c->host_sq.p, 0, n_pixels * sizeof(float), c->stream));
-        d_sq = c->host_sq.as<float>();
-    }
-    if (int rc = render_impl(c, part, c->host_rgb.as<float>(), d_sq, stats, nullptr, false); rc != SPCU_OK) return rc;
-    CK(c, cudaMemcpyAsync(rgb_sum, c->host_rgb.p, n_pixels * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-    if (lum_sumsq) {
-        CK(c, cudaMemcpyAsync(lum_sumsq, c->host_sq.p, n_pixels * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-    }
-    return sync_and_check_faults(c, stats != nullptr);
+    return host_buffer_render(c, lum_sumsq != nullptr, false, rgb_sum, lum_sumsq, stats != nullptr, [&](float* d_rgb_sum, float* d_sq) {
+        return render_impl(c, part, d_rgb_sum, d_sq, stats, nullptr, false);
+    });
 }
 
 int spcu_render_frame_reduced(spcu_ctx* c, const spcu_partition* part, int with_sumsq, float* rgb_sum, float* lum_sumsq,
@@ -738,24 +679,11 @@ int spcu_render_frame_reduced(spcu_ctx* c, const spcu_partition* part, int with_
     if (root && (!rgb_sum || (with_sumsq && !lum_sumsq))) {
         return fail(c, SPCU_ERR_INVALID, "rank 0 needs the host buffers");
     }
-    const size_t n_pixels = static_cast<size_t>(c->ds.width) * c->ds.height;
-    CK(c, c->host_rgb.reserve(n_pixels * 3 * sizeof(float)));
-    CK(c, cudaMemsetAsync(c->host_rgb.p, 0, n_pixels * 3 * sizeof(float), c->stream));
-    float* d_sq = nullptr;
-    if (with_sumsq) {
-        CK(c, c->host_sq.reserve(n_pixels * sizeof(float)));
-        CK(c, cudaMemsetAsync(c->host_sq.p, 0, n_pixels * sizeof(float), c->stream));
-        d_sq = c->host_sq.as<float>();
-    }
-    if (int rc = render_impl(c, part, c->host_rgb.as<float>(), d_sq, stats, nullptr, false); rc != SPCU_OK) return rc;
-    if (int rc = spcu_reduce_to_root(c, c->host_rgb.as<float>(), d_sq, c->stream); rc != SPCU_OK) return rc;
-    if (root) {
-        CK(c, cudaMemcpyAsync(rgb_sum, c->host_rgb.p, n_pixels * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-        if (with_sumsq) {
-            CK(c, cudaMemcpyAsync(lum_sumsq, c->host_sq.p, n_pixels * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-        }
-    }
-    return sync_and_check_faults(c, stats != nullptr);
+    return host_buffer_render(c, with_sumsq != 0, false, root ? rgb_sum : nullptr, root ? lum_sumsq : nullptr, stats != nullptr,
+                              [&](float* d_rgb_sum, float* d_sq) {
+                                  if (int rc = render_impl(c, part, d_rgb_sum, d_sq, stats, nullptr, false); rc != SPCU_OK) return rc;
+                                  return spcu_reduce_to_root(c, d_rgb_sum, d_sq, c->stream);
+                              });
 }
 
 int spcu_render_image(spcu_ctx* c, const spcu_partition* part, uint32_t format, void* out, spcu_stats* stats)
@@ -764,17 +692,18 @@ int spcu_render_image(spcu_ctx* c, const spcu_partition* part, uint32_t format, 
     if (!part || part->sample_end <= part->sample_begin) {
         return fail(c, SPCU_ERR_INVALID, "empty sample range");
     }
-    const size_t n_pixels = static_cast<size_t>(c->ds.width) * c->ds.height;
-    CK(c, c->host_rgb.reserve(n_pixels * 3 * sizeof(float)));
-    CK(c, cudaMemsetAsync(c->host_rgb.p, 0, n_pixels * 3 * sizeof(float), c->stream));
-    if (int rc = render_impl(c, part, c->host_rgb.as<float>(), nullptr, stats, nullptr, false); rc != SPCU_OK) return rc;
-    if (int rc = sync_and_check_faults(c, stats != nullptr); rc != SPCU_OK) return rc;
+    if (int rc = host_buffer_render(c, false, false, nullptr, nullptr, stats != nullptr,
+                                    [&](float* d_rgb_sum, float*) { return render_impl(c, part, d_rgb_sum, nullptr, stats, nullptr, false); });
+        rc != SPCU_OK) {
+        return rc;
+    }
     return pack_device_image(c, c->host_rgb.as<float>(), nullptr, c->ds.width, c->ds.height, part->sample_end - part->sample_begin, format,
                              out);
 }
 
 // Ray batches through the renderer's own traversal stages: the kernels a frame runs (begin + persistent walk, lane refill,
-// pair leaf steps), not the one-thread-per-ray kernels behind spcu_trace_*.
+// pair leaf steps), not the one-thread-per-ray kernels behind spcu_trace_*.  They borrow lane 0 of the render's wavefront
+// state (shadow rays use light plane 0).
 static int stage_batch(spcu_ctx* c, const spcu_ray* rays, uint64_t n, uint32_t traversal, spcu_hit* hits, spcu_hit* light_hits,
                        uint8_t* occluded)
 {
@@ -787,39 +716,35 @@ static int stage_batch(spcu_ctx* c, const spcu_ray* rays, uint64_t n, uint32_t t
         return fail(c, SPCU_ERR_INVALID, "unknown traversal %u", traversal);
     }
     const cudaStream_t st = c->stream;
-    if (c->scratch_in_use && c->scratch_stream != st) {
-        CK(c, cudaStreamWaitEvent(st, c->ev1, 0));
-    }
-    const uint32_t chunk = static_cast<uint32_t>(std::min<uint64_t>(std::max<uint64_t>(n, 1), kBatchRays));
-    // the batch borrows the render's wavefront state: keep its capacity when it is already large enough (capacity is also the
-    // stride of the per-light planes, and shadow rays use plane 0)
-    const uint32_t capacity = (c->wave.capacity >= chunk && c->wave_lights == c->ds.n_lights) ? c->wave.capacity : chunk;
-    if (int rc = ensure_wave(c, capacity); rc != SPCU_OK) return rc;
-    const uint32_t n_segments = std::min<uint32_t>(c->n_materials, kMaxMaterialSegments) + 1u;
-    CK(c, c->sorted_queue.reserve(static_cast<size_t>(n_segments) * capacity * sizeof(uint32_t)));
+    if (int rc = wait_for_scratch(c, st); rc != SPCU_OK) return rc;
+    const uint32_t chunk      = static_cast<uint32_t>(std::min<uint64_t>(std::max<uint64_t>(n, 1), kBatchRays));
+    const uint32_t n_segments = material_segments(c);
+    WaveLane&      lane       = c->lanes[0];
+    if (int rc = lay_out_lane(c, lane, chunk, n_segments); rc != SPCU_OK) return rc;
+    CK(c, c->counters.reserve(kCounterBytes));
     CK(c, c->q_rays.reserve(static_cast<size_t>(chunk) * sizeof(spcu_ray)));
     CK(c, c->q_out.reserve(static_cast<size_t>(chunk) * sizeof(spcu_hit)));
     CK(c, c->q_aux.reserve(static_cast<size_t>(chunk) * sizeof(spcu_hit)));
     auto*        d_counters = c->counters.as<unsigned long long>();
-    uint32_t*    d_counts   = c->queue_counts.as<uint32_t>();
+    uint32_t*    d_counts   = lane.queue_counts;
     const Launch L{ c->sm_count, st, c->features };
     for (uint64_t done = 0; done < n; done += chunk) {
         const uint32_t m = static_cast<uint32_t>(std::min<uint64_t>(chunk, n - done));
         CK(c, cudaMemcpyAsync(c->q_rays.p, rays + done, static_cast<size_t>(m) * sizeof(spcu_ray), cudaMemcpyHostToDevice, st));
         CK(c, cudaMemsetAsync(d_counts, 0, (8 + n_segments) * sizeof(uint32_t), st));
-        CK(c, cudaMemsetAsync(d_counters, 0, kCounterBlock * sizeof(unsigned long long) + sizeof(TraceCounters), st));
+        CK(c, cudaMemsetAsync(d_counters, 0, kCounterBytes, st));
         uint32_t* n_cur = d_counts + 0;
-        launch_batch_fill(c->wave, c->q_rays.as<spcu_ray>(), m, c->queues[kQCur].as<uint32_t>(), n_cur, shadow, st);
+        launch_batch_fill(lane.wave, c->q_rays.as<spcu_ray>(), m, lane.queues[kQCur], n_cur, shadow, st);
         if (shadow) {
-            launch_shadow(L, c->ds, c->wave, c->queues[kQCur].as<uint32_t>(), n_cur, m, 0, d_counts + 1, nullptr, nullptr,
-                          c->queues[kQWalk].as<uint32_t>(), d_counts + 2, d_counters, nullptr);
+            launch_shadow(L, c->ds, lane.wave, lane.queues[kQCur], n_cur, m, 0, d_counts + 1, nullptr, nullptr, lane.queues[kQWalk],
+                          d_counts + 2, d_counters, nullptr);
             CK(c, cudaGetLastError());
-            CK(c, cudaMemcpyAsync(occluded + done, c->wave.occluded, m, cudaMemcpyDeviceToHost, st));
+            CK(c, cudaMemcpyAsync(occluded + done, lane.wave.occluded, m, cudaMemcpyDeviceToHost, st));
         } else {
-            SortedQueue sorted{ c->sorted_queue.as<uint32_t>(), d_counts + 8, n_segments, capacity };
-            launch_extend(L, c->ds, c->wave, c->queues[kQCur].as<uint32_t>(), n_cur, m, d_counts + 1, sorted,
-                          traversal == SPCU_TRAVERSAL_ORDERED, c->queues[kQWalk].as<uint32_t>(), d_counts + 2, d_counters, nullptr);
-            launch_batch_gather_extend(c->wave, m, c->q_out.as<spcu_hit>(), light_hits ? c->q_aux.as<spcu_hit>() : nullptr, st);
+            SortedQueue sorted{ lane.sorted, d_counts + 8, n_segments, chunk };
+            launch_extend(L, c->ds, lane.wave, lane.queues[kQCur], n_cur, m, d_counts + 1, sorted, traversal == SPCU_TRAVERSAL_ORDERED,
+                          lane.queues[kQWalk], d_counts + 2, d_counters, nullptr);
+            launch_batch_gather_extend(lane.wave, m, c->q_out.as<spcu_hit>(), light_hits ? c->q_aux.as<spcu_hit>() : nullptr, st);
             CK(c, cudaGetLastError());
             CK(c, cudaMemcpyAsync(hits + done, c->q_out.p, static_cast<size_t>(m) * sizeof(spcu_hit), cudaMemcpyDeviceToHost, st));
             if (light_hits) {
