@@ -25,7 +25,7 @@
 extern "C" {
 #endif
 
-#define SPCU_ABI_VERSION 1
+#define SPCU_ABI_VERSION 2
 
 /* ---- error codes ------------------------------------------------------------------------- */
 #define SPCU_OK 0
@@ -308,15 +308,22 @@ int spcu_render_device(spcu_ctx* ctx, const spcu_partition* part, float* d_rgb_s
  * is tested with n = s_k, and the pass after it renders [s_k, s_{k+1}) of the pixels that failed the test only.  The test,
  * float32 with one rounding per operation (R, G, B = the pixel's rgb_sum, Q = its lum_sumsq):
  *   L = (0.2126 R + 0.7152 G) + 0.0722 B;  m = L / n;  d = Q / n - m m;  v = d > 0 ? d (n / (n - 1)) : 0;
- *   stop  <=>  R, G, B, Q finite  and  v / n <= (rel_error (m + abs_floor))^2
+ *   pass  <=>  R, G, B, Q finite  and  v / n <= (rel_error (m + abs_floor))^2
+ * With radius 0 an active pixel stops at s_k iff it passes.  With radius r > 0 it stops iff every pixel q of its window
+ *   W(p) = { q : |x_q - x_p| <= r, |y_q - y_p| <= r, q in the same 8x8 tile as p, q inside the image }
+ * passes, where a pixel that stopped at an earlier boundary counts as passing and every other one is tested with n = s_k.
+ * All of a boundary's tests are made before any of its decisions, so the decisions do not depend on thread order.  r >= 7
+ * makes the window the whole tile: a tile then stops at one boundary.  n_p cannot decrease as r grows.
  * So pixel p gets samples [0, n_p) with min(min_spp, sample_end) <= n_p <= sample_end, and its sums equal bit for bit those
  * of a fixed render of [0, n_p): the result does not depend on the tile partition, the batch shape or the kernel
- * organisation.  Stopping on an estimated variance biases the mean slightly in principle (DESIGN.md). */
+ * organisation (a window never leaves its tile, and a tile belongs to one partition).  What stopping on an estimated
+ * variance does to the mean, and what the window does about it, is measured in DESIGN.md §11. */
 typedef struct spcu_adaptive {
     uint32_t min_spp;   /* samples before the first test, >= 2                                              */
     uint32_t pass_spp;  /* samples added per pass, >= 1                                                     */
     float    rel_error; /* target standard error relative to the mean luminance, finite, >= 0             */
     float    abs_floor; /* added to the mean in the target, so that near-black pixels can stop; finite, >= 0 */
+    uint32_t radius;    /* half-width of the window of the stopping rule, 0..7 (0: each pixel on its own)         */
 } spcu_adaptive;
 
 /* Adaptive render of a tile partition into host buffers, OVERWRITTEN like spcu_render_frame's: rgb_sum / lum_sumsq (may be

@@ -1,11 +1,11 @@
 #!/usr/bin/env python
 """Adaptive sampling against fixed spp at equal image quality: time, paths and relMSE of fixed renders (16 .. 256 spp) and of
-adaptive renders with a budget of 256 at several target errors, on the 1080p configs, against a 1024 spp "truth" render of
+adaptive renders with a budget of 256 at several target errors and window radii, on the 1080p configs, against a 1024 spp "truth" render of
 another seed.  relMSE = mean over pixels of (L - L_truth)^2 / (L_truth^2 + 1e-3) (the converged tests' metric, per pixel).
 Times: host clock around a call that ends in a synchronise (host-buffer entry points), after a warm-up call of the same
 shape; median of --reps calls.  One JSON line per point, then one "equal_relmse" line per adaptive point: the fixed-spp time
 at the same relMSE, interpolated log-log between the two fixed points around it (null outside the fixed range).
-    python profiles/scripts/adaptive_probe.py --out profiles/rNN_adaptive_probe.jsonl"""
+    python profiles/scripts/adaptive_probe.py [--radius 0 1 2 7] --out profiles/rNN_adaptive_probe.jsonl"""
 import argparse
 import json
 import subprocess
@@ -62,6 +62,7 @@ def main():
     ap.add_argument("--out", required=True)
     ap.add_argument("--reps", type=int, default=3)
     ap.add_argument("--scenes", nargs="*", default=SCENES)
+    ap.add_argument("--radius", type=int, nargs="+", default=[0], help="window radii of the stopping rule (0..7)")
     args = ap.parse_args()
     info = gpu_info()
     ctx = capi.Context(0)
@@ -92,18 +93,19 @@ def main():
                 fixed.append((e, sec))
                 emit({**base, "mode": "fixed", "spp": spp, "seconds": sec, "paths": st["paths"], "mean_spp": float(spp),
                       "passes": 1, "relmse": e, "device_ms": st["device_ms"]})
-            for rel in ERRORS:
+            for radius, rel in ((r, e) for r in args.radius for e in ERRORS):
                 part = ctx.partition(spp=TRUTH_SPP, sample_end=BUDGET, seed=SEED)
                 sec, (rgb, _, spp_map, st) = timed(lambda: ctx.render_adaptive(part, rel, min_spp=MIN_SPP, pass_spp=PASS_SPP,
-                                                                               abs_floor=ABS_FLOOR, want_sumsq=False), args.reps)
+                                                                               abs_floor=ABS_FLOOR, want_sumsq=False,
+                                                                               radius=radius), args.reps)
                 n = spp_map.astype(np.float64)
                 e = relmse(rgb, n[..., None])
                 t_fixed = interp_fixed_time(fixed, e)
-                emit({**base, "mode": "adaptive", "rel_error": rel, "abs_floor": ABS_FLOOR, "budget": BUDGET, "min_spp": MIN_SPP,
+                emit({**base, "mode": "adaptive", "rel_error": rel, "radius": radius, "abs_floor": ABS_FLOOR, "budget": BUDGET, "min_spp": MIN_SPP,
                       "pass_spp": PASS_SPP, "seconds": sec, "paths": st["paths"], "mean_spp": float(n.mean()),
                       "passes": st["passes"], "stopped_early": float((spp_map < BUDGET).mean()), "relmse": e,
                       "device_ms": st["device_ms"]})
-                emit({**base, "mode": "equal_relmse", "rel_error": rel, "relmse": e, "adaptive_seconds": sec,
+                emit({**base, "mode": "equal_relmse", "rel_error": rel, "radius": radius, "relmse": e, "adaptive_seconds": sec,
                       "fixed_seconds_at_equal_relmse": t_fixed, "speedup": (t_fixed / sec) if t_fixed else None})
     ctx.close()
 

@@ -14,7 +14,7 @@ PKG = Path(__file__).resolve().parent
 import os
 LIB_PATH = Path(os.environ.get("SPCU_LIB", PKG / "csrc" / "libspcu.so"))  # SPCU_LIB: experiments with another build
 
-ABI_VERSION = 1
+ABI_VERSION = 2
 INTEGRATORS = {"iterative_rrnee": 0, "brute_force_iterative_rr": 1, "direct_lighting": 2, "whitted": 3}
 
 
@@ -103,7 +103,8 @@ class Stats(C.Structure):
 
 class Adaptive(C.Structure):
     """spcu_adaptive: parameters of spcu_render_adaptive (include/spcu.h)."""
-    _fields_ = [("min_spp", C.c_uint32), ("pass_spp", C.c_uint32), ("rel_error", C.c_float), ("abs_floor", C.c_float)]
+    _fields_ = [("min_spp", C.c_uint32), ("pass_spp", C.c_uint32), ("rel_error", C.c_float), ("abs_floor", C.c_float),
+                ("radius", C.c_uint32)]
 
 
 class StageTime(C.Structure):
@@ -503,14 +504,15 @@ class Context:
         return out
 
     def render_adaptive(self, part: Partition, rel_error: float, min_spp: int = 16, pass_spp: int = 16, abs_floor: float = 0.0,
-                        want_sumsq: bool = True):
+                        want_sumsq: bool = True, radius: int = 0):
         """Adaptive sampling (spcu_render_adaptive): each pixel of the partition gets samples [0, n_p) until the standard error of
-        its mean luminance is at most rel_error * (mean + abs_floor), n_p <= part.sample_end (the budget).  Outputs are
-        overwritten: (rgb_sum [H,W,3], lum_sumsq [H,W] | None, spp_map [H,W] uint32 = n_p, stats dict with "passes")."""
+        its mean luminance is at most rel_error * (mean + abs_floor), n_p <= part.sample_end (the budget).  radius > 0: a pixel
+        stops only when every pixel within `radius` of it in its 8x8 tile meets the target too.  Outputs are overwritten:
+        (rgb_sum [H,W,3], lum_sumsq [H,W] | None, spp_map [H,W] uint32 = n_p, stats dict with "passes")."""
         rgb = np.empty((self.height, self.width, 3), dtype=np.float32)
         sq = np.empty((self.height, self.width), dtype=np.float32) if want_sumsq else None
         spp_map = np.empty((self.height, self.width), dtype=np.uint32)
-        ad = Adaptive(min_spp, pass_spp, rel_error, abs_floor)
+        ad = Adaptive(min_spp, pass_spp, rel_error, abs_floor, radius)
         passes = C.c_uint32()
         st = Stats()
         self._check(self.lib.spcu_render_adaptive(self.h, C.byref(part), C.byref(ad), _ptr(rgb), _ptr(sq) if want_sumsq else None,

@@ -122,8 +122,9 @@ struct spcu_ctx
     spcu::DevBuf              host_rgb, host_sq; // device accumulators of the host-buffer entry point
     spcu::DevBuf              packed;            // packed output image (spcu_render_image / spcu_pack_image)
     // adaptive sampling (spcu_render_adaptive): ping-pong active pixel lists, the per-pixel sample counts, a lum_sumsq
-    // accumulator for callers that pass none, the compaction's scratch + active count, and the call's event pair
-    spcu::DevBuf              ad_list[2], ad_spp_map, ad_sq, ad_scratch;
+    // accumulator for callers that pass none, the compaction's scratch + active count, the per-tile pass flags of the
+    // neighbourhood test (radius > 0), and the call's event pair
+    spcu::DevBuf              ad_list[2], ad_spp_map, ad_sq, ad_scratch, ad_mask;
     cudaEvent_t               ad_ev[2] = { nullptr, nullptr };
     void*                     stage[2]    = { nullptr, nullptr }; // page-locked staging of large host->device copies
     cudaEvent_t               stage_ev[2] = { nullptr, nullptr };

@@ -126,10 +126,15 @@ cudaError_t launch_smwave(const Launch& l, const DScene& s, const uint32_t* d_pi
 // ---- adaptive_kernels.cu (exact float32 arithmetic: --fmad=false, no fast-math) ----------------------------------------------
 // The stopping test of spcu_render_adaptive at a pass boundary, for list entries [0, n) after n_samples samples: pixels that
 // pass get d_spp_map[pix] = n_samples, the others are copied, in list order, to d_next_list; *d_n_next = how many.
+// radius > 0: a pixel stops only if every pixel of its window (|dx|, |dy| <= radius, clipped to its 8x8 tile and the image)
+// passes; d_pass_mask (adaptive_mask_bytes, one word per tile, set to all-ones at the start of the call) holds the pass
+// flags between boundaries.  radius == 0 launches the per-pixel test only and does not touch d_pass_mask.
 // d_scratch: adaptive_scratch_bytes(n) bytes.  Enqueue only.
 size_t      adaptive_scratch_bytes(uint32_t n);
+size_t      adaptive_mask_bytes(uint32_t width, uint32_t height);
 cudaError_t launch_adaptive_compact(const uint32_t* d_list, uint32_t n, const float* d_rgb_sum, const float* d_lum_sumsq,
-                                    uint32_t n_samples, float rel_error, float abs_floor, uint32_t* d_spp_map, uint32_t* d_next_list,
+                                    uint32_t n_samples, float rel_error, float abs_floor, uint32_t width, uint32_t height,
+                                    uint32_t radius, unsigned long long* d_pass_mask, uint32_t* d_spp_map, uint32_t* d_next_list,
                                     void* d_scratch, uint32_t* d_n_next, cudaStream_t st);
 // d_spp_map[d_list[i]] = value for i < n
 cudaError_t launch_adaptive_fill(const uint32_t* d_list, uint32_t n, uint32_t value, uint32_t* d_spp_map, cudaStream_t st);

@@ -501,6 +501,10 @@ int adaptive_impl(spcu_ctx* c, const spcu_partition* part, const spcu_adaptive* 
         return fail(c, SPCU_ERR_INVALID, "bad adaptive parameters: min_spp %u (>= 2), pass_spp %u (>= 1), rel_error %g, abs_floor %g "
                     "(finite, >= 0)", ad->min_spp, ad->pass_spp, ad->rel_error, ad->abs_floor);
     }
+    if (ad->radius > 7) {
+        return fail(c, SPCU_ERR_INVALID, "bad adaptive window radius %u (0..7: the window is clipped to the pixel's 8x8 tile)",
+                    ad->radius);
+    }
     if (part && part->sample_begin != 0) {
         return fail(c, SPCU_ERR_INVALID, "adaptive rendering starts at sample 0 (sample_begin %u)", part->sample_begin);
     }
@@ -531,6 +535,11 @@ int adaptive_impl(spcu_ctx* c, const spcu_partition* part, const spcu_adaptive* 
         }
         CK(c, c->ad_scratch.reserve(sizeof(uint32_t) + adaptive_scratch_bytes(n))); // active count, then the compaction's scratch
         uint32_t* d_n_next = c->ad_scratch.as<uint32_t>();
+        if (ad->radius > 0) { // all pass: pixels that stop keep their set bit, those never tested are outside every window
+            const size_t mask_bytes = adaptive_mask_bytes(c->ds.width, c->ds.height);
+            CK(c, c->ad_mask.reserve(mask_bytes));
+            CK(c, cudaMemsetAsync(c->ad_mask.p, 0xff, mask_bytes, st));
+        }
         uint32_t  begin = 0, end = std::min(ad->min_spp, budget);
         for (;;) {
             spcu_stats ps{}; // (read back after every pass: the fault counter is checked there)
@@ -541,9 +550,9 @@ int adaptive_impl(spcu_ctx* c, const spcu_partition* part, const spcu_adaptive* 
                 break;
             }
             uint32_t* next = c->ad_list[passes & 1u].as<uint32_t>(); // never the list being read (pass 0 reads c->pix_list)
-            CK(c, launch_adaptive_compact(list, n, d_rgb_sum, d_sq, end, ad->rel_error, ad->abs_floor, d_spp_map, next, d_n_next + 1,
-                                          d_n_next, st));
-            total.kernel_launches += 3;
+            CK(c, launch_adaptive_compact(list, n, d_rgb_sum, d_sq, end, ad->rel_error, ad->abs_floor, c->ds.width, c->ds.height,
+                                          ad->radius, c->ad_mask.as<unsigned long long>(), d_spp_map, next, d_n_next + 1, d_n_next, st));
+            total.kernel_launches += ad->radius > 0 ? 4 : 3;
             CK(c, cudaMemcpyAsync(&n, d_n_next, sizeof n, cudaMemcpyDeviceToHost, st));
             CK(c, cudaStreamSynchronize(st)); // the next pass's batches are shaped by the number of active pixels
             list = next;

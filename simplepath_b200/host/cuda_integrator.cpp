@@ -128,7 +128,7 @@ CudaIntegrator::~CudaIntegrator() = default;
 
 // Sum of radiance samples per pixel, row major W*H*3.
 void CudaIntegrator::render_sum(const Scene& scene, unsigned spp, std::vector<float>& rgb_sum, std::vector<std::uint32_t>* spp_map,
-                                float rel_error) const
+                                float rel_error, std::uint32_t radius) const
 {
     if (m_devices.empty()) {
         for (int i = 0; i < m_options.n_devices; ++i) {
@@ -225,7 +225,7 @@ void CudaIntegrator::render_sum(const Scene& scene, unsigned spp, std::vector<fl
     if (spp_map) { // (one device: render_frame checks)
         // passes of 16 samples (fewer when the budget is smaller); the first test needs at least 2 samples
         const std::uint32_t  k = std::min(16u, spp);
-        const spcu_adaptive  ad{ std::max(2u, k), k, rel_error, 0.0f };
+        const spcu_adaptive  ad{ std::max(2u, k), k, rel_error, 0.0f, radius };
         const spcu_partition part{ 0u, 1u, 0u, spp, spp, code, m_options.seed };
         spp_map->resize(n / 3u);
         std::uint32_t passes = 0;
@@ -236,8 +236,9 @@ void CudaIntegrator::render_sum(const Scene& scene, unsigned spp, std::vector<fl
             early += c < spp ? 1u : 0u;
         }
         const double pixels = static_cast<double>(spp_map->size());
-        std::fprintf(stderr, "CudaIntegrator: adaptive sampling to %g: %u passes, mean %.2f spp of %u, %.1f %% of pixels stopped early\n",
-                     rel_error, passes, static_cast<double>(m_stats.paths) / pixels, spp, 100.0 * static_cast<double>(early) / pixels);
+        std::fprintf(stderr, "CudaIntegrator: adaptive sampling to %g, window radius %u: %u passes, mean %.2f spp of %u, %.1f %% of pixels "
+                     "stopped early\n", rel_error, radius, passes, static_cast<double>(m_stats.paths) / pixels, spp,
+                     100.0 * static_cast<double>(early) / pixels);
         return;
     }
     std::vector<spcu_stats> stats(n_dev);
@@ -274,10 +275,20 @@ bool CudaIntegrator::render_frame(const Scene& scene, unsigned spp, Image& image
         if (end == adaptive || *end != '\0') {
             throw std::runtime_error(std::string("CudaIntegrator: SPCU_ADAPTIVE must be a relative standard error, not '") + adaptive + "'");
         }
+        std::uint32_t radius = 0; // SPCU_ADAPTIVE_RADIUS=<0..7>: a pixel stops only when its window in its tile has converged
+        if (const char* r = std::getenv("SPCU_ADAPTIVE_RADIUS"); r && *r) {
+            char*               r_end = nullptr;
+            const unsigned long v     = std::strtoul(r, &r_end, 10);
+            if (r_end == r || *r_end != '\0' || *r < '0' || *r > '9' || v > 7) {
+                throw std::runtime_error(std::string("CudaIntegrator: SPCU_ADAPTIVE_RADIUS must be a window radius from 0 to 7, not '") + r +
+                                         "'");
+            }
+            radius = static_cast<std::uint32_t>(v);
+        }
         if (m_options.n_devices > 1) {
             throw std::runtime_error("CudaIntegrator: SPCU_ADAPTIVE renders on one device; unset SPCU_DEVICES or set it to 1");
         }
-        render_sum(scene, spp, sum, &counts, rel);
+        render_sum(scene, spp, sum, &counts, rel, radius);
     } else {
         render_sum(scene, spp, sum);
     }
