@@ -56,14 +56,19 @@ def test_per_pixel_vs_oracle(ctx, oracle_port, scene, integrator):
     rgb, sq, st = ctx.render(part)
     want, want_sq, want_st = oracle_port.render(flat.pointer(), jitter, part)
     assert st["paths"] == want_st["paths"] == flat.width * flat.height * spp
-    # stated tolerance: a pixel "agrees" when every channel is within 2e-3 * (1 + |oracle|) of the oracle's sum.
+    # stated tolerance: a pixel "agrees" when every channel, and its sum of squared luminance, is within 2e-3 * (1 + |oracle|)
+    # of the oracle's sum.
     # The bounds below are 3-4x the worst case measured over all 84 (scene, pipeline, integrator) combinations
     # (profiles/scripts/parity_margins.py -> profiles/r03t_parity_margins.jsonl: 0.13 % of pixels, 0.035 % of the mean
     # luminance, 0.24 % of the shade calls, 0.09 % / 0.04 % of the light / any-hit queries, closest-hit counts equal).
     tol = 2e-3 * (1.0 + np.abs(want))
-    bad = (np.abs(rgb - want) > tol).any(axis=-1)
+    bad = (np.abs(rgb - want) > tol).any(axis=-1) | (np.abs(sq - want_sq) > 2e-3 * (1.0 + np.abs(want_sq)))
     assert bad.mean() < 0.005, f"{name}/{integrator}: {bad.mean():.2%} of pixels differ from the oracle"
     assert abs(lum(rgb).mean() - lum(want).mean()) <= 0.002 * lum(want).mean() + 1e-6
+    # a scale error below the per-pixel band (a 1e-3 one passes it) moves the median relative difference of the pixels that
+    # agree, which rounding alone leaves at 0 (measured at 1080p: tests/test_gpu_render_steady_state.py)
+    lit = ~bad & (want_sq > 0)
+    assert abs(np.median(sq[lit] / want_sq[lit] - 1.0)) < 1e-4 and abs(np.median(lum(rgb)[lit] / lum(want)[lit] - 1.0)) < 1e-4
     # identical random numbers => identical path structure except for those few paths
     for key in ("rays_closest", "rays_lights"):
         assert abs(st[key] - want_st[key]) <= 0.005 * want_st[key] + 8, (key, st[key], want_st[key])
