@@ -339,6 +339,57 @@ int spcu_render_adaptive(spcu_ctx* ctx, const spcu_partition* part, const spcu_a
 int spcu_render_adaptive_device(spcu_ctx* ctx, const spcu_partition* part, const spcu_adaptive* ad, float* d_rgb_sum,
                                 float* d_lum_sumsq, uint32_t* d_spp_map, uint32_t* n_passes, spcu_stats* stats, void* stream);
 
+/* ---- denoising -----------------------------------------------------------------------------------------------------------
+ * Turns a low-sample frame into a smoother image: the spatial filter of SVGF (an edge-avoiding à-trous wavelet filter whose
+ * luminance term is scaled by each pixel's standard deviation), guided by the first hit of each pixel's camera ray.  Replaces
+ * nothing in the reference (it divides the sums by the sample count, main.cpp:100-102).  DESIGN.md §12 has the measurements.
+ *
+ * Guide buffers: one record per pixel of the uploaded scene's image, from the camera ray of sample 0 (the ray a render traces
+ * first), with the extend stage's rule and the exact walk: intersect_lights with the ray's limits, then intersect with t_max
+ * shrunk to the light's distance; a geometry hit under that limit wins, else a light hit, else the ray missed.  id and depth
+ * equal what spcu_extend_batch(camera ray of (pix, 0), SPCU_TRAVERSAL_EXACT) returns. */
+typedef struct spcu_guide {
+    float   normal[3]; /* unit shading normal of the first geometry hit, facing the camera; 0 otherwise             */
+    float   depth;     /* distance of the accepted hit (geometry or light); the ray's t_max (FLT_MAX) on a miss     */
+    float   albedo[3]; /* one-sample material (a clearcoat's base, followed): sum over its BxDFs in table order of
+                          r * pi (Lambert) or r (microfacet, specular), float32; 0 for light hits and misses         */
+    int32_t id;        /* >= 0 geometry primitive (reference-order ID); -2 - k light k (ID order); -1 miss          */
+} spcu_guide;          /* 32 bytes */
+/* Host out[h*w] / device d_out[h*w] (on `stream`, cudaStream_t as void*, NULL = default stream), overwritten. */
+int spcu_render_guides(spcu_ctx* ctx, spcu_guide* out);
+int spcu_render_guides_device(spcu_ctx* ctx, spcu_guide* d_out, void* stream);
+
+/* The filter, float32 with one rounding per operation and taps summed in a fixed order (a numpy model reproduces it bit for
+ * bit).  Per pixel p with n = n_p samples (spp_map[p], or spp):
+ *   n = 0: empty — outputs 0 and is never a tap.  R, G, B or Q (lum_sumsq) not finite: outputs sum / n and is never a tap.
+ *   otherwise c = sum / n per channel, l = (0.2126 c_R + 0.7152 c_G) + 0.0722 c_B, var = the variance of the mean luminance
+ *   of the adaptive test (spcu_adaptive above: v / n), 0 when n < 2.
+ * Iteration i = 0 .. iterations-1, step h = 2^i:
+ *   var~_p = 3x3 weighted mean of var over the neighbours that are taps (centre 1/4, edges 1/8, corners 1/16, row-major sums);
+ *   taps q = p + h (dx, dy), dx, dy in -2..2, row-major, skipped outside the image or when not a tap;
+ *   k = b[dx] b[dy], b = (1/16, 1/4, 3/8, 1/4, 1/16); the centre's w = k; for another tap:
+ *     classes of p and q differ (geometry hit, light hit, miss): w = 0; else
+ *     both geometry: w_n = max(0, (n_x n'_x + n_y n'_y) + n_z n'_z)^128 (seven squarings),
+ *                    a_z = |z_p - z_q| / ((sigma_z z_p) (h max(|dx|, |dy|))),  a_a = max_c |alb_p,c - alb_q,c| / sigma_a;
+ *     otherwise w_n = 1, a_z = a_a = 0;
+ *     a_l = |l_p - l_q| / (sigma_l sqrt(var~_p) + 1e-4);   w = (k w_n) / (((1 + a_l a_l) + a_z a_z) + a_a a_a);
+ *   S_c += w c_q, S_w += w, S_v += (w w) var_q;  c' = S_c / S_w, var' = S_v / (S_w S_w), l' from c'.
+ * The output is c' after the last iteration: the denoised MEAN colour out[(y*w+x)*3+c]. */
+typedef struct spcu_denoise_params {
+    uint32_t iterations; /* 1..8; iteration i uses step 2^i                        */
+    float    sigma_l;    /* luminance, in standard deviations; finite, > 0        */
+    float    sigma_z;    /* relative depth change per pixel of offset; finite, > 0 */
+    float    sigma_a;    /* albedo difference; finite, > 0                         */
+} spcu_denoise_params;
+/* From a frame's sums (host buffers of the image's size; spp_map NULL = every pixel has `spp` samples).  The guides are
+ * computed inside from the uploaded scene.  Outputs overwritten.  SPCU_ERR_INVALID for parameters outside the ranges above,
+ * lum_sumsq NULL, or spp 0 without a map; the context stays usable. */
+int spcu_denoise(spcu_ctx* ctx, const float* rgb_sum, const float* lum_sumsq, const uint32_t* spp_map, uint32_t spp,
+                 const spcu_denoise_params* p, float* out);
+/* Same on DEVICE buffers, enqueued on `stream` (cudaStream_t as void*, NULL = default stream); d_out may be d_rgb_sum. */
+int spcu_denoise_device(spcu_ctx* ctx, const float* d_rgb_sum, const float* d_lum_sumsq, const uint32_t* d_spp_map,
+                        uint32_t spp, const spcu_denoise_params* p, float* d_out, void* stream);
+
 /* ---- multi-GPU: accumulators summed into rank 0 with NCCL over NVLink (SURVEY.md §8e) ------------------------------------
  * The scene is replicated (every rank uploads it), the work is partitioned by spcu_partition (tiles or sample ranges), there
  * is no exchange during tracing; ONE ncclReduce(sum, root 0) per accumulator ends a frame.  Replaces nothing in the reference

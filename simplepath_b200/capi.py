@@ -107,6 +107,21 @@ class Adaptive(C.Structure):
                 ("radius", C.c_uint32)]
 
 
+class Guide(C.Structure):
+    """spcu_guide: first-hit guide record of a pixel (include/spcu.h)."""
+    _fields_ = [("normal", C.c_float * 3), ("depth", C.c_float), ("albedo", C.c_float * 3), ("id", C.c_int32)]
+
+
+class DenoiseParams(C.Structure):
+    """spcu_denoise_params: parameters of spcu_denoise (include/spcu.h)."""
+    _fields_ = [("iterations", C.c_uint32), ("sigma_l", C.c_float), ("sigma_z", C.c_float), ("sigma_a", C.c_float)]
+
+
+GUIDE_DTYPE = np.dtype([("normal", "<f4", 3), ("depth", "<f4"), ("albedo", "<f4", 3), ("id", "<i4")])
+assert GUIDE_DTYPE.itemsize == C.sizeof(Guide) == 32
+DENOISE_DEFAULTS = {"iterations": 5, "sigma_l": 8.0, "sigma_z": 0.1, "sigma_a": 0.1}  # DESIGN.md §12, profiles/r07a
+
+
 class StageTime(C.Structure):
     _fields_ = [("name", C.c_char * 24), ("launches", C.c_uint64), ("items", C.c_uint64), ("ms", C.c_float),
                 ("traverses", C.c_uint32)]
@@ -122,6 +137,7 @@ EXPORTS = [
     "spcu_comm_unique_id", "spcu_comm_init_rank", "spcu_comm_init_all", "spcu_comm_destroy", "spcu_comm_rank", "spcu_comm_size",
     "spcu_reduce_to_root", "spcu_render_frame_reduced",
     "spcu_render_adaptive", "spcu_render_adaptive_device", "spcu_pack_image_counts",
+    "spcu_render_guides", "spcu_render_guides_device", "spcu_denoise", "spcu_denoise_device",
 ]
 NCCL_ID_BYTES = 128
 OPT_COUNT_NODES, OPT_STAGE_TIMING, OPT_PIPELINE, OPT_TRAVERSAL, OPT_GENERIC_KERNELS, OPT_BATCH_LANES = 0, 1, 2, 3, 4, 5
@@ -221,6 +237,14 @@ def load(path: Path | str | None = None) -> C.CDLL:
     lib.spcu_render_adaptive_device.argtypes = [vp, C.POINTER(Partition), C.POINTER(Adaptive), vp, vp, vp, C.POINTER(C.c_uint32),
                                                 C.POINTER(Stats), vp]
     lib.spcu_render_adaptive_device.restype = C.c_int
+    lib.spcu_render_guides.argtypes = [vp, vp]
+    lib.spcu_render_guides.restype = C.c_int
+    lib.spcu_render_guides_device.argtypes = [vp, vp, vp]
+    lib.spcu_render_guides_device.restype = C.c_int
+    lib.spcu_denoise.argtypes = [vp, vp, vp, vp, C.c_uint32, C.POINTER(DenoiseParams), vp]
+    lib.spcu_denoise.restype = C.c_int
+    lib.spcu_denoise_device.argtypes = [vp, vp, vp, vp, C.c_uint32, C.POINTER(DenoiseParams), vp, vp]
+    lib.spcu_denoise_device.restype = C.c_int
     lib.spcu_render_image.argtypes = [vp, C.POINTER(Partition), C.c_uint32, vp, C.POINTER(Stats)]
     lib.spcu_render_image.restype = C.c_int
     lib.spcu_triangle_bounds.argtypes = [vp, vp, C.c_uint32, vp]
@@ -520,6 +544,35 @@ class Context:
         stats = st.as_dict()
         stats["passes"] = passes.value
         return rgb, sq, spp_map, stats
+
+    def render_guides(self) -> np.ndarray:
+        """First-hit guide records of sample 0's camera rays (spcu_render_guides): structured array [H, W] of GUIDE_DTYPE."""
+        out = np.empty((self.height, self.width), dtype=GUIDE_DTYPE)
+        self._check(self.lib.spcu_render_guides(self.h, _ptr(out)), "spcu_render_guides")
+        return out
+
+    def denoise(self, rgb_sum, lum_sumsq, spp, iterations: int = DENOISE_DEFAULTS["iterations"],
+                sigma_l: float = DENOISE_DEFAULTS["sigma_l"], sigma_z: float = DENOISE_DEFAULTS["sigma_z"],
+                sigma_a: float = DENOISE_DEFAULTS["sigma_a"]) -> np.ndarray:
+        """Denoised mean colour [H, W, 3] of a frame's sums (spcu_denoise).  spp: the samples of every pixel (int), or the
+        per-pixel counts [H, W] of render_adaptive.  pack_image(result, 1, fmt) packs it."""
+        rgb_sum = np.ascontiguousarray(rgb_sum, dtype=np.float32)
+        sq = None if lum_sumsq is None else np.ascontiguousarray(lum_sumsq, dtype=np.float32)
+        h, w = rgb_sum.shape[:2]
+        if (h, w) != (self.height, self.width) or (sq is not None and sq.shape != (h, w)):
+            raise ValueError(f"sums of shape {rgb_sum.shape} for a {self.height}x{self.width} scene")
+        counts = None
+        if isinstance(spp, np.ndarray):
+            counts = np.ascontiguousarray(spp, dtype=np.uint32)
+            if counts.shape != (h, w):
+                raise ValueError(f"spp map of shape {counts.shape} for a {h}x{w} image")
+            spp = 0
+        out = np.empty((h, w, 3), dtype=np.float32)
+        p = DenoiseParams(iterations, sigma_l, sigma_z, sigma_a)
+        self._check(self.lib.spcu_denoise(self.h, _ptr(rgb_sum), _ptr(sq) if sq is not None else None,
+                                          _ptr(counts) if counts is not None else None, spp, C.byref(p), _ptr(out)),
+                    "spcu_denoise")
+        return out
 
     def render_image(self, part: Partition, fmt: int):
         """Render + pack on the device: (packed image [H, W, 3], stats)."""

@@ -3,6 +3,7 @@
 // with --fmad=false and without fast-math (Makefile), and every operation of the test is an explicitly rounded intrinsic, so
 // that a float32 numpy model (simplepath_b200/adaptive.py) reproduces every decision bit for bit.
 #include "ctx.h"
+#include "pixel_stats.cuh"
 
 using namespace spcu;
 
@@ -17,12 +18,8 @@ __device__ __forceinline__ bool converged(const float* __restrict__ rgb_sum, con
                                           float nf, float rel_error, float abs_floor)
 {
     const float R = rgb_sum[3 * pix + 0], G = rgb_sum[3 * pix + 1], B = rgb_sum[3 * pix + 2], Q = lum_sumsq[pix];
-    // luminance() of shade.cuh, one rounding per operation
-    const float L   = __fadd_rn(__fadd_rn(__fmul_rn(0.2126f, R), __fmul_rn(0.7152f, G)), __fmul_rn(0.0722f, B));
-    const float m   = __fdiv_rn(L, nf);
-    const float d   = __fsub_rn(__fdiv_rn(Q, nf), __fmul_rn(m, m));
-    const float v   = d > 0.0f ? __fmul_rn(d, __fdiv_rn(nf, __fsub_rn(nf, 1.0f))) : 0.0f;
-    const float se2 = __fdiv_rn(v, nf);
+    float       m;
+    const float se2 = mean_lum_variance(R, G, B, Q, nf, m);
     const float t   = __fmul_rn(rel_error, __fadd_rn(m, abs_floor));
     return isfinite(R) && isfinite(G) && isfinite(B) && isfinite(Q) && se2 <= __fmul_rn(t, t);
 }

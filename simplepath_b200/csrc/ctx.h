@@ -126,6 +126,8 @@ struct spcu_ctx
     // neighbourhood test (radius > 0), and the call's event pair
     spcu::DevBuf              ad_list[2], ad_spp_map, ad_sq, ad_scratch, ad_mask;
     cudaEvent_t               ad_ev[2] = { nullptr, nullptr };
+    // denoising (spcu_denoise): the guide buffers and the ping-pong colour / variance buffers of the filter's iterations
+    spcu::DevBuf              dn_guides, dn_col[2], dn_var[2];
     void*                     stage[2]    = { nullptr, nullptr }; // page-locked staging of large host->device copies
     cudaEvent_t               stage_ev[2] = { nullptr, nullptr };
     bool                      stage_busy[2] = { false, false };

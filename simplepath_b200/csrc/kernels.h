@@ -139,6 +139,15 @@ cudaError_t launch_adaptive_compact(const uint32_t* d_list, uint32_t n, const fl
 // d_spp_map[d_list[i]] = value for i < n
 cudaError_t launch_adaptive_fill(const uint32_t* d_list, uint32_t n, uint32_t value, uint32_t* d_spp_map, cudaStream_t st);
 
+// ---- denoise_kernels.cu (exact float32 arithmetic: --fmad=false, no fast-math) -------------------------------------------------
+// spcu_render_guides: d_out[pix] for every pixel of the image (spcu_guide, include/spcu.h).  Enqueue only.
+cudaError_t launch_guides(const DScene& s, spcu_guide* d_out, cudaStream_t st);
+// spcu_denoise's filter (include/spcu.h) over width x height pixels: d_col / d_var are the two ping-pong buffers of the
+// iterations (n float4 / n float each), d_out[pix*3+c] the result (may alias d_rgb_sum).  Parameters already checked.  Enqueue only.
+cudaError_t launch_denoise(const spcu_guide* d_guides, const float* d_rgb_sum, const float* d_lum_sumsq, const uint32_t* d_spp_map,
+                           uint32_t spp, uint32_t width, uint32_t height, const spcu_denoise_params& p, float4* d_col[2],
+                           float* d_var[2], float* d_out, cudaStream_t st);
+
 // pixel list of one rank: tiles t with t % stride == offset, 8x8 tiles row major (TileScheduler.h:66-82)
 uint32_t    count_partition_pixels(uint32_t width, uint32_t height, uint32_t tile_offset, uint32_t tile_stride);
 // d_tile_prefix_scratch: one uint32 per owned tile.  Synchronises the stream.

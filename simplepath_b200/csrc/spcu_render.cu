@@ -589,12 +589,12 @@ int sync_and_check_faults(spcu_ctx* c, bool already_checked)
     return faults ? queue_fault(c, faults) : SPCU_OK;
 }
 
-// The host-buffer entry points: device accumulators for the image (c->host_rgb, and c->host_sq `with_sumsq`), zeroed or, to
-// `accumulate`, holding the caller's sums; `render(d_rgb_sum, d_lum_sumsq)` enqueues the call's work on the context's stream;
-// the sums go back to rgb_sum / lum_sumsq where those are not NULL, and the call ends in the fault check.
+// The host-buffer entry points: device accumulators for the image (c->host_rgb, and c->host_sq `with_sumsq`), zeroed or, where
+// rgb_in (and sq_in) are given, holding those host arrays; `render(d_rgb_sum, d_lum_sumsq)` enqueues the call's work on the
+// context's stream; the accumulators go back to rgb_sum / lum_sumsq where those are not NULL, and the call ends in the fault check.
 template <typename Render>
-int host_buffer_render(spcu_ctx* c, bool with_sumsq, bool accumulate, float* rgb_sum, float* lum_sumsq, bool already_checked,
-                       Render&& render)
+int host_buffer_render(spcu_ctx* c, bool with_sumsq, const float* rgb_in, const float* sq_in, float* rgb_sum, float* lum_sumsq,
+                       bool already_checked, Render&& render)
 {
     const size_t sq_bytes = static_cast<size_t>(c->ds.width) * c->ds.height * sizeof(float), rgb_bytes = 3 * sq_bytes;
     CK(c, c->host_rgb.reserve(rgb_bytes));
@@ -603,9 +603,9 @@ int host_buffer_render(spcu_ctx* c, bool with_sumsq, bool accumulate, float* rgb
         CK(c, c->host_sq.reserve(sq_bytes));
         d_sq = c->host_sq.as<float>();
     }
-    if (accumulate) {
-        CK(c, cudaMemcpyAsync(c->host_rgb.p, rgb_sum, rgb_bytes, cudaMemcpyHostToDevice, c->stream));
-        if (d_sq) CK(c, cudaMemcpyAsync(d_sq, lum_sumsq, sq_bytes, cudaMemcpyHostToDevice, c->stream));
+    if (rgb_in) {
+        CK(c, cudaMemcpyAsync(c->host_rgb.p, rgb_in, rgb_bytes, cudaMemcpyHostToDevice, c->stream));
+        if (d_sq) CK(c, cudaMemcpyAsync(d_sq, sq_in, sq_bytes, cudaMemcpyHostToDevice, c->stream));
     } else {
         CK(c, cudaMemsetAsync(c->host_rgb.p, 0, rgb_bytes, c->stream));
         if (d_sq) CK(c, cudaMemsetAsync(d_sq, 0, sq_bytes, c->stream));
@@ -614,6 +614,43 @@ int host_buffer_render(spcu_ctx* c, bool with_sumsq, bool accumulate, float* rgb
     if (rgb_sum) CK(c, cudaMemcpyAsync(rgb_sum, c->host_rgb.p, rgb_bytes, cudaMemcpyDeviceToHost, c->stream));
     if (lum_sumsq && d_sq) CK(c, cudaMemcpyAsync(lum_sumsq, d_sq, sq_bytes, cudaMemcpyDeviceToHost, c->stream));
     return sync_and_check_faults(c, already_checked);
+}
+
+// spcu_denoise(_device): guides into c->dn_guides, then the filter through the ping-pong buffers c->dn_col / c->dn_var.  Those
+// are context scratch like the renders' (wait_for_scratch): a call on another stream starts after the previous user is done.
+int denoise_impl(spcu_ctx* c, const float* d_rgb_sum, const float* d_lum_sumsq, const uint32_t* d_spp_map, uint32_t spp,
+                 const spcu_denoise_params* p, float* d_out, cudaStream_t st)
+{
+    if (int rc = need_scene(c); rc != SPCU_OK) return rc;
+    if (!p || !d_rgb_sum || !d_lum_sumsq || !d_out) {
+        return fail(c, SPCU_ERR_INVALID, "parameters, rgb_sum, lum_sumsq or out is NULL");
+    }
+    if (p->iterations < 1 || p->iterations > 8 || !std::isfinite(p->sigma_l) || !(p->sigma_l > 0.0f) || !std::isfinite(p->sigma_z) ||
+        !(p->sigma_z > 0.0f) || !std::isfinite(p->sigma_a) || !(p->sigma_a > 0.0f)) {
+        return fail(c, SPCU_ERR_INVALID, "bad denoise parameters: iterations %u (1..8), sigma_l %g, sigma_z %g, sigma_a %g (finite, > 0)",
+                    p->iterations, p->sigma_l, p->sigma_z, p->sigma_a);
+    }
+    if (!d_spp_map && spp == 0) {
+        return fail(c, SPCU_ERR_INVALID, "spp is 0 and there is no spp map");
+    }
+    const size_t n = static_cast<size_t>(c->ds.width) * c->ds.height;
+    CK(c, c->dn_guides.reserve(n * sizeof(spcu_guide)));
+    float4* col[2];
+    float*  var[2];
+    for (int k = 0; k < 2; ++k) {
+        CK(c, c->dn_col[k].reserve(n * sizeof(float4)));
+        CK(c, c->dn_var[k].reserve(n * sizeof(float)));
+        col[k] = c->dn_col[k].as<float4>();
+        var[k] = c->dn_var[k].as<float>();
+    }
+    if (int rc = wait_for_scratch(c, st); rc != SPCU_OK) return rc;
+    CK(c, launch_guides(c->ds, c->dn_guides.as<spcu_guide>(), st));
+    CK(c, launch_denoise(c->dn_guides.as<spcu_guide>(), d_rgb_sum, d_lum_sumsq, d_spp_map, spp, c->ds.width, c->ds.height, *p, col, var,
+                         d_out, st));
+    CK(c, cudaEventRecord(c->ev1, st));
+    c->scratch_in_use = true;
+    c->scratch_stream = st;
+    return SPCU_OK;
 }
 
 } // namespace
@@ -643,7 +680,7 @@ int spcu_render_adaptive(spcu_ctx* c, const spcu_partition* part, const spcu_ada
     const size_t map_bytes = static_cast<size_t>(c->ds.width) * c->ds.height * sizeof(uint32_t);
     CK(c, c->ad_spp_map.reserve(map_bytes));
     // (every pass's fault counter has been read)
-    return host_buffer_render(c, true, false, rgb_sum, lum_sumsq, true, [&](float* d_rgb_sum, float* d_sq) {
+    return host_buffer_render(c, true, nullptr, nullptr, rgb_sum, lum_sumsq, true, [&](float* d_rgb_sum, float* d_sq) {
         if (int rc = adaptive_impl(c, part, ad, d_rgb_sum, d_sq, c->ad_spp_map.as<uint32_t>(), n_passes, stats, nullptr, false);
             rc != SPCU_OK) {
             return rc;
@@ -659,8 +696,60 @@ int spcu_render(spcu_ctx* c, const spcu_partition* part, float* rgb_sum, float* 
     if (!rgb_sum) {
         return fail(c, SPCU_ERR_INVALID, "rgb_sum is NULL");
     }
-    return host_buffer_render(c, lum_sumsq != nullptr, true, rgb_sum, lum_sumsq, stats != nullptr, [&](float* d_rgb_sum, float* d_sq) {
+    return host_buffer_render(c, lum_sumsq != nullptr, rgb_sum, lum_sumsq, rgb_sum, lum_sumsq, stats != nullptr, [&](float* d_rgb_sum, float* d_sq) {
         return render_impl(c, part, d_rgb_sum, d_sq, stats, nullptr, false);
+    });
+}
+
+int spcu_render_guides_device(spcu_ctx* c, spcu_guide* d_out, void* stream)
+{
+    if (int rc = need_scene(c); rc != SPCU_OK) return rc;
+    if (!d_out) {
+        return fail(c, SPCU_ERR_INVALID, "out is NULL");
+    }
+    CK(c, launch_guides(c->ds, d_out, static_cast<cudaStream_t>(stream)));
+    return SPCU_OK;
+}
+
+int spcu_render_guides(spcu_ctx* c, spcu_guide* out)
+{
+    if (int rc = need_scene(c); rc != SPCU_OK) return rc;
+    if (!out) {
+        return fail(c, SPCU_ERR_INVALID, "out is NULL");
+    }
+    const size_t bytes = static_cast<size_t>(c->ds.width) * c->ds.height * sizeof(spcu_guide);
+    CK(c, c->dn_guides.reserve(bytes));
+    if (int rc = wait_for_scratch(c, c->stream); rc != SPCU_OK) return rc;
+    CK(c, launch_guides(c->ds, c->dn_guides.as<spcu_guide>(), c->stream));
+    CK(c, cudaMemcpyAsync(out, c->dn_guides.p, bytes, cudaMemcpyDeviceToHost, c->stream));
+    CK(c, cudaStreamSynchronize(c->stream));
+    return SPCU_OK;
+}
+
+int spcu_denoise_device(spcu_ctx* c, const float* d_rgb_sum, const float* d_lum_sumsq, const uint32_t* d_spp_map, uint32_t spp,
+                        const spcu_denoise_params* p, float* d_out, void* stream)
+{
+    return denoise_impl(c, d_rgb_sum, d_lum_sumsq, d_spp_map, spp, p, d_out, static_cast<cudaStream_t>(stream));
+}
+
+// The sums go up into the host-buffer accumulators, the filter writes the mean colour over the colour sums there, and that
+// buffer comes back to `out`.
+int spcu_denoise(spcu_ctx* c, const float* rgb_sum, const float* lum_sumsq, const uint32_t* spp_map, uint32_t spp,
+                 const spcu_denoise_params* p, float* out)
+{
+    if (int rc = need_scene(c); rc != SPCU_OK) return rc;
+    if (!rgb_sum || !lum_sumsq || !out) {
+        return fail(c, SPCU_ERR_INVALID, "rgb_sum, lum_sumsq or out is NULL");
+    }
+    const size_t n = static_cast<size_t>(c->ds.width) * c->ds.height;
+    return host_buffer_render(c, true, rgb_sum, lum_sumsq, out, nullptr, true, [&](float* d_rgb_sum, float* d_sq) {
+        uint32_t* d_map = nullptr;
+        if (spp_map) {
+            CK(c, c->ad_spp_map.reserve(n * sizeof(uint32_t)));
+            d_map = c->ad_spp_map.as<uint32_t>();
+            CK(c, cudaMemcpyAsync(d_map, spp_map, n * sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
+        }
+        return denoise_impl(c, d_rgb_sum, d_sq, d_map, spp, p, d_rgb_sum, c->stream);
     });
 }
 
@@ -675,7 +764,7 @@ int spcu_render_frame(spcu_ctx* c, const spcu_partition* part, float* rgb_sum, f
     if (!rgb_sum) {
         return fail(c, SPCU_ERR_INVALID, "rgb_sum is NULL");
     }
-    return host_buffer_render(c, lum_sumsq != nullptr, false, rgb_sum, lum_sumsq, stats != nullptr, [&](float* d_rgb_sum, float* d_sq) {
+    return host_buffer_render(c, lum_sumsq != nullptr, nullptr, nullptr, rgb_sum, lum_sumsq, stats != nullptr, [&](float* d_rgb_sum, float* d_sq) {
         return render_impl(c, part, d_rgb_sum, d_sq, stats, nullptr, false);
     });
 }
@@ -688,7 +777,7 @@ int spcu_render_frame_reduced(spcu_ctx* c, const spcu_partition* part, int with_
     if (root && (!rgb_sum || (with_sumsq && !lum_sumsq))) {
         return fail(c, SPCU_ERR_INVALID, "rank 0 needs the host buffers");
     }
-    return host_buffer_render(c, with_sumsq != 0, false, root ? rgb_sum : nullptr, root ? lum_sumsq : nullptr, stats != nullptr,
+    return host_buffer_render(c, with_sumsq != 0, nullptr, nullptr, root ? rgb_sum : nullptr, root ? lum_sumsq : nullptr, stats != nullptr,
                               [&](float* d_rgb_sum, float* d_sq) {
                                   if (int rc = render_impl(c, part, d_rgb_sum, d_sq, stats, nullptr, false); rc != SPCU_OK) return rc;
                                   return spcu_reduce_to_root(c, d_rgb_sum, d_sq, c->stream);
@@ -701,7 +790,7 @@ int spcu_render_image(spcu_ctx* c, const spcu_partition* part, uint32_t format, 
     if (!part || part->sample_end <= part->sample_begin) {
         return fail(c, SPCU_ERR_INVALID, "empty sample range");
     }
-    if (int rc = host_buffer_render(c, false, false, nullptr, nullptr, stats != nullptr,
+    if (int rc = host_buffer_render(c, false, nullptr, nullptr, nullptr, nullptr, stats != nullptr,
                                     [&](float* d_rgb_sum, float*) { return render_impl(c, part, d_rgb_sum, nullptr, stats, nullptr, false); });
         rc != SPCU_OK) {
         return rc;

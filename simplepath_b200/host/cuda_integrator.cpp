@@ -128,7 +128,7 @@ CudaIntegrator::~CudaIntegrator() = default;
 
 // Sum of radiance samples per pixel, row major W*H*3.
 void CudaIntegrator::render_sum(const Scene& scene, unsigned spp, std::vector<float>& rgb_sum, std::vector<std::uint32_t>* spp_map,
-                                float rel_error, std::uint32_t radius) const
+                                float rel_error, std::uint32_t radius, std::vector<float>* lum_sumsq) const
 {
     if (m_devices.empty()) {
         for (int i = 0; i < m_options.n_devices; ++i) {
@@ -219,6 +219,11 @@ void CudaIntegrator::render_sum(const Scene& scene, unsigned spp, std::vector<fl
     }
     const std::size_t n = static_cast<std::size_t>(scene.image_width) * scene.image_height * 3u;
     rgb_sum.resize(n); // spcu_render_frame overwrites: nothing to zero, nothing to upload
+    float* sq = nullptr;
+    if (lum_sumsq) {
+        lum_sumsq->resize(n / 3u);
+        sq = lum_sumsq->data();
+    }
 
     const auto           n_dev = static_cast<std::uint32_t>(m_devices.size());
     const std::uint32_t  code  = integrator_code(m_options.inner);
@@ -229,7 +234,7 @@ void CudaIntegrator::render_sum(const Scene& scene, unsigned spp, std::vector<fl
         const spcu_partition part{ 0u, 1u, 0u, spp, spp, code, m_options.seed };
         spp_map->resize(n / 3u);
         std::uint32_t passes = 0;
-        m_devices[0]->check(spcu_render_adaptive(m_devices[0]->ctx, &part, &ad, rgb_sum.data(), nullptr, spp_map->data(), &passes, &m_stats),
+        m_devices[0]->check(spcu_render_adaptive(m_devices[0]->ctx, &part, &ad, rgb_sum.data(), sq, spp_map->data(), &passes, &m_stats),
                             "spcu_render_adaptive");
         std::uint64_t early = 0;
         for (const std::uint32_t c : *spp_map) {
@@ -247,7 +252,8 @@ void CudaIntegrator::render_sum(const Scene& scene, unsigned spp, std::vector<fl
     // device 0 by ncclReduce over NVLink (spcu_render_frame_reduced) and ONE frame crosses to the host.
     on_every_device([&](std::size_t k) {
         const spcu_partition part{ static_cast<std::uint32_t>(k), n_dev, 0u, spp, spp, code, m_options.seed };
-        m_devices[k]->check(spcu_render_frame_reduced(m_devices[k]->ctx, &part, 0, k == 0 ? rgb_sum.data() : nullptr, nullptr, &stats[k]),
+        m_devices[k]->check(spcu_render_frame_reduced(m_devices[k]->ctx, &part, sq ? 1 : 0, k == 0 ? rgb_sum.data() : nullptr,
+                                                      k == 0 ? sq : nullptr, &stats[k]),
                             "spcu_render_frame_reduced");
     });
     m_stats = stats[0];
@@ -267,7 +273,16 @@ bool CudaIntegrator::render_frame(const Scene& scene, unsigned spp, Image& image
     if (spp == 0) {
         throw std::runtime_error("CudaIntegrator: samples per pixel must be >= 1");
     }
+    // SPCU_DENOISE=1: the image is the denoised mean (spcu_denoise on device 0, with Context.denoise's defaults)
+    bool denoise = false;
+    if (const char* d = std::getenv("SPCU_DENOISE"); d && *d) {
+        if (std::string(d) != "1") {
+            throw std::runtime_error(std::string("CudaIntegrator: SPCU_DENOISE must be 1 (or unset), not '") + d + "'");
+        }
+        denoise = true;
+    }
     std::vector<float>         sum;
+    std::vector<float>         sumsq; // SPCU_DENOISE: the filter's variance estimate needs the sums of squared luminance
     std::vector<std::uint32_t> counts; // SPCU_ADAPTIVE=<rel_error>: --samples is the budget, each pixel has its own count
     if (const char* adaptive = std::getenv("SPCU_ADAPTIVE"); adaptive && *adaptive) {
         char*       end = nullptr;
@@ -288,12 +303,25 @@ bool CudaIntegrator::render_frame(const Scene& scene, unsigned spp, Image& image
         if (m_options.n_devices > 1) {
             throw std::runtime_error("CudaIntegrator: SPCU_ADAPTIVE renders on one device; unset SPCU_DEVICES or set it to 1");
         }
-        render_sum(scene, spp, sum, &counts, rel, radius);
+        render_sum(scene, spp, sum, &counts, rel, radius, denoise ? &sumsq : nullptr);
     } else {
-        render_sum(scene, spp, sum);
+        render_sum(scene, spp, sum, nullptr, 0.0f, 0, denoise ? &sumsq : nullptr);
     }
     const auto  w   = static_cast<std::size_t>(scene.image_width);
     const auto  h   = static_cast<std::size_t>(scene.image_height);
+    if (denoise) { // after the reduction: device 0 holds the scene, the frame's sums go back to it once more
+        const spcu_denoise_params p{ 5u, 8.0f, 0.1f, 0.1f }; // Context.denoise's defaults (DESIGN.md §12)
+        std::vector<float>        mean(sum.size());
+        const auto                t0 = std::chrono::steady_clock::now();
+        m_devices[0]->check(spcu_denoise(m_devices[0]->ctx, sum.data(), sumsq.data(), counts.empty() ? nullptr : counts.data(), spp, &p,
+                                         mean.data()),
+                            "spcu_denoise");
+        const double ms = 1e3 * std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
+        std::fprintf(stderr, "CudaIntegrator: denoised (%u iterations, sigma_l %g, sigma_z %g, sigma_a %g) in %.2f ms\n", p.iterations,
+                     static_cast<double>(p.sigma_l), static_cast<double>(p.sigma_z), static_cast<double>(p.sigma_a), ms);
+        sum.swap(mean);
+        counts.assign(w * h, 1u); // the means, divided by 1 below (exact)
+    }
     for (std::size_t y = 0; y < h; ++y) {
         for (std::size_t x = 0; x < w; ++x) {
             const float* p = &sum[(y * w + x) * 3u];

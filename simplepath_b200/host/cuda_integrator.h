@@ -54,9 +54,10 @@ private:
     RGB integrate_impl(const Ray&, const Scene& scene, MemoryArena&, Sampler&, const Point2& pixel_coords) const override;
 
     // spp_map != NULL: adaptive sampling (spcu_render_adaptive, one device) to the standard error `rel_error` with the window
-    // radius `radius` of the stopping rule, spp the budget; *spp_map = the samples each pixel received
+    // radius `radius` of the stopping rule, spp the budget; *spp_map = the samples each pixel received.
+    // lum_sumsq != NULL: also the per-pixel sums of squared luminance (W*H), which the denoiser needs
     void render_sum(const Scene& scene, unsigned spp, std::vector<float>& rgb_sum, std::vector<std::uint32_t>* spp_map = nullptr,
-                    float rel_error = 0.0f, std::uint32_t radius = 0) const;
+                    float rel_error = 0.0f, std::uint32_t radius = 0, std::vector<float>* lum_sumsq = nullptr) const;
 
     struct Device;
     Options                              m_options;
