@@ -390,6 +390,27 @@ int spcu_denoise(spcu_ctx* ctx, const float* rgb_sum, const float* lum_sumsq, co
 int spcu_denoise_device(spcu_ctx* ctx, const float* d_rgb_sum, const float* d_lum_sumsq, const uint32_t* d_spp_map,
                         uint32_t spp, const spcu_denoise_params* p, float* d_out, void* stream);
 
+/* The energy-conserving (flux) form of the same filter.  The weights above are not symmetric (a_l is scaled by var~_p, a_z by
+ * z_p), so a bright pixel with a large variance takes in its dim neighbours while they reject it, and its energy is lost.
+ * Here neighbours exchange colour in pairs: what p gains from q, q loses to p.  Pixel data, classes, taps, var~ and the
+ * ranges of the parameters are as above; per iteration i (step h = 2^i), for taps p != q at offset h (dx, dy):
+ *   w_pq = 0 when the classes differ; else with k = b[dx] b[dy] and m = max(|dx|, |dy|):
+ *     both geometry: w_n as above, a_z = |z_p - z_q| / ((sigma_z min(z_p, z_q)) (h m)), a_a as above;
+ *     otherwise w_n = 1, a_z = a_a = 0;
+ *     a_l = |l_p - l_q| / (sigma_l sqrt(max(var~_p, var~_q)) + 1e-4);   w_pq = (k w_n) / (((1 + a_l a_l) + a_z a_z) + a_a a_a).
+ *   Every operand pair meets in a commutative operation, min, max or |a - b|, so w_pq and w_qp have the same bits.
+ *   W_p = over p's taps in row-major order, 9/64 for the centre and w_pq for every other tap (the centre's k plus the pairs);
+ *   alpha_pq = w_pq / max(W_p, W_q) (symmetric), f_pq,c = alpha_pq (c_q,c - c_p,c) = -f_qp,c exactly;
+ *   over the taps q != p in row-major order: S_c += f_pq,c, A += alpha_pq, S_v += (alpha_pq alpha_pq) var_q;
+ *   c'_p = c_p + S_c, a_0 = 1 - A, var'_p = (a_0 a_0) var_p + S_v, l' from c'.  Pixels that are no taps pass through.
+ * So the sum of every colour channel over the image is kept up to the rounding of each pixel's sums; a constant image comes
+ * back bit for bit; and as A <= 1 - (9/64) / W_p, each output is a convex combination of the pixel and its taps.  Arguments,
+ * outputs, rejections and the in-place allowance are spcu_denoise(_device)'s; spcu_denoise_params is shared. */
+int spcu_denoise_conserving(spcu_ctx* ctx, const float* rgb_sum, const float* lum_sumsq, const uint32_t* spp_map, uint32_t spp,
+                            const spcu_denoise_params* p, float* out);
+int spcu_denoise_conserving_device(spcu_ctx* ctx, const float* d_rgb_sum, const float* d_lum_sumsq, const uint32_t* d_spp_map,
+                                   uint32_t spp, const spcu_denoise_params* p, float* d_out, void* stream);
+
 /* ---- multi-GPU: accumulators summed into rank 0 with NCCL over NVLink (SURVEY.md §8e) ------------------------------------
  * The scene is replicated (every rank uploads it), the work is partitioned by spcu_partition (tiles or sample ranges), there
  * is no exchange during tracing; ONE ncclReduce(sum, root 0) per accumulator ends a frame.  Replaces nothing in the reference

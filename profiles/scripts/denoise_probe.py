@@ -9,8 +9,12 @@
   - the fixed-spp render time (host clock around spcu_render_frame, median of --reps) at which a raw render reaches each
     denoised relMSE, interpolated log-log between the fixed renders around it (null beyond 256 spp), next to the time of the
     denoised frame (render + filter).
+With --conserve it compares the gather form (spcu_denoise) with the energy-conserving flux form (spcu_denoise_conserving)
+instead: device time of guides + filter for both forms at 1080p and 2160p, 3 and 5 iterations; relMSE raw and denoised and
+the mean luminance change at 4 and 16 spp for sigma_l 2 / 4 / 8 and both forms, against the same 512-spp truth.
 Every line carries the GPU's name and power limit.
-    python profiles/scripts/denoise_probe.py --out profiles/r07a_denoise_probe.jsonl"""
+    python profiles/scripts/denoise_probe.py --out profiles/r07a_denoise_probe.jsonl
+    python profiles/scripts/denoise_probe.py --conserve --out profiles/r08a_denoise_conserving_probe.jsonl"""
 import argparse
 import ctypes as C
 import json
@@ -38,6 +42,9 @@ SETTINGS = [dict(iterations=5, sigma_l=4.0, sigma_z=0.1, sigma_a=0.1), dict(iter
             dict(iterations=5, sigma_l=64.0, sigma_z=0.1, sigma_a=0.1)]
 ADAPTIVE = dict(budget=64, min_spp=4, pass_spp=4, rel_error=0.05, abs_floor=0.03, radius=2)
 TRUTH_SPP, SEED, TRUTH_SEED = 512, 20261020, 77
+FORMS = {"gather": "spcu_denoise_device", "conserving": "spcu_denoise_conserving_device"}
+CONSERVE_AT = [4, 16]
+CONSERVE_SIGMA_L = [2.0, 4.0, 8.0]
 
 
 def scaled(flat: FlatSceneData, k: int) -> FlatSceneData:
@@ -82,11 +89,61 @@ def kernel_times(ctx, flat, rgb, sq, spp, reps):
     return res
 
 
+def form_times(ctx, rgb, sq, spp, reps):
+    """Guides + filter device time of both forms at 3 and 5 iterations (defaults otherwise)."""
+    d_rgb = torch.from_numpy(np.ascontiguousarray(rgb)).cuda()
+    d_sq = torch.from_numpy(np.ascontiguousarray(sq)).cuda()
+    d_out = torch.empty_like(d_rgb)
+    stream = C.c_void_p(torch.cuda.current_stream().cuda_stream)
+    res = {}
+    for iterations in (3, 5):
+        p = capi.DenoiseParams(iterations, capi.DENOISE_DEFAULTS["sigma_l"], capi.DENOISE_DEFAULTS["sigma_z"],
+                               capi.DENOISE_DEFAULTS["sigma_a"])
+        for form, fn in FORMS.items():
+            call = getattr(ctx.lib, fn)
+            res[f"{form}_ms_it{iterations}"] = event_ms(lambda: ctx._check(call(
+                ctx.h, C.c_void_p(d_rgb.data_ptr()), C.c_void_p(d_sq.data_ptr()), None, spp, C.byref(p), C.c_void_p(d_out.data_ptr()),
+                stream), fn), reps)
+    return res
+
+
+def conserve_probe(ctx, args, emit):
+    for scene in args.scenes:
+        flat = host.workload(scene)
+        base = {"scene": scene}
+        for k in (1, 2):  # device times at 1080p and 2160p
+            fk = scaled(flat, k) if k > 1 else flat
+            ctx.set_wavefront_size(0)
+            ctx.upload_scene(fk.pointer(), rsequence.jitter_table(4), keepalive=fk)
+            rgb, sq, _ = ctx.render_frame(ctx.partition(spp=4, seed=SEED))
+            emit({**base, "mode": "kernel_time", "width": fk.width, "height": fk.height, "spp": 4,
+                  **form_times(ctx, rgb, sq, 4, args.reps)})
+        ctx.upload_scene(flat.pointer(), rsequence.jitter_table(TRUTH_SPP), keepalive=flat)
+        truth, _, _ = ctx.render_frame(ctx.partition(spp=TRUTH_SPP, seed=TRUTH_SEED), want_sumsq=False)
+        lt = lum(truth.astype(np.float64) / TRUTH_SPP)
+        denom = lt ** 2 + 1e-3
+        base.update(width=flat.width, height=flat.height, pipeline=ctx.resolved_pipeline(), truth_spp=TRUTH_SPP)
+        for spp in CONSERVE_AT:
+            rgb, sq, _ = ctx.render_frame(ctx.partition(spp=TRUTH_SPP, sample_end=spp, seed=SEED))
+            raw_l = lum(rgb.astype(np.float64) / spp)
+            raw = float(((raw_l - lt) ** 2 / denom).mean())
+            for sigma_l in CONSERVE_SIGMA_L:
+                for form in FORMS:
+                    s = dict(capi.DENOISE_DEFAULTS, sigma_l=sigma_l)
+                    out_l = lum(ctx.denoise(rgb, sq, spp, conserve_energy=form == "conserving", **s).astype(np.float64))
+                    e = float(((out_l - lt) ** 2 / denom).mean())
+                    emit({**base, "mode": "denoised", "form": form, "input": f"fixed_{spp}", **s, "relmse_raw": raw,
+                          "relmse_denoised": e, "factor": raw / e, "mean_lum_truth": float(lt.mean()),
+                          "mean_lum_raw": float(raw_l.mean()), "mean_lum_denoised": float(out_l.mean()),
+                          "mean_lum_change": float(out_l.mean() / raw_l.mean() - 1)})
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", required=True)
     ap.add_argument("--reps", type=int, default=5)
     ap.add_argument("--scenes", nargs="*", default=SCENES)
+    ap.add_argument("--conserve", action="store_true", help="compare the gather and the energy-conserving form")
     args = ap.parse_args()
     info = gpu_info()
     ctx = capi.Context(0)
@@ -96,7 +153,9 @@ def main():
             print(line, flush=True)
             f.write(line + "\n")
 
-        for scene in args.scenes:
+        if args.conserve:
+            conserve_probe(ctx, args, emit)
+        for scene in ([] if args.conserve else args.scenes):
             flat = host.workload(scene)
             base = {"scene": scene}
             for k in (1, 2):  # kernel times at 1080p and 2160p

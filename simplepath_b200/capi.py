@@ -138,6 +138,7 @@ EXPORTS = [
     "spcu_reduce_to_root", "spcu_render_frame_reduced",
     "spcu_render_adaptive", "spcu_render_adaptive_device", "spcu_pack_image_counts",
     "spcu_render_guides", "spcu_render_guides_device", "spcu_denoise", "spcu_denoise_device",
+    "spcu_denoise_conserving", "spcu_denoise_conserving_device",
 ]
 NCCL_ID_BYTES = 128
 OPT_COUNT_NODES, OPT_STAGE_TIMING, OPT_PIPELINE, OPT_TRAVERSAL, OPT_GENERIC_KERNELS, OPT_BATCH_LANES = 0, 1, 2, 3, 4, 5
@@ -245,6 +246,10 @@ def load(path: Path | str | None = None) -> C.CDLL:
     lib.spcu_denoise.restype = C.c_int
     lib.spcu_denoise_device.argtypes = [vp, vp, vp, vp, C.c_uint32, C.POINTER(DenoiseParams), vp, vp]
     lib.spcu_denoise_device.restype = C.c_int
+    lib.spcu_denoise_conserving.argtypes = [vp, vp, vp, vp, C.c_uint32, C.POINTER(DenoiseParams), vp]
+    lib.spcu_denoise_conserving.restype = C.c_int
+    lib.spcu_denoise_conserving_device.argtypes = [vp, vp, vp, vp, C.c_uint32, C.POINTER(DenoiseParams), vp, vp]
+    lib.spcu_denoise_conserving_device.restype = C.c_int
     lib.spcu_render_image.argtypes = [vp, C.POINTER(Partition), C.c_uint32, vp, C.POINTER(Stats)]
     lib.spcu_render_image.restype = C.c_int
     lib.spcu_triangle_bounds.argtypes = [vp, vp, C.c_uint32, vp]
@@ -553,9 +558,10 @@ class Context:
 
     def denoise(self, rgb_sum, lum_sumsq, spp, iterations: int = DENOISE_DEFAULTS["iterations"],
                 sigma_l: float = DENOISE_DEFAULTS["sigma_l"], sigma_z: float = DENOISE_DEFAULTS["sigma_z"],
-                sigma_a: float = DENOISE_DEFAULTS["sigma_a"]) -> np.ndarray:
+                sigma_a: float = DENOISE_DEFAULTS["sigma_a"], conserve_energy: bool = False) -> np.ndarray:
         """Denoised mean colour [H, W, 3] of a frame's sums (spcu_denoise).  spp: the samples of every pixel (int), or the
-        per-pixel counts [H, W] of render_adaptive.  pack_image(result, 1, fmt) packs it."""
+        per-pixel counts [H, W] of render_adaptive.  pack_image(result, 1, fmt) packs it.  conserve_energy: the flux form
+        (spcu_denoise_conserving), which keeps every colour channel's sum over the image."""
         rgb_sum = np.ascontiguousarray(rgb_sum, dtype=np.float32)
         sq = None if lum_sumsq is None else np.ascontiguousarray(lum_sumsq, dtype=np.float32)
         h, w = rgb_sum.shape[:2]
@@ -569,9 +575,9 @@ class Context:
             spp = 0
         out = np.empty((h, w, 3), dtype=np.float32)
         p = DenoiseParams(iterations, sigma_l, sigma_z, sigma_a)
-        self._check(self.lib.spcu_denoise(self.h, _ptr(rgb_sum), _ptr(sq) if sq is not None else None,
-                                          _ptr(counts) if counts is not None else None, spp, C.byref(p), _ptr(out)),
-                    "spcu_denoise")
+        name = "spcu_denoise_conserving" if conserve_energy else "spcu_denoise"
+        self._check(getattr(self.lib, name)(self.h, _ptr(rgb_sum), _ptr(sq) if sq is not None else None,
+                                            _ptr(counts) if counts is not None else None, spp, C.byref(p), _ptr(out)), name)
         return out
 
     def render_image(self, part: Partition, fmt: int):

@@ -147,6 +147,12 @@ cudaError_t launch_guides(const DScene& s, spcu_guide* d_out, cudaStream_t st);
 cudaError_t launch_denoise(const spcu_guide* d_guides, const float* d_rgb_sum, const float* d_lum_sumsq, const uint32_t* d_spp_map,
                            uint32_t spp, uint32_t width, uint32_t height, const spcu_denoise_params& p, float4* d_col[2],
                            float* d_var[2], float* d_out, cudaStream_t st);
+// spcu_denoise_conserving's flux form of the filter, with the same buffers plus n floats each for var~ (d_var_pf) and the weight
+// sums W (d_wsum).  Parameters already checked.  Enqueue only.
+cudaError_t launch_denoise_conserving(const spcu_guide* d_guides, const float* d_rgb_sum, const float* d_lum_sumsq,
+                                      const uint32_t* d_spp_map, uint32_t spp, uint32_t width, uint32_t height,
+                                      const spcu_denoise_params& p, float4* d_col[2], float* d_var[2], float* d_var_pf, float* d_wsum,
+                                      float* d_out, cudaStream_t st);
 
 // pixel list of one rank: tiles t with t % stride == offset, 8x8 tiles row major (TileScheduler.h:66-82)
 uint32_t    count_partition_pixels(uint32_t width, uint32_t height, uint32_t tile_offset, uint32_t tile_stride);

@@ -616,10 +616,11 @@ int host_buffer_render(spcu_ctx* c, bool with_sumsq, const float* rgb_in, const 
     return sync_and_check_faults(c, already_checked);
 }
 
-// spcu_denoise(_device): guides into c->dn_guides, then the filter through the ping-pong buffers c->dn_col / c->dn_var.  Those
-// are context scratch like the renders' (wait_for_scratch): a call on another stream starts after the previous user is done.
+// spcu_denoise(_device) and, `conserve`, spcu_denoise_conserving(_device): guides into c->dn_guides, then the filter through
+// the ping-pong buffers c->dn_col / c->dn_var (and, for the flux form, c->dn_var_pf / c->dn_wsum).  Those are context scratch
+// like the renders' (wait_for_scratch): a call on another stream starts after the previous user is done.
 int denoise_impl(spcu_ctx* c, const float* d_rgb_sum, const float* d_lum_sumsq, const uint32_t* d_spp_map, uint32_t spp,
-                 const spcu_denoise_params* p, float* d_out, cudaStream_t st)
+                 const spcu_denoise_params* p, float* d_out, cudaStream_t st, bool conserve)
 {
     if (int rc = need_scene(c); rc != SPCU_OK) return rc;
     if (!p || !d_rgb_sum || !d_lum_sumsq || !d_out) {
@@ -643,14 +644,44 @@ int denoise_impl(spcu_ctx* c, const float* d_rgb_sum, const float* d_lum_sumsq, 
         col[k] = c->dn_col[k].as<float4>();
         var[k] = c->dn_var[k].as<float>();
     }
+    if (conserve) {
+        CK(c, c->dn_var_pf.reserve(n * sizeof(float)));
+        CK(c, c->dn_wsum.reserve(n * sizeof(float)));
+    }
     if (int rc = wait_for_scratch(c, st); rc != SPCU_OK) return rc;
     CK(c, launch_guides(c->ds, c->dn_guides.as<spcu_guide>(), st));
-    CK(c, launch_denoise(c->dn_guides.as<spcu_guide>(), d_rgb_sum, d_lum_sumsq, d_spp_map, spp, c->ds.width, c->ds.height, *p, col, var,
-                         d_out, st));
+    if (conserve) {
+        CK(c, launch_denoise_conserving(c->dn_guides.as<spcu_guide>(), d_rgb_sum, d_lum_sumsq, d_spp_map, spp, c->ds.width, c->ds.height,
+                                        *p, col, var, c->dn_var_pf.as<float>(), c->dn_wsum.as<float>(), d_out, st));
+    } else {
+        CK(c, launch_denoise(c->dn_guides.as<spcu_guide>(), d_rgb_sum, d_lum_sumsq, d_spp_map, spp, c->ds.width, c->ds.height, *p, col,
+                             var, d_out, st));
+    }
     CK(c, cudaEventRecord(c->ev1, st));
     c->scratch_in_use = true;
     c->scratch_stream = st;
     return SPCU_OK;
+}
+
+// spcu_denoise / spcu_denoise_conserving: the sums go up into the host-buffer accumulators, the filter writes the mean colour
+// over the colour sums there, and that buffer comes back to `out`.
+int denoise_host(spcu_ctx* c, const float* rgb_sum, const float* lum_sumsq, const uint32_t* spp_map, uint32_t spp,
+                 const spcu_denoise_params* p, float* out, bool conserve)
+{
+    if (int rc = need_scene(c); rc != SPCU_OK) return rc;
+    if (!rgb_sum || !lum_sumsq || !out) {
+        return fail(c, SPCU_ERR_INVALID, "rgb_sum, lum_sumsq or out is NULL");
+    }
+    const size_t n = static_cast<size_t>(c->ds.width) * c->ds.height;
+    return host_buffer_render(c, true, rgb_sum, lum_sumsq, out, nullptr, true, [&](float* d_rgb_sum, float* d_sq) {
+        uint32_t* d_map = nullptr;
+        if (spp_map) {
+            CK(c, c->ad_spp_map.reserve(n * sizeof(uint32_t)));
+            d_map = c->ad_spp_map.as<uint32_t>();
+            CK(c, cudaMemcpyAsync(d_map, spp_map, n * sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
+        }
+        return denoise_impl(c, d_rgb_sum, d_sq, d_map, spp, p, d_rgb_sum, c->stream, conserve);
+    });
 }
 
 } // namespace
@@ -729,28 +760,25 @@ int spcu_render_guides(spcu_ctx* c, spcu_guide* out)
 int spcu_denoise_device(spcu_ctx* c, const float* d_rgb_sum, const float* d_lum_sumsq, const uint32_t* d_spp_map, uint32_t spp,
                         const spcu_denoise_params* p, float* d_out, void* stream)
 {
-    return denoise_impl(c, d_rgb_sum, d_lum_sumsq, d_spp_map, spp, p, d_out, static_cast<cudaStream_t>(stream));
+    return denoise_impl(c, d_rgb_sum, d_lum_sumsq, d_spp_map, spp, p, d_out, static_cast<cudaStream_t>(stream), false);
 }
 
-// The sums go up into the host-buffer accumulators, the filter writes the mean colour over the colour sums there, and that
-// buffer comes back to `out`.
 int spcu_denoise(spcu_ctx* c, const float* rgb_sum, const float* lum_sumsq, const uint32_t* spp_map, uint32_t spp,
                  const spcu_denoise_params* p, float* out)
 {
-    if (int rc = need_scene(c); rc != SPCU_OK) return rc;
-    if (!rgb_sum || !lum_sumsq || !out) {
-        return fail(c, SPCU_ERR_INVALID, "rgb_sum, lum_sumsq or out is NULL");
-    }
-    const size_t n = static_cast<size_t>(c->ds.width) * c->ds.height;
-    return host_buffer_render(c, true, rgb_sum, lum_sumsq, out, nullptr, true, [&](float* d_rgb_sum, float* d_sq) {
-        uint32_t* d_map = nullptr;
-        if (spp_map) {
-            CK(c, c->ad_spp_map.reserve(n * sizeof(uint32_t)));
-            d_map = c->ad_spp_map.as<uint32_t>();
-            CK(c, cudaMemcpyAsync(d_map, spp_map, n * sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
-        }
-        return denoise_impl(c, d_rgb_sum, d_sq, d_map, spp, p, d_rgb_sum, c->stream);
-    });
+    return denoise_host(c, rgb_sum, lum_sumsq, spp_map, spp, p, out, false);
+}
+
+int spcu_denoise_conserving_device(spcu_ctx* c, const float* d_rgb_sum, const float* d_lum_sumsq, const uint32_t* d_spp_map,
+                                   uint32_t spp, const spcu_denoise_params* p, float* d_out, void* stream)
+{
+    return denoise_impl(c, d_rgb_sum, d_lum_sumsq, d_spp_map, spp, p, d_out, static_cast<cudaStream_t>(stream), true);
+}
+
+int spcu_denoise_conserving(spcu_ctx* c, const float* rgb_sum, const float* lum_sumsq, const uint32_t* spp_map, uint32_t spp,
+                            const spcu_denoise_params* p, float* out)
+{
+    return denoise_host(c, rgb_sum, lum_sumsq, spp_map, spp, p, out, true);
 }
 
 int spcu_resolved_pipeline(const spcu_ctx* c)

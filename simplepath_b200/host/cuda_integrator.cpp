@@ -273,11 +273,15 @@ bool CudaIntegrator::render_frame(const Scene& scene, unsigned spp, Image& image
     if (spp == 0) {
         throw std::runtime_error("CudaIntegrator: samples per pixel must be >= 1");
     }
-    // SPCU_DENOISE=1: the image is the denoised mean (spcu_denoise on device 0, with Context.denoise's defaults)
-    bool denoise = false;
+    // SPCU_DENOISE=1: the image is the denoised mean (spcu_denoise on device 0, with Context.denoise's defaults);
+    // SPCU_DENOISE=conserve: the same with the energy-conserving flux form (spcu_denoise_conserving)
+    bool denoise = false, conserve = false;
     if (const char* d = std::getenv("SPCU_DENOISE"); d && *d) {
-        if (std::string(d) != "1") {
-            throw std::runtime_error(std::string("CudaIntegrator: SPCU_DENOISE must be 1 (or unset), not '") + d + "'");
+        conserve = std::string(d) == "conserve";
+        if (std::string(d) != "1" && !conserve) {
+            throw std::runtime_error(std::string("CudaIntegrator: SPCU_DENOISE must be 1 (the gather form), conserve (the energy-conserving "
+                                                 "form) or unset, not '") +
+                                     d + "'");
         }
         denoise = true;
     }
@@ -313,12 +317,13 @@ bool CudaIntegrator::render_frame(const Scene& scene, unsigned spp, Image& image
         const spcu_denoise_params p{ 5u, 8.0f, 0.1f, 0.1f }; // Context.denoise's defaults (DESIGN.md §12)
         std::vector<float>        mean(sum.size());
         const auto                t0 = std::chrono::steady_clock::now();
-        m_devices[0]->check(spcu_denoise(m_devices[0]->ctx, sum.data(), sumsq.data(), counts.empty() ? nullptr : counts.data(), spp, &p,
-                                         mean.data()),
-                            "spcu_denoise");
+        const auto                filter = conserve ? spcu_denoise_conserving : spcu_denoise;
+        m_devices[0]->check(filter(m_devices[0]->ctx, sum.data(), sumsq.data(), counts.empty() ? nullptr : counts.data(), spp, &p, mean.data()),
+                            conserve ? "spcu_denoise_conserving" : "spcu_denoise");
         const double ms = 1e3 * std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
-        std::fprintf(stderr, "CudaIntegrator: denoised (%u iterations, sigma_l %g, sigma_z %g, sigma_a %g) in %.2f ms\n", p.iterations,
-                     static_cast<double>(p.sigma_l), static_cast<double>(p.sigma_z), static_cast<double>(p.sigma_a), ms);
+        std::fprintf(stderr, "CudaIntegrator: denoised, %s form (%u iterations, sigma_l %g, sigma_z %g, sigma_a %g) in %.2f ms\n",
+                     conserve ? "energy-conserving" : "gather", p.iterations, static_cast<double>(p.sigma_l), static_cast<double>(p.sigma_z),
+                     static_cast<double>(p.sigma_a), ms);
         sum.swap(mean);
         counts.assign(w * h, 1u); // the means, divided by 1 below (exact)
     }
