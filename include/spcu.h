@@ -339,6 +339,46 @@ int spcu_render_adaptive(spcu_ctx* ctx, const spcu_partition* part, const spcu_a
 int spcu_render_adaptive_device(spcu_ctx* ctx, const spcu_partition* part, const spcu_adaptive* ad, float* d_rgb_sum,
                                 float* d_lum_sumsq, uint32_t* d_spp_map, uint32_t* n_passes, spcu_stats* stats, void* stream);
 
+/* Adaptive sampling with predicted sample counts: the same test and stopping rule, but a pixel that fails the test jumps
+ * towards the count its variance says it needs instead of taking pass_spp more samples, so that a round is a few large render
+ * calls.  The partition's sample_end is the budget; sample_begin must be 0.  A pixel's count is always one of the grid
+ *   g_0 = min(min_spp, sample_end),  g_{i+1} = min(2 g_i, sample_end)  (up to g_last = sample_end),
+ * which depends only on these parameters.  Round 0 renders [0, g_0) of every pixel of the partition at grid index j = 0.
+ * After each round every active pixel with g_j < sample_end is tested with n = g_j (the test of spcu_adaptive, same bits),
+ * all tests before any decision; then it stops with n_p = g_j by the rule of spcu_adaptive for its radius (same window),
+ * a stopped pixel counting as passing.  A pixel that does not stop moves to grid index t and renders [g_j, g_t) in the
+ * next round:
+ *   need = v / (T T), float32 with one rounding per operation, v = the test's unbiased variance (d (n / (n - 1)), or 0) and
+ *          T = rel_error (m + abs_floor); need = +inf where T T is 0 or not finite, the quotient is not finite, or a sum is
+ *          not finite;
+ *   t    = j + 1 if the pixel passed its own test (but not its window), else the smallest i in (j, min(j + max_step, last)]
+ *          with (float)g_i >= need, or that upper end if there is none.
+ * (With 0 < T T < inf a pixel that passes has need <= g_j: both rules give j + 1.)  A pixel that reaches g_last = sample_end
+ * stops with n_p = sample_end and counts as passing from then on.  So every n_p is on the grid, t - j <= max_step, and a
+ * pixel's sums equal bit for bit those of a fixed render of [0, n_p) (its ranges are contiguous and the resolve adds them in
+ * sample order): the result does not depend on the tile partition, batch lanes, wavefront size or kernel organisation, a
+ * pixel's path depending only on its own sums and on its window.  n_p cannot decrease as the radius grows.  max_step = 1
+ * is a plain doubling schedule without prediction; with sample_end = 2 min_spp the grid is {min_spp, 2 min_spp} and the
+ * result is that of spcu_render_adaptive with pass_spp = min_spp.  Measured in DESIGN.md §11. */
+typedef struct spcu_adaptive_predicted {
+    uint32_t min_spp;   /* samples before the first test, >= 2                                                        */
+    float    rel_error; /* as spcu_adaptive                                                                           */
+    float    abs_floor; /* as spcu_adaptive                                                                           */
+    uint32_t radius;    /* 0..7, the window of spcu_adaptive                                                          */
+    uint32_t max_step;  /* 1..8: a pixel at grid count g_j renders at most up to g_{j + max_step}                     */
+} spcu_adaptive_predicted;
+
+/* Predicted-count render into host buffers, overwritten as by spcu_render_adaptive (spp_map[y*w+x] = n_p, 0 outside the
+ * partition).  n_rounds (may be NULL) = rounds rendered, n_calls (may be NULL) = render calls, one per non-empty bucket (j, t)
+ * of a round, made in order of j, then t.  SPCU_ERR_INVALID for min_spp < 2, max_step outside 1..8, radius > 7, a rel_error
+ * or abs_floor that is negative or not finite, or sample_begin != 0; the context stays usable. */
+int spcu_render_adaptive_predicted(spcu_ctx* ctx, const spcu_partition* part, const spcu_adaptive_predicted* ap, float* rgb_sum,
+                                   float* lum_sumsq, uint32_t* spp_map, uint32_t* n_rounds, uint32_t* n_calls, spcu_stats* stats);
+/* Same into DEVICE buffers of the image's size on `stream`, as spcu_render_adaptive_device; one synchronise per round. */
+int spcu_render_adaptive_predicted_device(spcu_ctx* ctx, const spcu_partition* part, const spcu_adaptive_predicted* ap,
+                                          float* d_rgb_sum, float* d_lum_sumsq, uint32_t* d_spp_map, uint32_t* n_rounds,
+                                          uint32_t* n_calls, spcu_stats* stats, void* stream);
+
 /* ---- denoising -----------------------------------------------------------------------------------------------------------
  * Turns a low-sample frame into a smoother image: the spatial filter of SVGF (an edge-avoiding à-trous wavelet filter whose
  * luminance term is scaled by each pixel's standard deviation), guided by the first hit of each pixel's camera ray.  Replaces

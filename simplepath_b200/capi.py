@@ -107,6 +107,12 @@ class Adaptive(C.Structure):
                 ("radius", C.c_uint32)]
 
 
+class AdaptivePredicted(C.Structure):
+    """spcu_adaptive_predicted: parameters of spcu_render_adaptive_predicted (include/spcu.h)."""
+    _fields_ = [("min_spp", C.c_uint32), ("rel_error", C.c_float), ("abs_floor", C.c_float), ("radius", C.c_uint32),
+                ("max_step", C.c_uint32)]
+
+
 class Guide(C.Structure):
     """spcu_guide: first-hit guide record of a pixel (include/spcu.h)."""
     _fields_ = [("normal", C.c_float * 3), ("depth", C.c_float), ("albedo", C.c_float * 3), ("id", C.c_int32)]
@@ -137,6 +143,7 @@ EXPORTS = [
     "spcu_comm_unique_id", "spcu_comm_init_rank", "spcu_comm_init_all", "spcu_comm_destroy", "spcu_comm_rank", "spcu_comm_size",
     "spcu_reduce_to_root", "spcu_render_frame_reduced",
     "spcu_render_adaptive", "spcu_render_adaptive_device", "spcu_pack_image_counts",
+    "spcu_render_adaptive_predicted", "spcu_render_adaptive_predicted_device",
     "spcu_render_guides", "spcu_render_guides_device", "spcu_denoise", "spcu_denoise_device",
     "spcu_denoise_conserving", "spcu_denoise_conserving_device",
 ]
@@ -238,6 +245,12 @@ def load(path: Path | str | None = None) -> C.CDLL:
     lib.spcu_render_adaptive_device.argtypes = [vp, C.POINTER(Partition), C.POINTER(Adaptive), vp, vp, vp, C.POINTER(C.c_uint32),
                                                 C.POINTER(Stats), vp]
     lib.spcu_render_adaptive_device.restype = C.c_int
+    lib.spcu_render_adaptive_predicted.argtypes = [vp, C.POINTER(Partition), C.POINTER(AdaptivePredicted), vp, vp, vp,
+                                                   C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), C.POINTER(Stats)]
+    lib.spcu_render_adaptive_predicted.restype = C.c_int
+    lib.spcu_render_adaptive_predicted_device.argtypes = [vp, C.POINTER(Partition), C.POINTER(AdaptivePredicted), vp, vp, vp,
+                                                          C.POINTER(C.c_uint32), C.POINTER(C.c_uint32), C.POINTER(Stats), vp]
+    lib.spcu_render_adaptive_predicted_device.restype = C.c_int
     lib.spcu_render_guides.argtypes = [vp, vp]
     lib.spcu_render_guides.restype = C.c_int
     lib.spcu_render_guides_device.argtypes = [vp, vp, vp]
@@ -548,6 +561,26 @@ class Context:
                                                   _ptr(spp_map), C.byref(passes), C.byref(st)), "spcu_render_adaptive")
         stats = st.as_dict()
         stats["passes"] = passes.value
+        return rgb, sq, spp_map, stats
+
+    def render_adaptive_predicted(self, part: Partition, rel_error: float, min_spp: int = 16, max_step: int = 4,
+                                  abs_floor: float = 0.0, want_sumsq: bool = True, radius: int = 0):
+        """Adaptive sampling with predicted sample counts (spcu_render_adaptive_predicted): the test and stopping rule of
+        render_adaptive, but a pixel that fails jumps up to max_step doublings of its count (min_spp, 2 min_spp, 4 min_spp, ...
+        up to part.sample_end) towards the count its variance predicts.  max_step=1 (plain doubling) measured fastest, and
+        larger steps stop bunny's pixels early at radius 2 (DESIGN.md §11.1).  Returns what render_adaptive returns, with
+        "rounds" and "calls" (render calls) in the stats dict."""
+        rgb = np.empty((self.height, self.width, 3), dtype=np.float32)
+        sq = np.empty((self.height, self.width), dtype=np.float32) if want_sumsq else None
+        spp_map = np.empty((self.height, self.width), dtype=np.uint32)
+        ap = AdaptivePredicted(min_spp, rel_error, abs_floor, radius, max_step)
+        rounds, calls = C.c_uint32(), C.c_uint32()
+        st = Stats()
+        self._check(self.lib.spcu_render_adaptive_predicted(self.h, C.byref(part), C.byref(ap), _ptr(rgb), _ptr(sq) if want_sumsq else None,
+                                                            _ptr(spp_map), C.byref(rounds), C.byref(calls), C.byref(st)),
+                    "spcu_render_adaptive_predicted")
+        stats = st.as_dict()
+        stats["rounds"], stats["calls"] = rounds.value, calls.value
         return rgb, sq, spp_map, stats
 
     def render_guides(self) -> np.ndarray:

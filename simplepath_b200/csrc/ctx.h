@@ -123,8 +123,8 @@ struct spcu_ctx
     spcu::DevBuf              packed;            // packed output image (spcu_render_image / spcu_pack_image)
     // adaptive sampling (spcu_render_adaptive): ping-pong active pixel lists, the per-pixel sample counts, a lum_sumsq
     // accumulator for callers that pass none, the compaction's scratch + active count, the per-tile pass flags of the
-    // neighbourhood test (radius > 0), and the call's event pair
-    spcu::DevBuf              ad_list[2], ad_spp_map, ad_sq, ad_scratch, ad_mask;
+    // neighbourhood test (radius > 0), and the call's event pair; spcu_render_adaptive_predicted also each pixel's grid index
+    spcu::DevBuf              ad_list[2], ad_spp_map, ad_sq, ad_scratch, ad_mask, ad_level;
     cudaEvent_t               ad_ev[2] = { nullptr, nullptr };
     // denoising (spcu_denoise): the guide buffers and the ping-pong colour / variance buffers of the filter's iterations;
     // spcu_denoise_conserving also the prefiltered variance var~ and the weight sums W of an iteration

@@ -136,6 +136,30 @@ cudaError_t launch_adaptive_compact(const uint32_t* d_list, uint32_t n, const fl
                                     uint32_t n_samples, float rel_error, float abs_floor, uint32_t width, uint32_t height,
                                     uint32_t radius, unsigned long long* d_pass_mask, uint32_t* d_spp_map, uint32_t* d_next_list,
                                     void* d_scratch, uint32_t* d_n_next, cudaStream_t st);
+// spcu_render_adaptive_predicted (include/spcu.h), one round's decisions over list entries [0, n), every one below the budget,
+// at grid index d_level[pix] (g_j = min(g0 << j, budget), g_last = budget).  A pixel that stops gets d_spp_map[pix] = g_j; one
+// that moves to t gets d_level[pix] = t and goes, in list order, to the bucket of (j, t) in d_next_list, buckets in the order
+//   id(j, t) = j * min(max_step, last) + (t - j - 1) for t < last,  (last - 1) * min(max_step, last) + j for t = last;
+// those of t = last also get d_spp_map[pix] = budget and, radius > 0, their pass flag.  d_bucket_offset[b] = where bucket b
+// starts, for b < adaptive_predict_buckets(last, max_step), and d_bucket_offset[that] = the total.  radius > 0: every entry's
+// pass flag has been written by launch_adaptive_test before (d_pass_mask as for launch_adaptive_compact).
+// d_scratch: adaptive_predict_scratch_bytes(n, buckets) bytes.  Enqueue only.
+// bucket ids run over [0, (last - 1) * min(max_step, last) + last)
+__host__ __device__ inline uint32_t adaptive_predict_bucket(uint32_t j, uint32_t t, uint32_t last, uint32_t max_step)
+{
+    const uint32_t span = max_step < last ? max_step : last;
+    return t < last ? j * span + (t - j - 1u) : (last - 1u) * span + j;
+}
+uint32_t    adaptive_predict_buckets(uint32_t last, uint32_t max_step);
+size_t      adaptive_predict_scratch_bytes(uint32_t n, uint32_t n_buckets);
+cudaError_t launch_adaptive_test(const uint32_t* d_list, uint32_t n, const float* d_rgb_sum, const float* d_lum_sumsq,
+                                 uint32_t n_samples, float rel_error, float abs_floor, uint32_t width,
+                                 unsigned long long* d_pass_mask, cudaStream_t st);
+cudaError_t launch_adaptive_predict(const uint32_t* d_list, uint32_t n, const float* d_rgb_sum, const float* d_lum_sumsq,
+                                    uint32_t g0, uint32_t budget, uint32_t last, uint32_t max_step, float rel_error,
+                                    float abs_floor, uint32_t width, uint32_t height, uint32_t radius,
+                                    unsigned long long* d_pass_mask, uint8_t* d_level, uint32_t* d_spp_map, uint32_t* d_next_list,
+                                    void* d_scratch, uint32_t* d_bucket_offset, cudaStream_t st);
 // d_spp_map[d_list[i]] = value for i < n
 cudaError_t launch_adaptive_fill(const uint32_t* d_list, uint32_t n, uint32_t value, uint32_t* d_spp_map, cudaStream_t st);
 

@@ -576,6 +576,145 @@ int adaptive_impl(spcu_ctx* c, const spcu_partition* part, const spcu_adaptive* 
     return SPCU_OK;
 }
 
+// spcu_render_adaptive_predicted(_device): rounds over bucketed pixel lists (grid, prediction and stopping rule:
+// include/spcu.h).  Round 0 renders the partition's own list; after it the pixels still going ping-pong between
+// c->ad_list[0/1], bucket-contiguous, each pixel's grid index in c->ad_level.  One render call per non-empty bucket.
+int adaptive_predicted_impl(spcu_ctx* c, const spcu_partition* part, const spcu_adaptive_predicted* ap, float* d_rgb_sum,
+                            float* d_lum_sumsq, uint32_t* d_spp_map, uint32_t* n_rounds, uint32_t* n_calls, spcu_stats* stats,
+                            cudaStream_t caller_stream, bool have_caller_stream)
+{
+    if (int rc = need_scene(c); rc != SPCU_OK) return rc;
+    if (!ap || !d_spp_map) {
+        return fail(c, SPCU_ERR_INVALID, "adaptive parameters or spp map is NULL");
+    }
+    if (ap->min_spp < 2 || ap->max_step < 1 || ap->max_step > 8 || !std::isfinite(ap->rel_error) || !(ap->rel_error >= 0.0f) ||
+        !std::isfinite(ap->abs_floor) || !(ap->abs_floor >= 0.0f)) {
+        return fail(c, SPCU_ERR_INVALID, "bad adaptive parameters: min_spp %u (>= 2), max_step %u (1..8), rel_error %g, abs_floor %g "
+                    "(finite, >= 0)", ap->min_spp, ap->max_step, ap->rel_error, ap->abs_floor);
+    }
+    if (ap->radius > 7) {
+        return fail(c, SPCU_ERR_INVALID, "bad adaptive window radius %u (0..7: the window is clipped to the pixel's 8x8 tile)",
+                    ap->radius);
+    }
+    if (part && part->sample_begin != 0) {
+        return fail(c, SPCU_ERR_INVALID, "adaptive rendering starts at sample 0 (sample_begin %u)", part->sample_begin);
+    }
+    cudaStream_t st = nullptr;
+    if (int rc = prepare_render(c, part, d_rgb_sum, caller_stream, have_caller_stream, st); rc != SPCU_OK) return rc;
+
+    const size_t n_pixels = static_cast<size_t>(c->ds.width) * c->ds.height;
+    float*       d_sq     = d_lum_sumsq;
+    if (!d_sq) { // the stopping test needs the sums of squares
+        CK(c, c->ad_sq.reserve(n_pixels * sizeof(float)));
+        d_sq = c->ad_sq.as<float>();
+    }
+    for (auto& e : c->ad_ev) {
+        if (!e) CK(c, cudaEventCreate(&e));
+    }
+    CK(c, cudaEventRecord(c->ad_ev[0], st));
+    CK(c, cudaMemsetAsync(d_rgb_sum, 0, n_pixels * 3 * sizeof(float), st));
+    CK(c, cudaMemsetAsync(d_sq, 0, n_pixels * sizeof(float), st));
+    CK(c, cudaMemsetAsync(d_spp_map, 0, n_pixels * sizeof(uint32_t), st));
+    spcu_stats     total{};
+    uint32_t       rounds = 0, calls = 0;
+    const uint32_t budget = part->sample_end;
+    // the grid g_0 = min(min_spp, budget), g_{i+1} = min(2 g_i, budget): at most 32 counts below 2^32
+    std::vector<uint32_t> g{ std::min(ap->min_spp, budget) };
+    while (g.back() < budget) {
+        g.push_back(static_cast<uint32_t>(std::min<uint64_t>(2ull * g.back(), budget)));
+    }
+    const uint32_t  last = static_cast<uint32_t>(g.size() - 1);
+    const uint32_t* list = c->pix_list.as<uint32_t>();
+    const uint32_t  n    = c->pix_list_n;
+    auto            render = [&](const uint32_t* l, uint32_t np, uint32_t begin, uint32_t end) {
+        spcu_stats ps{}; // (read back after every call: the fault counter is checked there)
+        if (int rc = render_batches(c, part, l, np, begin, end - begin, d_rgb_sum, d_sq, &ps, st); rc != SPCU_OK) return rc;
+        ++calls;
+        add_stats(total, ps);
+        return SPCU_OK;
+    };
+    if (n > 0 && budget > 0) {
+        if (int rc = render(list, n, 0, g[0]); rc != SPCU_OK) return rc;
+        rounds = 1;
+        if (last == 0) {
+            CK(c, launch_adaptive_fill(list, n, budget, d_spp_map, st));
+        } else {
+            const uint32_t n_buckets = adaptive_predict_buckets(last, ap->max_step);
+            for (auto& l : c->ad_list) {
+                CK(c, l.reserve(static_cast<size_t>(n) * sizeof(uint32_t)));
+            }
+            // bucket offsets + total, then the rounds' scratch
+            const size_t offsets_bytes = (static_cast<size_t>(n_buckets) + 1) * sizeof(uint32_t);
+            CK(c, c->ad_scratch.reserve(offsets_bytes + adaptive_predict_scratch_bytes(n, n_buckets)));
+            CK(c, c->ad_level.reserve(n_pixels));
+            CK(c, cudaMemsetAsync(c->ad_level.p, 0, n_pixels, st));
+            auto* d_offsets = c->ad_scratch.as<uint32_t>();
+            void* d_scratch = static_cast<char*>(c->ad_scratch.p) + offsets_bytes;
+            if (ap->radius > 0) { // all pass: pixels that stop set their bit, those never tested are outside every window
+                const size_t mask_bytes = adaptive_mask_bytes(c->ds.width, c->ds.height);
+                CK(c, c->ad_mask.reserve(mask_bytes));
+                CK(c, cudaMemsetAsync(c->ad_mask.p, 0xff, mask_bytes, st));
+            }
+            struct Range
+            {
+                uint32_t offset, count, n_samples;
+            };
+            std::vector<Range>    tested{ { 0, n, g[0] } }; // the entries of `list` to test, by their count
+            std::vector<uint32_t> h_offsets(n_buckets + 1);
+            uint32_t              n_test = n, next_k = 1;
+            while (n_test > 0) {
+                uint32_t* next = c->ad_list[next_k].as<uint32_t>(); // never the list being read (round 0 reads c->pix_list)
+                next_k ^= 1u;
+                if (ap->radius > 0) { // every pass flag is written before any decision reads one
+                    for (const Range& r : tested) {
+                        CK(c, launch_adaptive_test(list + r.offset, r.count, d_rgb_sum, d_sq, r.n_samples, ap->rel_error, ap->abs_floor,
+                                                   c->ds.width, c->ad_mask.as<unsigned long long>(), st));
+                    }
+                    total.kernel_launches += tested.size();
+                }
+                CK(c, launch_adaptive_predict(list, n_test, d_rgb_sum, d_sq, g[0], budget, last, ap->max_step, ap->rel_error, ap->abs_floor,
+                                              c->ds.width, c->ds.height, ap->radius, c->ad_mask.as<unsigned long long>(),
+                                              c->ad_level.as<uint8_t>(), d_spp_map, next, d_scratch, d_offsets, st));
+                total.kernel_launches += 3;
+                CK(c, cudaMemcpyAsync(h_offsets.data(), d_offsets, h_offsets.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+                CK(c, cudaStreamSynchronize(st)); // the round's calls are shaped by its buckets
+                list = next;
+                tested.clear();
+                bool rendered = false;
+                for (uint32_t j = 0; j < last; ++j) { // calls in a fixed order: j ascending, then t
+                    for (uint32_t t = j + 1; t <= std::min(j + ap->max_step, last); ++t) {
+                        const uint32_t b    = adaptive_predict_bucket(j, t, last, ap->max_step);
+                        const uint32_t size = h_offsets[b + 1] - h_offsets[b];
+                        if (size == 0) {
+                            continue;
+                        }
+                        if (int rc = render(list + h_offsets[b], size, g[j], g[t]); rc != SPCU_OK) return rc;
+                        rendered = true;
+                        if (t < last) {
+                            tested.push_back({ h_offsets[b], size, g[t] });
+                        }
+                    }
+                }
+                rounds += rendered ? 1u : 0u;
+                n_test = h_offsets[adaptive_predict_bucket(0, last, last, ap->max_step)]; // the buckets of t < last come first
+            }
+        }
+    }
+    CK(c, cudaEventRecord(c->ad_ev[1], st));
+    if (stats) {
+        CK(c, cudaEventSynchronize(c->ad_ev[1]));
+        CK(c, cudaEventElapsedTime(&total.device_ms, c->ad_ev[0], c->ad_ev[1]));
+        *stats = total;
+    }
+    if (n_rounds) {
+        *n_rounds = rounds;
+    }
+    if (n_calls) {
+        *n_calls = calls;
+    }
+    return SPCU_OK;
+}
+
 // The host-buffer entry points synchronise anyway: they also read the fault counter (kCntErrors) when no stats were asked
 // for, so a kernel that gave up on a bounded wait fails the call instead of returning a void image.
 int sync_and_check_faults(spcu_ctx* c, bool already_checked)
@@ -713,6 +852,35 @@ int spcu_render_adaptive(spcu_ctx* c, const spcu_partition* part, const spcu_ada
     // (every pass's fault counter has been read)
     return host_buffer_render(c, true, nullptr, nullptr, rgb_sum, lum_sumsq, true, [&](float* d_rgb_sum, float* d_sq) {
         if (int rc = adaptive_impl(c, part, ad, d_rgb_sum, d_sq, c->ad_spp_map.as<uint32_t>(), n_passes, stats, nullptr, false);
+            rc != SPCU_OK) {
+            return rc;
+        }
+        CK(c, cudaMemcpyAsync(spp_map, c->ad_spp_map.p, map_bytes, cudaMemcpyDeviceToHost, c->stream));
+        return SPCU_OK;
+    });
+}
+
+int spcu_render_adaptive_predicted_device(spcu_ctx* c, const spcu_partition* part, const spcu_adaptive_predicted* ap, float* d_rgb_sum,
+                                          float* d_lum_sumsq, uint32_t* d_spp_map, uint32_t* n_rounds, uint32_t* n_calls,
+                                          spcu_stats* stats, void* stream)
+{
+    return adaptive_predicted_impl(c, part, ap, d_rgb_sum, d_lum_sumsq, d_spp_map, n_rounds, n_calls, stats,
+                                   static_cast<cudaStream_t>(stream), true);
+}
+
+int spcu_render_adaptive_predicted(spcu_ctx* c, const spcu_partition* part, const spcu_adaptive_predicted* ap, float* rgb_sum,
+                                   float* lum_sumsq, uint32_t* spp_map, uint32_t* n_rounds, uint32_t* n_calls, spcu_stats* stats)
+{
+    if (int rc = need_scene(c); rc != SPCU_OK) return rc;
+    if (!rgb_sum || !spp_map) {
+        return fail(c, SPCU_ERR_INVALID, "rgb_sum or spp_map is NULL");
+    }
+    const size_t map_bytes = static_cast<size_t>(c->ds.width) * c->ds.height * sizeof(uint32_t);
+    CK(c, c->ad_spp_map.reserve(map_bytes));
+    // (every call's fault counter has been read)
+    return host_buffer_render(c, true, nullptr, nullptr, rgb_sum, lum_sumsq, true, [&](float* d_rgb_sum, float* d_sq) {
+        if (int rc = adaptive_predicted_impl(c, part, ap, d_rgb_sum, d_sq, c->ad_spp_map.as<uint32_t>(), n_rounds, n_calls, stats,
+                                             nullptr, false);
             rc != SPCU_OK) {
             return rc;
         }

@@ -128,7 +128,7 @@ CudaIntegrator::~CudaIntegrator() = default;
 
 // Sum of radiance samples per pixel, row major W*H*3.
 void CudaIntegrator::render_sum(const Scene& scene, unsigned spp, std::vector<float>& rgb_sum, std::vector<std::uint32_t>* spp_map,
-                                float rel_error, std::uint32_t radius, std::vector<float>* lum_sumsq) const
+                                float rel_error, std::uint32_t radius, std::vector<float>* lum_sumsq, std::uint32_t max_step) const
 {
     if (m_devices.empty()) {
         for (int i = 0; i < m_options.n_devices; ++i) {
@@ -230,17 +230,30 @@ void CudaIntegrator::render_sum(const Scene& scene, unsigned spp, std::vector<fl
     if (spp_map) { // (one device: render_frame checks)
         // passes of 16 samples (fewer when the budget is smaller); the first test needs at least 2 samples
         const std::uint32_t  k = std::min(16u, spp);
-        const spcu_adaptive  ad{ std::max(2u, k), k, rel_error, 0.0f, radius };
         const spcu_partition part{ 0u, 1u, 0u, spp, spp, code, m_options.seed };
         spp_map->resize(n / 3u);
-        std::uint32_t passes = 0;
-        m_devices[0]->check(spcu_render_adaptive(m_devices[0]->ctx, &part, &ad, rgb_sum.data(), sq, spp_map->data(), &passes, &m_stats),
-                            "spcu_render_adaptive");
+        std::uint32_t passes = 0, calls = 0;
+        if (max_step) { // predicted counts on the doubling grid from max(2, min(16, spp))
+            const spcu_adaptive_predicted ap{ std::max(2u, k), rel_error, 0.0f, radius, max_step };
+            m_devices[0]->check(spcu_render_adaptive_predicted(m_devices[0]->ctx, &part, &ap, rgb_sum.data(), sq, spp_map->data(), &passes,
+                                                               &calls, &m_stats),
+                                "spcu_render_adaptive_predicted");
+        } else {
+            const spcu_adaptive ad{ std::max(2u, k), k, rel_error, 0.0f, radius };
+            m_devices[0]->check(spcu_render_adaptive(m_devices[0]->ctx, &part, &ad, rgb_sum.data(), sq, spp_map->data(), &passes, &m_stats),
+                                "spcu_render_adaptive");
+        }
         std::uint64_t early = 0;
         for (const std::uint32_t c : *spp_map) {
             early += c < spp ? 1u : 0u;
         }
         const double pixels = static_cast<double>(spp_map->size());
+        if (max_step) {
+            std::fprintf(stderr, "CudaIntegrator: adaptive sampling to %g, predicted counts with max step %u, window radius %u: %u rounds, "
+                         "%u render calls, mean %.2f spp of %u, %.1f %% of pixels stopped early\n", rel_error, max_step, radius, passes,
+                         calls, static_cast<double>(m_stats.paths) / pixels, spp, 100.0 * static_cast<double>(early) / pixels);
+            return;
+        }
         std::fprintf(stderr, "CudaIntegrator: adaptive sampling to %g, window radius %u: %u passes, mean %.2f spp of %u, %.1f %% of pixels "
                      "stopped early\n", rel_error, radius, passes, static_cast<double>(m_stats.paths) / pixels, spp,
                      100.0 * static_cast<double>(early) / pixels);
@@ -304,10 +317,20 @@ bool CudaIntegrator::render_frame(const Scene& scene, unsigned spp, Image& image
             }
             radius = static_cast<std::uint32_t>(v);
         }
+        std::uint32_t max_step = 0; // SPCU_ADAPTIVE_STEP=<1..8>: predicted counts (spcu_render_adaptive_predicted); unset: passes
+        if (const char* m = std::getenv("SPCU_ADAPTIVE_STEP"); m && *m) {
+            char*               m_end = nullptr;
+            const unsigned long v     = std::strtoul(m, &m_end, 10);
+            if (m_end == m || *m_end != '\0' || *m < '0' || *m > '9' || v < 1 || v > 8) {
+                throw std::runtime_error(std::string("CudaIntegrator: SPCU_ADAPTIVE_STEP must be a largest step from 1 to 8, not '") + m +
+                                         "'");
+            }
+            max_step = static_cast<std::uint32_t>(v);
+        }
         if (m_options.n_devices > 1) {
             throw std::runtime_error("CudaIntegrator: SPCU_ADAPTIVE renders on one device; unset SPCU_DEVICES or set it to 1");
         }
-        render_sum(scene, spp, sum, &counts, rel, radius, denoise ? &sumsq : nullptr);
+        render_sum(scene, spp, sum, &counts, rel, radius, denoise ? &sumsq : nullptr, max_step);
     } else {
         render_sum(scene, spp, sum, nullptr, 0.0f, 0, denoise ? &sumsq : nullptr);
     }
